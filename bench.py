@@ -1,11 +1,13 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the B200 batch engine (BASELINE.json metric).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--n-spend N] [--n-issue N]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--n-spend N] [--n-issue N] [--dump-outputs DIR]
 
 One "step" = one pass of `batch_verify_spend_and_refund` over one batch of synthetic SpendProofs
 (default 1,048,576 per GPU = BASELINE.json configs[2]; weak scaling, so N=8 is the 8M-proof batch of
-configs[3]).  Prints ONE JSON line (rank 0):
+configs[3]).  The inputs are generated from fixed seeds, so the same arguments give the same inputs in every run.
+--dump-outputs DIR writes what the last timed step returned (see dump_outputs) so that two builds can be compared
+output for output.  Prints ONE JSON line (rank 0):
 
   value      : spend verify+refund per second, whole job, inputs resident in HBM, device-timed
   e2e        : same metric through the C ABI with pinned HOST buffers (H2D + kernels + D2H in the timed region)
@@ -28,6 +30,7 @@ import time
 import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True       # the tree may be read-only: the benchmark writes nothing there, bytecode caches included
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
@@ -56,6 +59,7 @@ IMAD_WIDE_LANES_PER_CLK_PER_SM = 32
 PROOF_BYTES = 16832
 UNIQUE_PROOFS = 2048                 # valid proofs from the ORACLE prover: CPU baseline sample + cross-check of the engine
 UNIQUE_REQUESTS = 16384
+DUMP_ROWS = 65536                    # --dump-outputs: proofs sampled from the timed batch; 65536 x 161 float32 values = 42 MB
 
 
 def log(*a):
@@ -177,6 +181,25 @@ def libsodium_bound(port_1thread):
         return {"unavailable": repr(ex)}
 
 
+def dump_outputs(out_dir, n, ref, nul, st):
+    """What one call of batch_verify_spend_and_refund over the timed batch returns to its caller -- refund records (n x 128 B),
+    nullifiers (n x 32 B) and statuses (n) -- for a fixed, seeded sample of DUMP_ROWS proofs (all of them when the batch is no
+    larger), as DIR/{refund,nullifier,status}.npy with one byte per float32 value (exact) and the sampled proof indices as
+    DIR/index.npy (float64)."""
+    import torch
+    m = min(n, DUMP_ROWS)
+    idx = np.sort(np.random.RandomState(20261020).choice(n, size=m, replace=False)) if m < n else np.arange(n)
+    sel = torch.as_tensor(idx, device=ref.device)
+    arrays = {"index": idx.astype(np.float64),
+              "refund": ref.view(n, 128)[sel].cpu().numpy().astype(np.float32),
+              "nullifier": nul.view(n, 32)[sel].cpu().numpy().astype(np.float32),
+              "status": st[sel].cpu().numpy().astype(np.float32)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    log(f"[bench] outputs of the last timed step ({m} of {n} proofs, {sum(a.nbytes for a in arrays.values()) / 2**20:.1f} MiB) written to {out_dir}")
+
+
 def run_reference(args, rank, world):
     """--impl reference: the reference's CPU algorithm (oracle port) on all host threads, bounded sample per step."""
     if rank != 0:
@@ -224,7 +247,16 @@ def main():
     ap.add_argument("--no-strong", action="store_true", help="skip the strong-scaling form of configs[3] (8M proofs split over the GPUs)")
     ap.add_argument("--no-multi-abi", action="store_true", help="skip the single-process multi-device C-ABI leg (N > 1)")
     ap.add_argument("--oracle-sample", type=int, default=1024, help="proofs of the timed batch re-verified and re-signed by the CPU oracle")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (refunds, nullifiers, statuses of a fixed, seeded sample of "
+                         f"{DUMP_ROWS} proofs; rank 0's shard when N > 1) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.warmup < 0:
+        ap.error("--warmup must not be negative")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 engine's timed step")
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local = int(os.environ.get("LOCAL_RANK", "0"))
 
     if args.impl == "reference":
@@ -247,7 +279,7 @@ def main():
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
         cpu_group = dist.new_group(backend="gloo")     # host-side barrier for the leg in which rank 0 drives every GPU itself
-    W, K = max(args.warmup, 0), max(args.steps, 1)
+    W, K = args.warmup, args.steps
     n, ni = args.n_spend, args.n_issue
     threads = max(1, (os.cpu_count() or 1) // world)
 
@@ -371,6 +403,8 @@ def main():
         ms = timed(spend_step, 0, K)
     launches = eng.launch_count - launches0
     clocks = clk.summary()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, n, d_ref, d_nul, d_st)
     value = world * n * K / (ms * 1e-3)
     sm_hz = 1e6 * (clocks.get("sm_mhz") or clocks.get("sm_max_mhz") or 1965.0)
     peak_model = sm_count * IMAD_WIDE_LANES_PER_CLK_PER_SM * sm_hz

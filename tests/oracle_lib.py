@@ -3,9 +3,12 @@
 TEST INFRASTRUCTURE ONLY: imported by tests/, __graft_entry__.smoke() and bench.py's
 cpu_baseline / --impl reference legs.  Nothing under anonymous-credit-tokens_b200/ imports it.
 """
+import atexit
 import ctypes as C
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -37,12 +40,16 @@ _lib = None
 
 
 def use_native_build():
-    """bench.py's CPU-baseline legs: rebuild the oracle with -march=native on the machine it is timed on (the shipped .so is
-    compiled for a portable x86-64-v2 target because it travels to the GPU box).  Falls back silently to the portable build."""
+    """bench.py's CPU-baseline legs: rebuild the oracle with -march=native on the machine it is timed on (the built .so is
+    compiled for a portable x86-64-v2 target, so that one build runs on any host).  The native build goes to a temporary
+    directory, removed at exit: the benchmark writes nothing into the tree, which may be read-only.  Falls back silently to
+    the portable build."""
     global _SO, _lib
-    native = os.path.join(ORACLE_DIR, "libact_oracle_native.so")
+    tmp = tempfile.mkdtemp(prefix="act-oracle-native-")
+    atexit.register(shutil.rmtree, tmp, ignore_errors=True)
+    native = os.path.join(tmp, "libact_oracle_native.so")
     try:
-        subprocess.check_call(["make", "-C", ORACLE_DIR, "-s", "-B", "native"], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+        subprocess.check_call(["make", "-C", ORACLE_DIR, "-s", "-B", "native", f"NATIVE={native}"], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
         if os.path.exists(native):
             _SO, _lib = native, None
             return True
