@@ -74,6 +74,9 @@ EXPORTED_SYMBOLS = [
     "act_engine_create_multi", "act_engine_replica_count", "act_engine_replica",
     "act_batch_issue_verify", "act_batch_issue_sign", "act_batch_spend_verify", "act_batch_refund_sign",
     "act_batch_verify_spend_and_refund_screened",
+    "act_nullifier_store_create", "act_nullifier_store_destroy", "act_nullifier_store_device", "act_nullifier_store_size",
+    "act_nullifier_store_screen_dev", "act_nullifier_store_screen", "act_nullifier_store_export",
+    "act_batch_verify_spend_and_refund_recorded",
 ]
 
 
@@ -141,6 +144,14 @@ def load_library():
     lib.act_batch_spend_verify.argtypes = [vp, sz, vp, vp, vp, vp]; lib.act_batch_spend_verify.restype = i32
     lib.act_batch_refund_sign.argtypes = [vp, sz, vp, vp, vp, sz, vp]; lib.act_batch_refund_sign.restype = i32
     lib.act_batch_verify_spend_and_refund_screened.argtypes = [vp, sz, vp, vp, sz, vp, vp, vp, vp]; lib.act_batch_verify_spend_and_refund_screened.restype = i32
+    lib.act_nullifier_store_create.argtypes = [C.POINTER(vp), i32, sz]; lib.act_nullifier_store_create.restype = i32
+    lib.act_nullifier_store_destroy.argtypes = [vp]; lib.act_nullifier_store_destroy.restype = None
+    lib.act_nullifier_store_device.argtypes = [vp]; lib.act_nullifier_store_device.restype = i32
+    lib.act_nullifier_store_size.argtypes = [vp]; lib.act_nullifier_store_size.restype = sz
+    lib.act_nullifier_store_screen_dev.argtypes = [vp, sz, vp, vp, vp, i32, vp]; lib.act_nullifier_store_screen_dev.restype = i32
+    lib.act_nullifier_store_screen.argtypes = [vp, sz, vp, vp, vp, i32]; lib.act_nullifier_store_screen.restype = i32
+    lib.act_nullifier_store_export.argtypes = [vp, vp, sz, C.POINTER(sz)]; lib.act_nullifier_store_export.restype = i32
+    lib.act_batch_verify_spend_and_refund_recorded.argtypes = [vp, vp, sz, vp, vp, vp, vp, vp]; lib.act_batch_verify_spend_and_refund_recorded.restype = i32
     _lib = lib
     return lib
 
@@ -379,6 +390,20 @@ class Engine:
                                                                    ref.ctypes.data, nul.ctypes.data, st.ctypes.data), "act_batch_verify_spend_and_refund_screened")
         return ref, nul, st
 
+    def batch_verify_spend_and_refund_recorded(self, proofs, rnd, store, out=None):
+        """batch_verify_spend_and_refund_screened with a NullifierStore in place of `seen`: replays of the batch or of anything in
+        the store get status 3 and no refund, and the nullifiers of the accepted proofs are recorded in the store.  The store must
+        be on the device of replica 0.  Returns (refunds, nullifiers, status)."""
+        pf = _u8(proofs); n = pf.size // PROOF_BYTES
+        r = _u8(rnd, n * RND_BYTES, "rnd")
+        if out is None:
+            ref = np.zeros(n * REFUND_BYTES, np.uint8); nul = np.zeros(n * 32, np.uint8); st = np.zeros(n, np.uint8)
+        else:
+            ref, nul, st = out
+        _check(self.lib.act_batch_verify_spend_and_refund_recorded(self._h, store._h, n, pf.ctypes.data, r.ctypes.data, ref.ctypes.data, nul.ctypes.data,
+                                                                   st.ctypes.data), "act_batch_verify_spend_and_refund_recorded")
+        return ref, nul, st
+
     def batch_verify_spend_and_refund_screened_ptr(self, n, proofs, rnd, n_seen, seen, refunds, nullifiers, status):
         _check(self.lib.act_batch_verify_spend_and_refund_screened(self._h, n, proofs, rnd, n_seen, seen, refunds, nullifiers, status),
                "act_batch_verify_spend_and_refund_screened")
@@ -467,6 +492,62 @@ class Engine:
 
     def batch_refund_check_dev(self, n, com, refund, status, stream=0):
         _check(self.lib.act_batch_refund_check_dev(self._h, n, com, refund, status, stream), "act_batch_refund_check_dev")
+
+
+class NullifierStore:
+    """The set of nullifiers already spent (the caller's NullifierDb of the reference, src/lib.rs:741-745), resident on one GPU
+    and kept between calls.  Independent of any engine; grows on its own.  Members are 32-byte nullifiers reduced mod l."""
+
+    def __init__(self, device=0, capacity=1 << 20):
+        self.lib = load_library()
+        self._h = C.c_void_p()
+        self.device = device
+        _check(self.lib.act_nullifier_store_create(C.byref(self._h), device, capacity), "act_nullifier_store_create")
+
+    def close(self):
+        if getattr(self, "_h", None) and self._h.value:
+            self.lib.act_nullifier_store_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *a):
+        self.close()
+
+    @property
+    def size(self):
+        """Exact number of members (synchronises)."""
+        return int(self.lib.act_nullifier_store_size(self._h))
+
+    def screen(self, status, nullifiers, record=True):
+        """Status-0 entries whose nullifier is in the store or earlier in the batch get 3 (DoubleSpendError); other statuses are
+        copied.  record: insert the nullifiers whose output status is 0.  Returns the new status array."""
+        st = _u8(status); n = st.size
+        nul = _u8(nullifiers, n * 32, "nullifiers")
+        out = np.zeros(n, np.uint8)
+        _check(self.lib.act_nullifier_store_screen(self._h, n, st.ctypes.data, nul.ctypes.data, out.ctypes.data, 1 if record else 0),
+               "act_nullifier_store_screen")
+        return out
+
+    def screen_dev(self, n, status, nullifiers, status_out, record=True, stream=0):
+        """Device pointers on the store's device (nullifiers 16-byte aligned); stream 0 = the store's own stream."""
+        _check(self.lib.act_nullifier_store_screen_dev(self._h, n, status, nullifiers, status_out, 1 if record else 0, stream),
+               "act_nullifier_store_screen_dev")
+
+    def export(self):
+        """Every member as uint8[size*32], order unspecified."""
+        cap = self.size
+        out = np.zeros(max(cap, 1) * 32, np.uint8)
+        cnt = C.c_size_t(0)
+        _check(self.lib.act_nullifier_store_export(self._h, out.ctypes.data, cap, C.byref(cnt)), "act_nullifier_store_export")
+        return out[:cnt.value * 32]
 
 
 # ---- CBOR wire formats (host; src/cbor.rs) ----

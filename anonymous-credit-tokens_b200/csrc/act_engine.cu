@@ -20,6 +20,7 @@
 #include "act_device.cuh"
 #include "act_aux.cuh"
 #include "act_prove.cuh"
+#include "act_store.cuh"
 
 // ---------------------------------------------------------------------------------------------------
 // kernels: thin index wrappers around the per-thread bodies in act_device.cuh
@@ -1123,6 +1124,232 @@ extern "C" int act_flag_replays(act_engine* e, size_t n, const uint8_t* status, 
     return rc;
 }
 
+// ---------------------------------------------------------------------------------------------------
+// device-resident nullifier store (act_store.cuh): the spent set, kept on one GPU between calls
+// ---------------------------------------------------------------------------------------------------
+struct act_nullifier_store {
+    int device = 0;
+    cudaStream_t stream = nullptr;        // the stream of calls that pass NULL
+    cudaEvent_t done = nullptr;           // recorded after every call: the next one (any stream) waits on it
+    uint4* table = nullptr; size_t slots = 0;
+    rp_key128 key = {0, 0}; uint64_t calls = 0;   // slot PRF key (OS CSPRNG, drawn at creation); per-call tweak of the dedupe table's
+    // d_misc: [0] exact size, [1] bad-key flag, [2] export counter;  h_misc: pinned read-back of [0..1]
+    unsigned long long* d_misc = nullptr; unsigned long long* h_misc = nullptr;
+    u32* dd_table = nullptr; size_t dd_cap = 0;   // in-batch dedupe (replay_insert/resolve_kernel), slots
+    u8* st_tmp = nullptr; size_t st_cap = 0;      // statuses after the store lookup
+};
+#define ACT_STORE_MIN_SLOTS 1024
+// slots for `keys` members at load <= 1/2; 0 when that is not representable
+static size_t store_slots_for(size_t keys) {
+    size_t s = ACT_STORE_MIN_SLOTS;
+    while (s / 2 < keys) { if (s > ((size_t)1 << 58)) return 0; s <<= 1; }
+    return s;
+}
+extern "C" void act_nullifier_store_destroy(act_nullifier_store* s) {
+    if (!s) return;
+    cudaSetDevice(s->device);
+    if (s->stream) cudaStreamSynchronize(s->stream);
+    if (s->done) cudaEventSynchronize(s->done);
+    cudaFree(s->table); cudaFree(s->d_misc); cudaFree(s->dd_table); cudaFree(s->st_tmp);
+    if (s->h_misc) cudaFreeHost(s->h_misc);
+    if (s->done) cudaEventDestroy(s->done);
+    if (s->stream) cudaStreamDestroy(s->stream);
+    explicit_bzero(&s->key, sizeof s->key);
+    delete s;
+}
+extern "C" int act_nullifier_store_create(act_nullifier_store** out, int device, size_t capacity) {
+    if (!out) return fail_msg("act_nullifier_store_create: null argument");
+    *out = nullptr;
+    int ndev = 0;
+    cudaError_t ce = cudaGetDeviceCount(&ndev);
+    if (ce != cudaSuccess || ndev == 0) return fail_msg("act_nullifier_store_create: no CUDA device (the store has no CPU path)");
+    if (device < 0 || device >= ndev) return fail_msg("act_nullifier_store_create: bad device index");
+    size_t slots = store_slots_for(capacity);
+    if (!slots) return fail_msg("act_nullifier_store_create: capacity too large");
+    CK(cudaSetDevice(device));
+    act_nullifier_store* s = new act_nullifier_store();
+    s->device = device;
+    int rc = 0;
+    do {
+#define CKB(call) { cudaError_t e_ = (call); if (e_ != cudaSuccess) { rc = fail(#call, e_); break; } }
+        size_t got = 0;
+        while (got < sizeof s->key) {
+            ssize_t r = getrandom(reinterpret_cast<char*>(&s->key) + got, sizeof s->key - got, 0);
+            if (r <= 0) break;
+            got += (size_t)r;
+        }
+        if (got < sizeof s->key) { rc = fail_msg("act_nullifier_store_create: the OS random source (getrandom) failed"); break; }
+        CKB(cudaStreamCreateWithFlags(&s->stream, cudaStreamNonBlocking));
+        CKB(cudaEventCreateWithFlags(&s->done, cudaEventDisableTiming));
+        CKB(cudaMalloc((void**)&s->d_misc, 4 * sizeof(unsigned long long)));
+        CKB(cudaHostAlloc((void**)&s->h_misc, 4 * sizeof(unsigned long long), cudaHostAllocDefault));
+        CKB(cudaMalloc((void**)&s->table, slots * 32));
+        s->slots = slots;
+        CKB(cudaMemsetAsync(s->table, 0xff, slots * 32, s->stream));
+        CKB(cudaMemsetAsync(s->d_misc, 0, 4 * sizeof(unsigned long long), s->stream));
+        CKB(cudaEventRecord(s->done, s->stream));
+        CKB(cudaStreamSynchronize(s->stream));
+#undef CKB
+    } while (0);
+    if (rc) { act_nullifier_store_destroy(s); return rc; }
+    *out = s;
+    return 0;
+}
+extern "C" int act_nullifier_store_device(const act_nullifier_store* s) { return s ? s->device : -1; }
+// exact member count; waits for the store's last call
+static int store_count(act_nullifier_store* s, size_t* count) {
+    CK(cudaSetDevice(s->device));
+    CK(cudaStreamWaitEvent(s->stream, s->done, 0));
+    CK(cudaMemcpyAsync(s->h_misc, s->d_misc, sizeof(unsigned long long), cudaMemcpyDeviceToHost, s->stream));
+    CK(cudaStreamSynchronize(s->stream));
+    *count = (size_t)s->h_misc[0];
+    return 0;
+}
+extern "C" size_t act_nullifier_store_size(const act_nullifier_store* s) {
+    size_t c = 0;
+    if (!s || store_count(const_cast<act_nullifier_store*>(s), &c)) return 0;
+    return c;
+}
+// a table of at least `slots` slots holding every current member; the old one is freed only once the new one is complete, so a
+// failed allocation leaves the store as it was.  `st` is idle when this runs (act_nullifier_store_screen_dev has synchronised it).
+static int store_grow(act_nullifier_store* s, size_t slots, cudaStream_t st) {
+    uint4* t = nullptr;
+    cudaError_t ce = cudaMalloc((void**)&t, slots * 32);
+    if (ce != cudaSuccess) { cudaGetLastError(); return fail("act_nullifier_store: growing the table (cudaMalloc)", ce); }
+    int rc = 0;
+    do {
+#define CKB(call) { cudaError_t e_ = (call); if (e_ != cudaSuccess) { rc = fail(#call, e_); break; } }
+        CKB(cudaMemsetAsync(t, 0xff, slots * 32, st));
+        store_rehash_kernel<<<nblocks(s->slots, 256), 256, 0, st>>>((u64)s->slots, s->table, t, (u64)(slots - 1), s->key);
+        CKB(cudaGetLastError());
+        CKB(cudaStreamSynchronize(st));
+#undef CKB
+    } while (0);
+    if (rc) { cudaFree(t); return rc; }
+    cudaFree(s->table);
+    s->table = t; s->slots = slots;
+    return 0;
+}
+// Screen of n (status, nullifier) pairs against the store and the batch itself, then (record != 0) insertion of the survivors.
+// In stream order: lookup (+ key check) -> one 16-byte read-back (bad-key flag and exact size) -> growth if the survivors could
+// cross the load limit -> in-batch dedupe -> insert.  Everything that can fail is decided before the insert is launched.
+extern "C" int act_nullifier_store_screen_dev(act_nullifier_store* s, size_t n, const void* status, const void* nullifiers, void* status_out,
+                                              int record, void* stream) {
+    if (!s) return fail_msg("null store");
+    if (n == 0) return 0;
+    if (!status || !nullifiers || !status_out) return fail_msg("act_nullifier_store_screen_dev: null buffer");
+    NEED_ALIGNED("act_nullifier_store_screen_dev", nullifiers);   // status bytes are read one by one
+    if (n >= 0x7fffffffu) return fail_msg("act_nullifier_store_screen_dev: batch too large (at most 2^31 - 2 keys per call)");
+    CK(cudaSetDevice(s->device));
+    for (const void* p : {status, nullifiers, (const void*)status_out}) {
+        cudaPointerAttributes a;
+        if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); return fail_msg("act_nullifier_store_screen_dev: not a device pointer"); }
+        if ((a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) || a.device != s->device)
+            return fail_msg("act_nullifier_store_screen_dev: buffers must be device memory on the store's device");
+    }
+    cudaStream_t st = stream ? (cudaStream_t)stream : s->stream;
+    CK(cudaStreamWaitEvent(st, s->done, 0));
+    if (s->st_cap < n) {   // the store's previous call has drained on st: its scratch can go
+        CK(cudaStreamSynchronize(st));
+        cudaFree(s->st_tmp); s->st_tmp = nullptr; s->st_cap = 0;
+        CK(cudaMalloc((void**)&s->st_tmp, n));
+        s->st_cap = n;
+    }
+    size_t dd = ACT_STORE_MIN_SLOTS;
+    while (dd < 2 * n) dd <<= 1;
+    if (s->dd_cap < dd) {
+        CK(cudaStreamSynchronize(st));
+        cudaFree(s->dd_table); s->dd_table = nullptr; s->dd_cap = 0;
+        CK(cudaMalloc((void**)&s->dd_table, dd * 4));
+        s->dd_cap = dd;
+    }
+    CK(cudaMemsetAsync(s->d_misc + 1, 0, sizeof(unsigned long long), st));
+    store_lookup_kernel<<<nblocks(n, 256), 256, 0, st>>>((u64)n, (const u8*)status, (const uint4*)nullifiers, s->table, (u64)(s->slots - 1), s->key,
+                                                        s->st_tmp, reinterpret_cast<u32*>(s->d_misc + 1));
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(s->h_misc, s->d_misc, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    if (s->h_misc[1]) {
+        CK(cudaEventRecord(s->done, st));
+        return fail_msg("act_nullifier_store_screen_dev: a nullifier with status 0 is not reduced mod l");
+    }
+    size_t size = (size_t)s->h_misc[0];
+    if (record && size + n > s->slots / 2) {
+        size_t want = store_slots_for(size + n);
+        if (!want) return fail_msg("act_nullifier_store_screen_dev: store too large");
+        int rc = store_grow(s, want, st);
+        if (rc) { cudaEventRecord(s->done, st); return rc; }
+    }
+    CK(cudaMemsetAsync(s->dd_table, 0xff, dd * 4, st));
+    rp_key128 seed = {s->key.k0 ^ (++s->calls * 0x9e3779b97f4a7c15ull), s->key.k1};
+    replay_insert_kernel<<<nblocks(n, 256), 256, 0, st>>>((u32)n, 0, s->st_tmp, nullptr, (const uint4*)nullifiers, s->dd_table, (u32)(dd - 1), seed);
+    replay_resolve_kernel<<<nblocks(n, 256), 256, 0, st>>>((u32)n, 0, s->st_tmp, nullptr, (const uint4*)nullifiers, s->dd_table, (u32)(dd - 1), seed,
+                                                           (u8*)status_out);
+    if (record)
+        store_insert_kernel<<<nblocks(n, 256), 256, 0, st>>>((u64)n, (const u8*)status_out, (const uint4*)nullifiers, s->table, (u64)(s->slots - 1),
+                                                            s->key, s->d_misc);
+    CK(cudaGetLastError());
+    CK(cudaEventRecord(s->done, st));
+    return 0;
+}
+extern "C" int act_nullifier_store_screen(act_nullifier_store* s, size_t n, const uint8_t* status, const uint8_t* nullifiers, uint8_t* status_out,
+                                          int record) {
+    if (!s) return fail_msg("null store");
+    if (n == 0) return 0;
+    if (!status || !nullifiers || !status_out) return fail_msg("act_nullifier_store_screen: null buffer");
+    CK(cudaSetDevice(s->device));
+    u8 *d_st = nullptr, *d_nul = nullptr, *d_out = nullptr;
+    int rc = 0;
+    do {
+#define CKB(call) { cudaError_t e_ = (call); if (e_ != cudaSuccess) { rc = fail(#call, e_); break; } }
+        CKB(cudaMalloc((void**)&d_st, n)); CKB(cudaMalloc((void**)&d_nul, n * 32)); CKB(cudaMalloc((void**)&d_out, n));
+        CKB(cudaMemcpyAsync(d_st, status, n, cudaMemcpyHostToDevice, s->stream));
+        CKB(cudaMemcpyAsync(d_nul, nullifiers, n * 32, cudaMemcpyHostToDevice, s->stream));
+        if ((rc = act_nullifier_store_screen_dev(s, n, d_st, d_nul, d_out, record, s->stream))) break;
+        CKB(cudaMemcpyAsync(status_out, d_out, n, cudaMemcpyDeviceToHost, s->stream));
+        CKB(cudaStreamSynchronize(s->stream));
+#undef CKB
+    } while (0);
+    cudaFree(d_st); cudaFree(d_nul); cudaFree(d_out);
+    return rc;
+}
+#define ACT_STORE_EXPORT_SLOTS ((size_t)1 << 24)   // table slots compacted per round trip (512 MB of table, at most as much of keys)
+extern "C" int act_nullifier_store_export(act_nullifier_store* s, uint8_t* out, size_t cap, size_t* count) {
+    if (!s) return fail_msg("null store");
+    if (!count || (cap && !out)) return fail_msg("act_nullifier_store_export: null argument");
+    size_t size = 0;
+    int rc = store_count(s, &size);
+    if (rc) return rc;
+    *count = size;
+    if (cap < size) return fail_msg("act_nullifier_store_export: the output holds fewer keys than the store");
+    if (size == 0) return 0;
+    cudaStream_t st = s->stream;
+    size_t chunk = s->slots < ACT_STORE_EXPORT_SLOTS ? s->slots : ACT_STORE_EXPORT_SLOTS;
+    uint4* d_out = nullptr;
+    size_t written = 0;
+    do {
+#define CKB(call) { cudaError_t e_ = (call); if (e_ != cudaSuccess) { rc = fail(#call, e_); break; } }
+        CKB(cudaMalloc((void**)&d_out, chunk * 32));
+        for (size_t lo = 0; lo < s->slots && !rc; lo += chunk) {
+            CKB(cudaMemsetAsync(s->d_misc + 2, 0, sizeof(unsigned long long), st));
+            store_compact_kernel<<<nblocks(chunk, 256), 256, 0, st>>>((u64)chunk, s->table + 2 * lo, d_out, s->d_misc + 2);
+            CKB(cudaGetLastError());
+            CKB(cudaMemcpyAsync(s->h_misc + 2, s->d_misc + 2, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+            CKB(cudaStreamSynchronize(st));
+            size_t k = (size_t)s->h_misc[2];
+            if (written + k > size) { rc = fail_msg("act_nullifier_store_export: more occupied slots than members"); break; }
+            CKB(cudaMemcpyAsync(out + written * 32, d_out, k * 32, cudaMemcpyDeviceToHost, st));
+            CKB(cudaStreamSynchronize(st));
+            written += k;
+        }
+#undef CKB
+    } while (0);
+    cudaFree(d_out);
+    cudaEventRecord(s->done, st);
+    if (!rc && written != size) rc = fail_msg("act_nullifier_store_export: fewer occupied slots than members");
+    return rc;
+}
+
 static int ensure_skeleton(act_engine* e, int kind) {
     if (kind < 0 || kind > 3) return fail_msg("bad record kind (0 request, 1 response, 2 proof, 3 refund)");
     if (e->d_skel[kind]) return 0;
@@ -1531,12 +1758,12 @@ static int ensure_gather(act_engine* r, size_t m) {
     r->g_cap = m;
     return 0;
 }
-extern "C" int act_batch_verify_spend_and_refund_screened(act_engine* e, size_t n, const uint8_t* proofs, const uint8_t* rnd, size_t n_seen, const uint8_t* seen,
-                                                           uint8_t* refunds, uint8_t* nullifiers, uint8_t* status) {
-    if (!e) return fail_msg("null engine");
-    if (n == 0) return 0;
-    if (!proofs || !rnd || !refunds || !nullifiers || !status || (n_seen && !seen)) return fail_msg("act_batch_verify_spend_and_refund_screened: null buffer");
+// the screen runs against `seen` (n_seen keys, host memory) when store is null, else against the store, recording the survivors
+static int verify_refund_and_screen(act_engine* e, size_t n, const uint8_t* proofs, const uint8_t* rnd, size_t n_seen, const uint8_t* seen,
+                                    act_nullifier_store* store, uint8_t* refunds, uint8_t* nullifiers, uint8_t* status) {
     std::vector<act_engine*> reps = e->replicas.empty() ? std::vector<act_engine*>{e} : e->replicas;
+    if (store && store->device != reps[0]->device)
+        return fail_msg("act_batch_verify_spend_and_refund_recorded: the store must be on the device of replica 0 (where the gather lands)");
     size_t G = reps.size();
     int rc = 0;
     for (size_t g = 0; g < G && !rc; g++) rc = ensure_gather(reps[g], shard_lo(n, g + 1, G) - shard_lo(n, g, G));
@@ -1567,7 +1794,11 @@ extern "C" int act_batch_verify_spend_and_refund_screened(act_engine* e, size_t 
         }
         CKB(cudaMalloc((void**)&d_out, n));
         if (n_seen) { CKB(cudaMalloc((void**)&d_seen, n_seen * 32)); CKB(cudaMemcpyAsync(d_seen, seen, n_seen * 32, cudaMemcpyHostToDevice, st)); }
-        if ((rc = act_flag_replays_dev(r0, n, G > 1 ? d_st : r0->g_st, G > 1 ? d_nul : r0->g_nul, n_seen, d_seen, d_out, st))) break;
+        const u8* g_st = G > 1 ? d_st : r0->g_st;
+        const u8* g_nul = G > 1 ? d_nul : r0->g_nul;
+        if (store) rc = act_nullifier_store_screen_dev(store, n, g_st, g_nul, d_out, 1, st);
+        else rc = act_flag_replays_dev(r0, n, g_st, g_nul, n_seen, d_seen, d_out, st);
+        if (rc) break;
         CKB(cudaMemcpyAsync(status, d_out, n, cudaMemcpyDeviceToHost, st));
         CKB(cudaStreamSynchronize(st));
 #undef CKB
@@ -1576,4 +1807,19 @@ extern "C" int act_batch_verify_spend_and_refund_screened(act_engine* e, size_t 
     if (rc) return rc;
     for (size_t i = 0; i < n; i++) if (status[i] == 3) memset(refunds + i * 128, 0, 128);
     return 0;
+}
+extern "C" int act_batch_verify_spend_and_refund_screened(act_engine* e, size_t n, const uint8_t* proofs, const uint8_t* rnd, size_t n_seen, const uint8_t* seen,
+                                                           uint8_t* refunds, uint8_t* nullifiers, uint8_t* status) {
+    if (!e) return fail_msg("null engine");
+    if (n == 0) return 0;
+    if (!proofs || !rnd || !refunds || !nullifiers || !status || (n_seen && !seen)) return fail_msg("act_batch_verify_spend_and_refund_screened: null buffer");
+    return verify_refund_and_screen(e, n, proofs, rnd, n_seen, seen, nullptr, refunds, nullifiers, status);
+}
+extern "C" int act_batch_verify_spend_and_refund_recorded(act_engine* e, act_nullifier_store* s, size_t n, const uint8_t* proofs, const uint8_t* rnd,
+                                                           uint8_t* refunds, uint8_t* nullifiers, uint8_t* status) {
+    if (!e) return fail_msg("null engine");
+    if (!s) return fail_msg("null store");
+    if (n == 0) return 0;
+    if (!proofs || !rnd || !refunds || !nullifiers || !status) return fail_msg("act_batch_verify_spend_and_refund_recorded: null buffer");
+    return verify_refund_and_screen(e, n, proofs, rnd, 0, nullptr, s, refunds, nullifiers, status);
 }

@@ -73,3 +73,30 @@ def flag_replays(status, nullifiers, seen=None, engine=None):
             t.record_stream(side)
         cur.wait_stream(side)
     return out
+
+
+def screen_with_store(status, nullifiers, store, record=True):
+    """The screen of flag_replays against a device-resident NullifierStore in place of `seen`, on torch's current stream; with
+    `record` the nullifiers that keep status 0 are inserted into the store.  status uint8[n] and nullifiers uint8[n*32] are CUDA
+    tensors on the store's device.  Returns a new status tensor (act_nullifier_store_screen_dev; no CPU path)."""
+    n = status.numel()
+    if n == 0:
+        return status.clone()
+    if not status.is_cuda:
+        raise RuntimeError("screen_with_store needs CUDA tensors (no CPU path)")
+    out = torch.empty_like(status)
+    status, nullifiers = status.contiguous(), nullifiers.contiguous()
+    cur = torch.cuda.current_stream(status.device)
+    if cur.cuda_stream != 0:
+        store.screen_dev(n, status.data_ptr(), nullifiers.data_ptr(), out.data_ptr(), record, cur.cuda_stream)
+    else:
+        # legacy default stream (handle 0 = the store's own stream in the C ABI): side stream ordered both ways, as in flag_replays
+        side = _SIDE.get(status.device)
+        if side is None:
+            side = _SIDE[status.device] = torch.cuda.Stream(device=status.device)
+        side.wait_stream(cur)
+        store.screen_dev(n, status.data_ptr(), nullifiers.data_ptr(), out.data_ptr(), record, side.cuda_stream)
+        for t in (status, nullifiers, out):
+            t.record_stream(side)
+        cur.wait_stream(side)
+    return out

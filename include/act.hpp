@@ -146,6 +146,36 @@ class PrivateKey {         // x and W = G*x; zeroised on destruction like the re
     PublicKey pub_;
 };
 
+// ---- the spent set: the caller's NullifierDb (examples/act.rs:60-77), resident on one GPU ---------------------------------------
+class NullifierStore {
+  public:
+    explicit NullifierStore(int device = 0, size_t capacity = size_t(1) << 20) {
+        if (act_nullifier_store_create(&s_, device, capacity)) throw EngineError("act_nullifier_store_create");
+    }
+    NullifierStore(const NullifierStore&) = delete;
+    NullifierStore& operator=(const NullifierStore&) = delete;
+    ~NullifierStore() { act_nullifier_store_destroy(s_); }
+    act_nullifier_store* raw() { return s_; }
+    int device() const { return act_nullifier_store_device(s_); }
+    size_t size() const { return act_nullifier_store_size(s_); }
+    // status-0 entries whose nullifier is in the store or earlier in the slice become 3 (DoubleSpendError); record: insert the
+    // nullifiers that keep 0.  `status` is updated in place.
+    void screen(std::vector<uint8_t>& status, const std::vector<uint8_t>& nullifiers, bool record = true) {
+        size_t n = status.size();
+        if (nullifiers.size() != n * 32) throw std::invalid_argument("NullifierStore::screen: 32 bytes of nullifier per status");
+        if (act_nullifier_store_screen(s_, n, status.data(), nullifiers.data(), status.data(), record ? 1 : 0)) throw EngineError("act_nullifier_store_screen");
+    }
+    std::vector<Bytes32> members() {
+        size_t cap = size(), count = 0;
+        std::vector<Bytes32> out(cap);
+        if (act_nullifier_store_export(s_, cap ? out[0].data() : nullptr, cap, &count)) throw EngineError("act_nullifier_store_export");
+        out.resize(count);
+        return out;
+    }
+  private:
+    act_nullifier_store* s_ = nullptr;
+};
+
 // ---- the engine: batch forms of the issuer-side calls ------------------------------------------------------------------------
 // Rng: anything with `void fill_bytes(uint8_t* dst, size_t n)` (the reference's `impl CryptoRngCore`).
 class Engine {
@@ -186,6 +216,27 @@ class Engine {
         std::vector<uint8_t> status(n), nul(n * 32), kprime(n * 128), refunds(n * ACT_REFUND_BYTES);
         const uint8_t* pf = n ? proofs[0].bytes.data() : nullptr;
         if (act_batch_spend_verify(e_, n, pf, nul.data(), status.data(), kprime.data())) throw EngineError("act_batch_spend_verify");
+        std::vector<uint8_t> rnd = draw(status, rng);
+        if (act_batch_refund_sign(e_, n, kprime.data(), status.data(), rnd.data(), rnd.size(), refunds.data())) throw EngineError("act_batch_refund_sign");
+        wipe(rnd);
+        std::vector<Result<RefundWithNullifier>> out(n);
+        for (size_t i = 0; i < n; i++) {
+            out[i].status = status[i];
+            std::memcpy(out[i].value.nullifier.data(), nul.data() + 32 * i, 32);
+            std::memcpy(out[i].value.refund.bytes.data(), refunds.data() + i * ACT_REFUND_BYTES, ACT_REFUND_BYTES);
+        }
+        return out;
+    }
+    // the issuer's loop of examples/act.rs:60-77 over ONE rng with the spent set in `store`: verify, check the nullifier (a replay of
+    // the store or of the slice is Err(DoubleSpendError) and gets no refund), refund -- 128 bytes drawn only for the survivors, in
+    // slice order -- and record.  Outputs, the rng's state and the store afterwards equal that loop's.
+    template <typename Rng>
+    std::vector<Result<RefundWithNullifier>> batch_verify_spend_and_refund(const std::vector<SpendProof>& proofs, Rng& rng, NullifierStore& store) {
+        size_t n = proofs.size();
+        std::vector<uint8_t> status(n), nul(n * 32), kprime(n * 128), refunds(n * ACT_REFUND_BYTES);
+        const uint8_t* pf = n ? proofs[0].bytes.data() : nullptr;
+        if (act_batch_spend_verify(e_, n, pf, nul.data(), status.data(), kprime.data())) throw EngineError("act_batch_spend_verify");
+        store.screen(status, nul, true);
         std::vector<uint8_t> rnd = draw(status, rng);
         if (act_batch_refund_sign(e_, n, kprime.data(), status.data(), rnd.data(), rnd.size(), refunds.data())) throw EngineError("act_batch_refund_sign");
         wipe(rnd);

@@ -19,6 +19,8 @@
  *   act_engine_create_multi            = one handle over several GPUs; host-buffer calls shard by request (SURVEY.md 8b, 8e)
  *   act_batch_verify_spend_and_refund_screened
  *                                      = refund() behind the caller's nullifier check (examples/act.rs:60-77) for a slice
+ *   act_nullifier_store_*, act_batch_verify_spend_and_refund_recorded
+ *                                      = that check against a nullifier database resident on the GPU, recorded as it goes
  *
  * Records hold WIRE bytes: points are 32-byte compressed ristretto255 encodings (validated on the
  * device exactly like CompressedRistretto::decompress, src/cbor.rs:62-77) and scalars are 32-byte
@@ -221,6 +223,38 @@ ACT_API int act_batch_refund_sign(act_engine* e, size_t n, const uint8_t* kprime
  * its nullifier is kept.  Single-device engines take the same call (no gather). */
 ACT_API int act_batch_verify_spend_and_refund_screened(act_engine* e, size_t n, const uint8_t* proofs, const uint8_t* rnd, size_t n_seen,
                                                        const uint8_t* seen, uint8_t* refunds, uint8_t* nullifiers, uint8_t* status);
+
+/* ---- device-resident nullifier store: the set of nullifiers already spent (the reference's NullifierDb, src/lib.rs:741-745,
+ * examples/act.rs:60-77), kept in the memory of one GPU between calls.  It holds no key material and is independent of any engine.
+ * Members are 32-byte nullifiers reduced mod l (what the engine emits); a screen whose status-0 keys include one that is not
+ * reduced fails as a whole.
+ *
+ * Screen semantics: those of act_flag_replays with the store in place of `seen`: among status-0 entries, one whose nullifier is in
+ * the store or occurred at an earlier status-0 index of the batch gets 3 (DoubleSpendError); other statuses are copied.  With
+ * record != 0 every nullifier whose output status is 0 is then inserted.  A recording call that fails (bad argument, wrong
+ * device, non-reduced key, failure to grow) leaves the store unchanged.  A store may be used from one host thread at a time;
+ * calls on different streams are ordered by an event. */
+typedef struct act_nullifier_store act_nullifier_store;
+/* capacity = nullifiers to size for up front; the store grows on its own (on-device rehash) when a recording call needs it */
+ACT_API int    act_nullifier_store_create(act_nullifier_store** out, int device, size_t capacity);
+/* frees everything and wipes the slot PRF key */
+ACT_API void   act_nullifier_store_destroy(act_nullifier_store* s);
+ACT_API int    act_nullifier_store_device(const act_nullifier_store* s);
+ACT_API size_t act_nullifier_store_size(const act_nullifier_store* s);     /* synchronises */
+/* the screen against store + batch; record != 0 inserts the survivors.  Bulk import = status all zero, record = 1
+   (status_out[i] == 0 <=> newly inserted).  The _dev form takes device memory of the store's device (nullifiers 16-byte aligned;
+   status_out may equal status) and a stream (NULL = the store's own); it waits once on that stream for a 16-byte read-back (the
+   key check and the exact size, which decides growth) and is asynchronous after it. */
+ACT_API int act_nullifier_store_screen_dev(act_nullifier_store* s, size_t n, const void* status, const void* nullifiers,
+                                           void* status_out, int record, void* stream);
+ACT_API int act_nullifier_store_screen(act_nullifier_store* s, size_t n, const uint8_t* status, const uint8_t* nullifiers,
+                                       uint8_t* status_out, int record);
+/* every member, 32 B each, order unspecified (for checkpoints); *count = size; fails if cap (in keys) < size */
+ACT_API int act_nullifier_store_export(act_nullifier_store* s, uint8_t* out, size_t cap, size_t* count);
+/* the issuer's step with the store: _screened with the store in place of `seen`, survivors recorded.
+   Replays get status 3 and a zero-filled refund, as in _screened.  The store must be on the device of replica 0. */
+ACT_API int act_batch_verify_spend_and_refund_recorded(act_engine* e, act_nullifier_store* s, size_t n, const uint8_t* proofs,
+                                                       const uint8_t* rnd, uint8_t* refunds, uint8_t* nullifiers, uint8_t* status);
 
 /* Client-side batch generators (SURVEY.md 8f-1), bit-exact with the reference's prover for the same RNG bytes but NOT
  * constant time: they exist to synthesise full-size batches of valid, unique fixtures on the device.

@@ -7,6 +7,11 @@ pub struct act_engine {
     _private: [u8; 0],
 }
 
+#[repr(C)]
+pub struct act_nullifier_store {
+    _private: [u8; 0],
+}
+
 pub const ACT_REQUEST_BYTES: usize = 128;
 pub const ACT_RESPONSE_BYTES: usize = 160;
 pub const ACT_PROOF_BYTES: usize = 16832;
@@ -73,6 +78,19 @@ extern "C" {
     pub fn act_batch_refund_check_dev(e: *mut act_engine, n: usize, com: *const c_void, refund: *const c_void, status: *mut c_void,
                                       stream: *mut c_void) -> c_int;
 
+    // the spent set resident on one GPU (NullifierDb kept between calls); independent of any engine
+    pub fn act_nullifier_store_create(out: *mut *mut act_nullifier_store, device: c_int, capacity: usize) -> c_int;
+    pub fn act_nullifier_store_destroy(s: *mut act_nullifier_store);
+    pub fn act_nullifier_store_device(s: *const act_nullifier_store) -> c_int;
+    pub fn act_nullifier_store_size(s: *const act_nullifier_store) -> usize;
+    pub fn act_nullifier_store_screen_dev(s: *mut act_nullifier_store, n: usize, status: *const c_void, nullifiers: *const c_void,
+                                          status_out: *mut c_void, record: c_int, stream: *mut c_void) -> c_int;
+    pub fn act_nullifier_store_screen(s: *mut act_nullifier_store, n: usize, status: *const u8, nullifiers: *const u8, status_out: *mut u8,
+                                      record: c_int) -> c_int;
+    pub fn act_nullifier_store_export(s: *mut act_nullifier_store, out: *mut u8, cap: usize, count: *mut usize) -> c_int;
+    // the issuer's step with the store in place of `seen`; survivors are recorded (store on the device of replica 0)
+    pub fn act_batch_verify_spend_and_refund_recorded(e: *mut act_engine, s: *mut act_nullifier_store, n: usize, proofs: *const u8,
+                                                      rnd: *const u8, refunds: *mut u8, nullifiers: *mut u8, status: *mut u8) -> c_int;
     pub fn act_flag_replays(e: *mut act_engine, n: usize, status: *const u8, nullifiers: *const u8, n_seen: usize, seen: *const u8,
                             status_out: *mut u8) -> c_int;
     pub fn act_flag_replays_dev(e: *mut act_engine, n: usize, status: *const c_void, nullifiers: *const c_void, n_seen: usize,
