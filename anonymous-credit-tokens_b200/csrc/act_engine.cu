@@ -14,6 +14,7 @@
 #include <mutex>
 #include <string>
 #include <thread>
+#include <utility>
 #include <vector>
 
 #include "../../include/act_engine.h"
@@ -366,6 +367,49 @@ static int fail_msg(const char* what) { g_err = what; return -1; }
         cudaError_t e_ = (call);                       \
         if (e_ != cudaSuccess) return fail(#call, e_); \
     } while (0)
+// returns the nonzero result of a call that reports its own error
+#define TRY(call)              \
+    do {                       \
+        int rc_ = (call);      \
+        if (rc_) return rc_;   \
+    } while (0)
+
+// One device allocation and its size in bytes.  The destructor frees it; it can be moved but not copied.  Create and destroy it
+// with its device current.  It converts to T*, so it passes to kernels and copies as the pointer itself.
+template <typename T>
+struct dev_buf {
+    T* p = nullptr;
+    size_t bytes = 0;
+    dev_buf() = default;
+    dev_buf(const dev_buf&) = delete;
+    dev_buf(dev_buf&& o) noexcept { *this = std::move(o); }
+    dev_buf& operator=(dev_buf&& o) noexcept { std::swap(p, o.p); std::swap(bytes, o.bytes); return *this; }   // o frees what was here
+    ~dev_buf() { if (p) cudaFree(p); }
+    operator T*() const { return p; }
+};
+// Gives `b` at least `bytes` bytes; the contents are not kept.  `drain` (if not null) is synchronised before the old buffer is
+// freed, for work queued there that may still read it.  A failed allocation leaves `b` empty and clears the runtime's last error,
+// which the next launch check on this thread would otherwise report.
+template <typename T>
+static int ensure(dev_buf<T>& b, size_t bytes, cudaStream_t drain = nullptr) {
+    if (b.bytes >= bytes) return 0;
+    if (drain) CK(cudaStreamSynchronize(drain));
+    b = dev_buf<T>();
+    cudaError_t e = cudaMalloc((void**)&b.p, bytes);
+    if (e != cudaSuccess) {
+        b.p = nullptr;
+        cudaGetLastError();
+        return fail(("cudaMalloc(" + std::to_string(bytes) + " bytes)").c_str(), e);
+    }
+    b.bytes = bytes;
+    return 0;
+}
+// Zero-fills a device buffer that held secret material, on `st`, and waits for it: on every way out of the scope that declares
+// it.  A path that has already queued the wipe in its own stream order sets p to null.
+struct wipe_dev_on_exit {
+    void* p; size_t n; cudaStream_t st;
+    ~wipe_dev_on_exit() { if (p) { cudaMemsetAsync(p, 0, n, st); cudaStreamSynchronize(st); } }
+};
 
 // Proofs per pipeline chunk (default; act_engine_set_spend_chunk or the environment variable ACT_SPEND_CHUNK change it per
 // engine).  The thread-per-proof stages (head, sign) need about 2 368 warps to fill the machine (148 SMs x 16 warps at 128
@@ -378,18 +422,16 @@ static int fail_msg(const char* what) { g_err = what; return -1; }
 #define ACT_SMALL_CHUNK 262144  // requests per chunk for the light-weight paths
 
 struct spend_scratch {
-    u32 *items = nullptr, *com_niels = nullptr, *kprime = nullptr, *flags = nullptr, *cvs = nullptr;
-    u32* cpts = nullptr;        // half-commitments C'/2 in extended coordinates: m x 256 x 128 B
-    vb_table* tabs = nullptr;   // window tables of the range kernel: grid x 128 threads x ACT_RANGE_SPLIT
-    u32* counter = nullptr;     // work counter of the range kernel (units drawn so far in the current launch)
+    dev_buf<u32> items, com_niels, kprime, flags, cvs;
+    dev_buf<u32> cpts;          // half-commitments C'/2 in extended coordinates: m x 256 x 128 B
+    dev_buf<vb_table> tabs;     // window tables of the range kernel: grid x 128 threads x ACT_RANGE_SPLIT
+    dev_buf<u32> counter;       // work counter of the range kernel (units drawn so far in the current launch)
     unsigned range_grid = 0;
-    size_t cap = 0;
     // recorded after every pipeline that used this scratch set; the next user (possibly on another stream) waits on it
     cudaEvent_t done = nullptr; bool used = false;
 };
-struct io_slot {  // device staging for the host-buffer entry points
-    u8 *in0 = nullptr, *in1 = nullptr, *in2 = nullptr, *out0 = nullptr, *out1 = nullptr, *st = nullptr;
-    size_t cap_in0 = 0, cap_in1 = 0, cap_in2 = 0, cap_out0 = 0, cap_out1 = 0, cap_st = 0;
+struct io_slot {  // device staging for the host-buffer entry points, indexed like host_io (st: status)
+    dev_buf<u8> in[3], out[2], st;
 };
 
 #define ACT_IO_SLOTS 3
@@ -397,9 +439,9 @@ struct act_engine {
     int device = 0;
     cudaStream_t stream[2] = {nullptr, nullptr};
     cudaEvent_t fork = nullptr, join[2] = {nullptr, nullptr};
-    act_ctx* d_ctx = nullptr;
-    ge_niels* d_tables = nullptr;
-    ge* d_bases = nullptr;
+    dev_buf<act_ctx> d_ctx;
+    dev_buf<ge_niels> d_tables;
+    dev_buf<ge> d_bases;
     spend_scratch scratch[2];
     // host-buffer entry points: ACT_IO_SLOTS staging sets filled on a copy stream of their own, so that the H2D of chunk
     // i+1 is already under way while chunk i computes and chunk i-1 drains (the two compute streams alternate as before)
@@ -412,12 +454,12 @@ struct act_engine {
     std::vector<act_engine*> replicas;
     // device copy of a call's status + nullifiers (33 B per proof), kept when a screened multi-device call asks for it:
     // what the NVLink gather to replica 0 reads (act_batch_verify_spend_and_refund_screened)
-    u8 *g_st = nullptr, *g_nul = nullptr; size_t g_cap = 0; bool g_keep = false;
-    int32_t* d_skel[4] = {nullptr, nullptr, nullptr, nullptr};   // canonical CBOR skeletons (request, response, proof, refund)
-    u32* d_rp_table = nullptr; size_t rp_cap = 0;                 // replay-screen hash table
-    rp_key128 rp_key = {0, 0}; uint64_t rp_calls = 0;             // its PRF key (OS CSPRNG, drawn at creation) and a per-call tweak
+    dev_buf<u8> g_st, g_nul; bool g_keep = false;
+    dev_buf<int32_t> d_skel[4];                        // canonical CBOR skeletons (request, response, proof, refund)
+    dev_buf<u32> d_rp_table;                           // replay-screen hash table
+    rp_key128 rp_key = {0, 0}; uint64_t rp_calls = 0;  // its PRF key (OS CSPRNG, drawn at creation) and a per-call tweak
     // prover scratch (one chunk): transcript items, half-points, chunk CVs, challenges, r3
-    u32 *pv_items = nullptr, *pv_cpts = nullptr, *pv_cvs = nullptr, *pv_gammas = nullptr, *pv_aux = nullptr; size_t pv_cap = 0;
+    dev_buf<u32> pv_items, pv_cpts, pv_cvs, pv_gammas, pv_aux;
     // optional per-kernel device timing (CUDA events on the launching stream)
     bool timing = false;
     struct timed { int kind; cudaEvent_t a, b; };
@@ -461,37 +503,43 @@ enum { K_RANGE = 0, K_HEAD, K_CHUNK, K_FINISH, K_SIGN, K_ISSUE, K_ISSUANCE_CHECK
         (e)->launches += 1;                                                                   \
     } while (0)
 
-static int ensure(u8** p, size_t* cap, size_t need) {
-    if (*cap >= need) return 0;
-    if (*p) cudaFree(*p);
-    *p = nullptr; *cap = 0;
-    CK(cudaMalloc((void**)p, need));
-    *cap = need;
-    return 0;
-}
+// one scratch set for chunks of up to n proofs
 static int ensure_scratch(spend_scratch* s, size_t n) {
-    if (!s->tabs) {
+    if (!s->range_grid) {
         int dev = 0, sms = 0, per_sm = 0;
         CK(cudaGetDevice(&dev));
         CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
         CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, spend_range_kernel, ACT_RANGE_BLOCK, 0));
         if (per_sm < 1) per_sm = 1;
         s->range_grid = (unsigned)(sms * per_sm);
-        CK(cudaMalloc((void**)&s->tabs, (size_t)s->range_grid * ACT_RANGE_BLOCK * ACT_RANGE_SPLIT * sizeof(vb_table)));
-        CK(cudaMalloc((void**)&s->counter, 4));
-        CK(cudaEventCreateWithFlags(&s->done, cudaEventDisableTiming));
     }
-    if (s->cap >= n) return 0;
-    cudaFree(s->items); cudaFree(s->com_niels); cudaFree(s->kprime); cudaFree(s->flags); cudaFree(s->cvs); cudaFree(s->cpts);
-    s->cap = 0;
-    CK(cudaMalloc((void**)&s->cpts, n * 2 * ACT_L * 128));
-    CK(cudaMalloc((void**)&s->items, n * ACT_ITEM_WORDS * 4));
-    CK(cudaMalloc((void**)&s->com_niels, n * ACT_L * 96));
-    CK(cudaMalloc((void**)&s->kprime, n * 128));
-    CK(cudaMalloc((void**)&s->flags, n * 4));
-    CK(cudaMalloc((void**)&s->cvs, n * ACT_SPEND_CHUNKS * 32));
-    s->cap = n;
+    TRY(ensure(s->tabs, (size_t)s->range_grid * ACT_RANGE_BLOCK * ACT_RANGE_SPLIT * sizeof(vb_table)));
+    TRY(ensure(s->counter, 4));
+    if (!s->done) CK(cudaEventCreateWithFlags(&s->done, cudaEventDisableTiming));
+    TRY(ensure(s->cpts, n * 2 * ACT_L * 128));
+    TRY(ensure(s->items, n * ACT_ITEM_WORDS * 4));
+    TRY(ensure(s->com_niels, n * ACT_L * 96));
+    TRY(ensure(s->kprime, n * 128));
+    TRY(ensure(s->flags, n * 4));
+    TRY(ensure(s->cvs, n * ACT_SPEND_CHUNKS * 32));
     return 0;
+}
+// the scratch sets a spend batch of n proofs uses, at the size of its largest chunk: set 1 only if the batch spans chunks
+static int ensure_spend_scratch(act_engine* e, size_t n) {
+    size_t cap = n < e->spend_chunk ? n : e->spend_chunk;
+    TRY(ensure_scratch(&e->scratch[0], cap));
+    if (n > e->spend_chunk) TRY(ensure_scratch(&e->scratch[1], cap));
+    return 0;
+}
+// n bytes from the OS CSPRNG; false if it fails
+static bool os_random(void* out, size_t n) {
+    size_t got = 0;
+    while (got < n) {
+        ssize_t r = getrandom(static_cast<char*>(out) + got, n - got, 0);
+        if (r <= 0) return false;
+        got += (size_t)r;
+    }
+    return true;
 }
 
 extern "C" const char* act_last_error(void) { return g_err.c_str(); }
@@ -512,14 +560,13 @@ extern "C" int act_params_derive(int device, const char* org, const char* svc, c
     std::string dom = std::string("ACT-v1:") + org + ":" + svc + ":" + dep + ":" + ver;  // src/lib.rs:293-296
     if (dom.size() > 900) return fail_msg("act_params_derive: domain separator longer than 900 bytes");
     CK(cudaSetDevice(device));
-    u8* d_dom = nullptr; u32* d_out = nullptr;
-    CK(cudaMalloc((void**)&d_dom, dom.size() + 1));
-    CK(cudaMalloc((void**)&d_out, 96));
+    dev_buf<u8> d_dom; dev_buf<u32> d_out;
+    TRY(ensure(d_dom, dom.size() + 1));
+    TRY(ensure(d_out, 96));
     CK(cudaMemcpy(d_dom, dom.data(), dom.size(), cudaMemcpyHostToDevice));
     params_derive_kernel<<<1, 1>>>(d_dom, (u32)dom.size(), d_out);
     CK(cudaGetLastError());
     CK(cudaMemcpy(h, d_out, 96, cudaMemcpyDeviceToHost));
-    cudaFree(d_dom); cudaFree(d_out);
     return 0;
 }
 
@@ -550,11 +597,9 @@ extern "C" void act_engine_destroy(act_engine* e) {
     cudaDeviceSynchronize();
     if (e->stream[0]) {   // every staging copy of signer randomness, and the local memory of the signing kernels
         for (int which = 0; which < 3; which++) {
-            for (int k = 0; k < ACT_IO_SLOTS; k++) {
-                io_slot& io = e->io[k];
-                u8* p = which == 0 ? io.in0 : which == 1 ? io.in1 : io.in2;
-                size_t cap = which == 0 ? io.cap_in0 : which == 1 ? io.cap_in1 : io.cap_in2;
-                if (p && cap) cudaMemsetAsync(p, 0, cap, e->stream[0]);
+            for (io_slot& io : e->io) {
+                dev_buf<u8>& b = io.in[which];
+                if (b.p) cudaMemsetAsync(b, 0, b.bytes, e->stream[0]);
             }
         }
         int sms = 0;
@@ -562,30 +607,77 @@ extern "C" void act_engine_destroy(act_engine* e) {
             scrub_local_kernel<<<sms * 2, 1024, 0, e->stream[0]>>>(nullptr);
         cudaStreamSynchronize(e->stream[0]);
     }
-    cudaFree(e->g_st); cudaFree(e->g_nul);
-    if (e->d_ctx) { cudaMemset(e->d_ctx, 0, sizeof(act_ctx)); cudaFree(e->d_ctx); }  // zeroise x on the device
-    cudaFree(e->d_tables); cudaFree(e->d_bases);
-    for (int k = 0; k < 4; k++) cudaFree(e->d_skel[k]);
-    cudaFree(e->d_rp_table);
-    cudaFree(e->pv_items); cudaFree(e->pv_cpts); cudaFree(e->pv_cvs); cudaFree(e->pv_gammas); cudaFree(e->pv_aux);
+    if (e->d_ctx.p) cudaMemset(e->d_ctx, 0, sizeof(act_ctx));  // zeroise x on the device
     if (e->fork) cudaEventDestroy(e->fork);
     for (int s = 0; s < 2; s++) if (e->join[s]) cudaEventDestroy(e->join[s]);
     for (int s = 0; s < 2; s++) {
-        spend_scratch& sc_ = e->scratch[s];
-        cudaFree(sc_.items); cudaFree(sc_.com_niels); cudaFree(sc_.kprime); cudaFree(sc_.flags); cudaFree(sc_.cvs); cudaFree(sc_.tabs); cudaFree(sc_.counter); cudaFree(sc_.cpts);
-        if (sc_.done) cudaEventDestroy(sc_.done);
+        if (e->scratch[s].done) cudaEventDestroy(e->scratch[s].done);
         if (e->stream[s]) cudaStreamDestroy(e->stream[s]);
     }
     for (int k = 0; k < ACT_IO_SLOTS; k++) {
-        io_slot& io = e->io[k];
-        cudaFree(io.in0); cudaFree(io.in1); cudaFree(io.in2); cudaFree(io.out0); cudaFree(io.out1); cudaFree(io.st);
         if (e->io_ready[k]) cudaEventDestroy(e->io_ready[k]);
         if (e->io_done[k]) cudaEventDestroy(e->io_done[k]);
     }
     if (e->copy) cudaStreamDestroy(e->copy);
-    delete e;
+    delete e;   // frees every device buffer
 }
 
+// streams, events, tables and the device context of a new engine; the caller destroys e if this fails
+static int engine_init(act_engine* e, const uint8_t h[96], const uint8_t sk_x[32], const uint8_t pk_w[32]) {
+    CK(cudaStreamCreateWithFlags(&e->stream[0], cudaStreamNonBlocking));
+    CK(cudaStreamCreateWithFlags(&e->stream[1], cudaStreamNonBlocking));
+    CK(cudaStreamCreateWithFlags(&e->copy, cudaStreamNonBlocking));
+    for (int k = 0; k < ACT_IO_SLOTS; k++) {
+        if (cudaEventCreateWithFlags(&e->io_ready[k], cudaEventDisableTiming) != cudaSuccess ||
+            cudaEventCreateWithFlags(&e->io_done[k], cudaEventDisableTiming) != cudaSuccess) return fail_msg("cudaEventCreate (io slots)");
+    }
+    CK(cudaEventCreateWithFlags(&e->fork, cudaEventDisableTiming));
+    CK(cudaEventCreateWithFlags(&e->join[0], cudaEventDisableTiming));
+    CK(cudaEventCreateWithFlags(&e->join[1], cudaEventDisableTiming));
+    TRY(ensure(e->d_ctx, sizeof(act_ctx)));
+    // replay-screen PRF key
+    if (!os_random(&e->rp_key, sizeof e->rp_key)) return fail_msg("act_engine_create: the OS random source (getrandom) failed");
+    size_t fb_entries = 0;
+    fb_layout L = make_fb_layout(&fb_entries);
+    TRY(ensure(e->d_tables, sizeof(ge_niels) * (fb_entries + ACT_CT_SIZE)));
+    TRY(ensure(e->d_bases, sizeof(ge) * ACT_FB_BASES));
+    dev_buf<u32> d_enc, d_ok;
+    dev_buf<ge> d_W;
+    TRY(ensure(d_enc, 128));
+    TRY(ensure(d_ok, 4));
+    TRY(ensure(d_W, sizeof(ge)));
+    CK(cudaMemcpy(d_enc, h, 96, cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(d_enc.p + 24, pk_w, 32, cudaMemcpyHostToDevice));
+    setup_decode_kernel<<<1, 1>>>(d_enc, e->d_bases, d_W, d_ok);
+    build_fb_tables_kernel<<<(L.first_thread[ACT_FB_BASES] + 31) / 32, 32>>>(e->d_bases, e->d_tables, L);
+    build_ct_table_kernel<<<1, ACT_CT_WIN>>>(e->d_bases, e->d_tables.p + fb_entries);
+    CK(cudaGetLastError());
+    u32 ok = 0;
+    CK(cudaMemcpy(&ok, d_ok, 4, cudaMemcpyDeviceToHost));
+    if (!ok) return fail_msg("act_engine_create: H1/H2/H3/W is not a valid ristretto255 encoding");
+    // context
+    act_ctx hc;
+    struct wipe_on_exit { void* p; size_t n; ~wipe_on_exit() { explicit_bzero(p, n); } } hc_guard{&hc, sizeof hc};   // every way out of this function
+    memset(&hc, 0, sizeof hc);
+    for (int b = 0; b < ACT_FB_BASES; b++) { hc.fb[b].p = e->d_tables.p + L.offset[b]; hc.fb[b].bits = L.bits[b]; hc.fb[b].win = fb_win_of(L.bits[b]); hc.fb[b].ent = fb_ent_of(L.bits[b]); }
+    hc.ct_g = e->d_tables.p + fb_entries;
+    memcpy(hc.h_enc, h, 96);
+    build_prefix(&hc, ACT_TR_REQUEST, "request", h);
+    build_prefix(&hc, ACT_TR_RESPOND, "respond", h);
+    build_prefix(&hc, ACT_TR_REFUND, "refund", h);
+    build_prefix(&hc, ACT_TR_SPEND, "spend", h);
+    CK(cudaMemcpy(&hc.W, d_W, sizeof(ge), cudaMemcpyDeviceToHost));
+    // raw key words; finalize_ctx_kernel reduces them mod l on the device
+    memcpy(hc.x.v, sk_x, 32);
+    CK(cudaMemcpy(e->d_ctx, &hc, sizeof hc, cudaMemcpyHostToDevice));
+    explicit_bzero(&hc, sizeof hc);
+    finalize_ctx_kernel<<<1, 1>>>(e->d_ctx, d_enc.p + 24, d_ok);
+    CK(cudaGetLastError());
+    CK(cudaDeviceSynchronize());
+    CK(cudaMemcpy(&ok, d_ok, 4, cudaMemcpyDeviceToHost));
+    if (!ok) return fail_msg("act_engine_create: pk_w is not the public key of sk_x (W != G*x)");
+    return 0;
+}
 extern "C" int act_engine_create(act_engine** out, int device, const uint8_t h[96], const uint8_t sk_x[32], const uint8_t pk_w[32]) {
     if (!out || !h || !sk_x || !pk_w) return fail_msg("act_engine_create: null argument");
     *out = nullptr;
@@ -596,73 +688,7 @@ extern "C" int act_engine_create(act_engine** out, int device, const uint8_t h[9
     CK(cudaSetDevice(device));
     act_engine* e = new act_engine();
     e->device = device;
-    int rc = 0;
-    u32 *d_enc = nullptr, *d_ok = nullptr;
-    ge* d_W = nullptr;
-    do {
-#define CKB(call) { cudaError_t e_ = (call); if (e_ != cudaSuccess) { rc = fail(#call, e_); break; } }
-        CKB(cudaStreamCreateWithFlags(&e->stream[0], cudaStreamNonBlocking));
-        CKB(cudaStreamCreateWithFlags(&e->stream[1], cudaStreamNonBlocking));
-        CKB(cudaStreamCreateWithFlags(&e->copy, cudaStreamNonBlocking));
-        for (int k = 0; k < ACT_IO_SLOTS && !rc; k++) {
-            if (cudaEventCreateWithFlags(&e->io_ready[k], cudaEventDisableTiming) != cudaSuccess ||
-                cudaEventCreateWithFlags(&e->io_done[k], cudaEventDisableTiming) != cudaSuccess) rc = fail_msg("cudaEventCreate (io slots)");
-        }
-        if (rc) break;
-        CKB(cudaEventCreateWithFlags(&e->fork, cudaEventDisableTiming));
-        CKB(cudaEventCreateWithFlags(&e->join[0], cudaEventDisableTiming));
-        CKB(cudaEventCreateWithFlags(&e->join[1], cudaEventDisableTiming));
-        CKB(cudaMalloc((void**)&e->d_ctx, sizeof(act_ctx)));
-        {   // replay-screen PRF key
-            size_t got = 0;
-            while (got < sizeof e->rp_key) {
-                ssize_t r = getrandom(reinterpret_cast<char*>(&e->rp_key) + got, sizeof e->rp_key - got, 0);
-                if (r <= 0) break;
-                got += (size_t)r;
-            }
-            if (got < sizeof e->rp_key) { rc = fail_msg("act_engine_create: the OS random source (getrandom) failed"); break; }
-        }
-        size_t fb_entries = 0;
-        fb_layout L = make_fb_layout(&fb_entries);
-        CKB(cudaMalloc((void**)&e->d_tables, sizeof(ge_niels) * (fb_entries + ACT_CT_SIZE)));
-        CKB(cudaMalloc((void**)&e->d_bases, sizeof(ge) * ACT_FB_BASES));
-        CKB(cudaMalloc((void**)&d_enc, 128));
-        CKB(cudaMalloc((void**)&d_ok, 4));
-        CKB(cudaMalloc((void**)&d_W, sizeof(ge)));
-        CKB(cudaMemcpy(d_enc, h, 96, cudaMemcpyHostToDevice));
-        CKB(cudaMemcpy(d_enc + 24, pk_w, 32, cudaMemcpyHostToDevice));
-        setup_decode_kernel<<<1, 1>>>(d_enc, e->d_bases, d_W, d_ok);
-        build_fb_tables_kernel<<<(L.first_thread[ACT_FB_BASES] + 31) / 32, 32>>>(e->d_bases, e->d_tables, L);
-        build_ct_table_kernel<<<1, ACT_CT_WIN>>>(e->d_bases, e->d_tables + fb_entries);
-        CKB(cudaGetLastError());
-        u32 ok = 0;
-        CKB(cudaMemcpy(&ok, d_ok, 4, cudaMemcpyDeviceToHost));
-        if (!ok) { rc = fail_msg("act_engine_create: H1/H2/H3/W is not a valid ristretto255 encoding"); break; }
-        // context
-        act_ctx hc;
-        struct wipe_on_exit { void* p; size_t n; ~wipe_on_exit() { explicit_bzero(p, n); } } hc_guard{&hc, sizeof hc};   // every way out of this block
-        memset(&hc, 0, sizeof hc);
-        for (int b = 0; b < ACT_FB_BASES; b++) { hc.fb[b].p = e->d_tables + L.offset[b]; hc.fb[b].bits = L.bits[b]; hc.fb[b].win = fb_win_of(L.bits[b]); hc.fb[b].ent = fb_ent_of(L.bits[b]); }
-        hc.ct_g = e->d_tables + fb_entries;
-        memcpy(hc.h_enc, h, 96);
-        build_prefix(&hc, ACT_TR_REQUEST, "request", h);
-        build_prefix(&hc, ACT_TR_RESPOND, "respond", h);
-        build_prefix(&hc, ACT_TR_REFUND, "refund", h);
-        build_prefix(&hc, ACT_TR_SPEND, "spend", h);
-        CKB(cudaMemcpy(&hc.W, d_W, sizeof(ge), cudaMemcpyDeviceToHost));
-        // raw key words; finalize_ctx_kernel reduces them mod l on the device
-        memcpy(hc.x.v, sk_x, 32);
-        CKB(cudaMemcpy(e->d_ctx, &hc, sizeof hc, cudaMemcpyHostToDevice));
-        explicit_bzero(&hc, sizeof hc);
-        finalize_ctx_kernel<<<1, 1>>>(e->d_ctx, d_enc + 24, d_ok);
-        CKB(cudaGetLastError());
-        CKB(cudaDeviceSynchronize());
-        CKB(cudaMemcpy(&ok, d_ok, 4, cudaMemcpyDeviceToHost));
-        if (!ok) { rc = fail_msg("act_engine_create: pk_w is not the public key of sk_x (W != G*x)"); break; }
-#undef CKB
-    } while (0);
-    cudaFree(d_enc); cudaFree(d_ok); cudaFree(d_W);
-    if (rc) { act_engine_destroy(e); return rc; }
+    if (int rc = engine_init(e, h, sk_x, pk_w)) { act_engine_destroy(e); return rc; }
     e->launches += 3;
     if (const char* env = getenv("ACT_SPEND_CHUNK")) {
         long v = atol(env);
@@ -689,28 +715,23 @@ extern "C" uint64_t act_engine_launch_count(const act_engine* e) {
 extern "C" int act_public_key(int device, const uint8_t sk_x[32], uint8_t pk_w[32]) {
     if (!sk_x || !pk_w) return fail_msg("act_public_key: null argument");
     CK(cudaSetDevice(device));
-    ge *d_b = nullptr, *d_W = nullptr; ge_niels* d_t = nullptr; u32 *d_x = nullptr, *d_o = nullptr, *d_enc = nullptr, *d_ok = nullptr;
-    int rc = 0;
-    do {
-#define CKB(call) { cudaError_t e_ = (call); if (e_ != cudaSuccess) { rc = fail(#call, e_); break; } }
-        CKB(cudaMalloc((void**)&d_b, sizeof(ge) * ACT_FB_BASES));
-        CKB(cudaMalloc((void**)&d_t, sizeof(ge_niels) * ACT_CT_SIZE));
-        CKB(cudaMalloc((void**)&d_x, 32)); CKB(cudaMalloc((void**)&d_o, 32));
-        // bases[0] = G via the set-up kernel with dummy (identity) encodings
-        CKB(cudaMalloc((void**)&d_enc, 128)); CKB(cudaMemset(d_enc, 0, 128));
-        CKB(cudaMalloc((void**)&d_ok, 4)); CKB(cudaMalloc((void**)&d_W, sizeof(ge)));
-        CKB(cudaMemcpy(d_x, sk_x, 32, cudaMemcpyHostToDevice));
-        setup_decode_kernel<<<1, 1>>>(d_enc, d_b, d_W, d_ok);
-        build_ct_table_kernel<<<1, ACT_CT_WIN>>>(d_b, d_t);
-        public_key_kernel<<<1, 1>>>(d_t, d_x, d_o);
-        CKB(cudaGetLastError());
-        CKB(cudaMemcpy(pk_w, d_o, 32, cudaMemcpyDeviceToHost));
-#undef CKB
-    } while (0);
-    // one way out: the device copy of the secret is overwritten before it is freed, whatever failed above
-    if (d_x) { cudaDeviceSynchronize(); cudaMemset(d_x, 0, 32); }
-    cudaFree(d_b); cudaFree(d_t); cudaFree(d_x); cudaFree(d_o); cudaFree(d_enc); cudaFree(d_ok); cudaFree(d_W);
-    return rc;
+    dev_buf<ge> d_b, d_W; dev_buf<ge_niels> d_t; dev_buf<u32> d_x, d_o, d_enc, d_ok;
+    // the device copy of the secret is overwritten before it is freed, whatever fails below (everything runs on the NULL stream)
+    wipe_dev_on_exit x_wipe{nullptr, 32, nullptr};
+    TRY(ensure(d_b, sizeof(ge) * ACT_FB_BASES));
+    TRY(ensure(d_t, sizeof(ge_niels) * ACT_CT_SIZE));
+    TRY(ensure(d_x, 32)); x_wipe.p = d_x;
+    TRY(ensure(d_o, 32));
+    // bases[0] = G via the set-up kernel with dummy (identity) encodings
+    TRY(ensure(d_enc, 128)); CK(cudaMemset(d_enc, 0, 128));
+    TRY(ensure(d_ok, 4)); TRY(ensure(d_W, sizeof(ge)));
+    CK(cudaMemcpy(d_x, sk_x, 32, cudaMemcpyHostToDevice));
+    setup_decode_kernel<<<1, 1>>>(d_enc, d_b, d_W, d_ok);
+    build_ct_table_kernel<<<1, ACT_CT_WIN>>>(d_b, d_t);
+    public_key_kernel<<<1, 1>>>(d_t, d_x, d_o);
+    CK(cudaGetLastError());
+    CK(cudaMemcpy(pk_w, d_o, 32, cudaMemcpyDeviceToHost));
+    return 0;
 }
 
 extern "C" int act_engine_set_timing(act_engine* e, int enable) {
@@ -781,35 +802,40 @@ extern "C" int act_measure_int_mul_peak(int device, double* limb_macs_per_s) {
     cudaDeviceProp p;
     CK(cudaGetDeviceProperties(&p, device));
     int blocks = p.multiProcessorCount * 8;     // 8 x 256 threads = 64 warps per SM, one wave
-    u32* out = nullptr;
-    CK(cudaMalloc((void**)&out, (size_t)blocks * 256 * 4));
-    cudaEvent_t a, b;
-    CK(cudaEventCreate(&a)); CK(cudaEventCreate(&b));
+    dev_buf<u32> out;
+    TRY(ensure(out, (size_t)blocks * 256 * 4));
+    cudaEvent_t a = nullptr, b = nullptr;
     double best = 1e30;
-    for (int r = 0; r < 8; r++) {   // the first launches also bring the clocks up
-        CK(cudaEventRecord(a));
-        int_mul_peak_kernel<<<blocks, 256>>>(out, 3);
-        CK(cudaEventRecord(b));
-        CK(cudaEventSynchronize(b));
-        float ms = 0;
-        CK(cudaEventElapsedTime(&ms, a, b));
-        if (r > 1 && ms < best) best = ms;
-    }
-    cudaEventDestroy(a); cudaEventDestroy(b); cudaFree(out);
+    auto timed = [&]() -> int {
+        CK(cudaEventCreate(&a)); CK(cudaEventCreate(&b));
+        for (int r = 0; r < 8; r++) {   // the first launches also bring the clocks up
+            CK(cudaEventRecord(a));
+            int_mul_peak_kernel<<<blocks, 256>>>(out, 3);
+            CK(cudaEventRecord(b));
+            CK(cudaEventSynchronize(b));
+            float ms = 0;
+            CK(cudaEventElapsedTime(&ms, a, b));
+            if (r > 1 && ms < best) best = ms;
+        }
+        return 0;
+    };
+    int rc = timed();
+    if (a) cudaEventDestroy(a);
+    if (b) cudaEventDestroy(b);
+    if (rc) return rc;
     *limb_macs_per_s = (double)blocks * 256 * PEAK_ITER * PEAK_CHAINS / (best * 1e-3);
     return 0;
 }
 
 extern "C" int act_selftest(int device) {
     CK(cudaSetDevice(device));
-    u32* d_fail = nullptr;
-    CK(cudaMalloc((void**)&d_fail, 4));
+    dev_buf<u32> d_fail;
+    TRY(ensure(d_fail, 4));
     CK(cudaMemset(d_fail, 0, 4));
     selftest_kernel<<<8, 64>>>(d_fail);
     CK(cudaGetLastError());
     u32 f = 0;
     CK(cudaMemcpy(&f, d_fail, 4, cudaMemcpyDeviceToHost));
-    cudaFree(d_fail);
     if (f) { char b[64]; snprintf(b, sizeof b, "act_selftest: failure mask 0x%x", f); g_err = b; return (int)f; }
     return 0;
 }
@@ -898,13 +924,10 @@ extern "C" int act_batch_verify_spend_and_refund_dev(act_engine* e, size_t n, co
     CK(cudaSetDevice(e->device));
     cudaStream_t user = stream ? (cudaStream_t)stream : e->stream[0];
     const size_t ACT_SPEND_CHUNK_RT = e->spend_chunk;
-    size_t cap = n < ACT_SPEND_CHUNK_RT ? n : ACT_SPEND_CHUNK_RT;
-    int rc;
     // chunks alternate over the engine's two streams (each with its own scratch) so that the thread-per-proof
     // kernels of one chunk overlap the range kernel of the next; fork from / join into the caller's stream.
     bool two = n > ACT_SPEND_CHUNK_RT;
-    if ((rc = ensure_scratch(&e->scratch[0], cap))) return rc;
-    if (two && (rc = ensure_scratch(&e->scratch[1], cap))) return rc;
+    TRY(ensure_spend_scratch(e, n));
     if (two) {
         CK(cudaEventRecord(e->fork, user));
         CK(cudaStreamWaitEvent(e->stream[0], e->fork, 0));
@@ -915,9 +938,8 @@ extern "C" int act_batch_verify_spend_and_refund_dev(act_engine* e, size_t n, co
         size_t m = n - off < ACT_SPEND_CHUNK_RT ? n - off : ACT_SPEND_CHUNK_RT;
         int slot = two ? (int)(ci & 1) : 0;
         cudaStream_t st = two ? e->stream[slot] : user;
-        rc = spend_chunk_launch(e, &e->scratch[slot], st, m, (const u32*)proofs + off * ACT_PROOF_WORDS, (const u32*)rnd + off * 32,
-                                (u32*)refunds + off * 32, (u32*)nullifiers + off * 8, (u8*)status + off);
-        if (rc) return rc;
+        TRY(spend_chunk_launch(e, &e->scratch[slot], st, m, (const u32*)proofs + off * ACT_PROOF_WORDS, (const u32*)rnd + off * 32,
+                               (u32*)refunds + off * 32, (u32*)nullifiers + off * 8, (u8*)status + off));
     }
     if (two) {
         CK(cudaEventRecord(e->join[0], e->stream[0]));
@@ -937,11 +959,9 @@ struct host_io {
 // Leaves no signer randomness behind on the device: zero-fills the staging copies of `rnd` (alpha together with the public
 // (z, gamma, e) yields x) and overwrites the local memory the signing kernels used.  Runs on `st`, asynchronously.
 static int scrub_after_signing(act_engine* e, cudaStream_t st, int secret_in) {
-    for (int k = 0; k < ACT_IO_SLOTS; k++) {
-        io_slot& io = e->io[k];
-        u8* p = secret_in == 0 ? io.in0 : secret_in == 1 ? io.in1 : secret_in == 2 ? io.in2 : nullptr;
-        size_t cap = secret_in == 0 ? io.cap_in0 : secret_in == 1 ? io.cap_in1 : secret_in == 2 ? io.cap_in2 : 0;
-        if (p && cap) CK(cudaMemsetAsync(p, 0, cap, st));
+    for (int k = 0; k < ACT_IO_SLOTS && secret_in >= 0; k++) {
+        dev_buf<u8>& b = e->io[k].in[secret_in];
+        if (b.p) CK(cudaMemsetAsync(b, 0, b.bytes, st));
     }
     int sms = 0;
     CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, e->device));
@@ -972,13 +992,9 @@ static int run_chunked(act_engine* e, size_t n, size_t chunk, const host_io& h, 
     // would free memory a running kernel still reads)
     for (size_t k = 0; k < (nchunks < ACT_IO_SLOTS ? nchunks : (size_t)ACT_IO_SLOTS); k++) {
         io_slot& io = e->io[k];
-        int rc;
-        if ((rc = ensure(&io.in0, &io.cap_in0, maxm * h.in_stride[0] + 16))) return rc;
-        if (h.in[1] && (rc = ensure(&io.in1, &io.cap_in1, maxm * h.in_stride[1] + 16))) return rc;
-        if (h.in[2] && (rc = ensure(&io.in2, &io.cap_in2, maxm * h.in_stride[2] + 16))) return rc;
-        if (h.out[0] && (rc = ensure(&io.out0, &io.cap_out0, maxm * h.out_stride[0] + 16))) return rc;
-        if (h.out[1] && (rc = ensure(&io.out1, &io.cap_out1, maxm * h.out_stride[1] + 16))) return rc;
-        if ((rc = ensure(&io.st, &io.cap_st, maxm + 16))) return rc;
+        for (int i = 0; i < 3; i++) if (h.in[i]) TRY(ensure(io.in[i], maxm * h.in_stride[i] + 16));
+        for (int i = 0; i < 2; i++) if (h.out[i]) TRY(ensure(io.out[i], maxm * h.out_stride[i] + 16));
+        TRY(ensure(io.st, maxm + 16));
     }
     size_t off = 0;
     for (size_t ci = 0; ci < nchunks; ci++) {
@@ -987,19 +1003,17 @@ static int run_chunked(act_engine* e, size_t n, size_t chunk, const host_io& h, 
         cudaStream_t st = e->stream[s];
         size_t m = sizes[ci];
         if (ci >= ACT_IO_SLOTS) CK(cudaEventSynchronize(e->io_done[k]));  // slot reuse: chunk ci-3 fully drained (incl. D2H)
-        int rc;
-        CK(cudaMemcpyAsync(io.in0, h.in[0] + off * h.in_stride[0], m * h.in_stride[0], cudaMemcpyHostToDevice, e->copy));
-        if (h.in[1]) CK(cudaMemcpyAsync(io.in1, h.in[1] + off * h.in_stride[1], m * h.in_stride[1], cudaMemcpyHostToDevice, e->copy));
-        if (h.in[2]) CK(cudaMemcpyAsync(io.in2, h.in[2] + off * h.in_stride[2], m * h.in_stride[2], cudaMemcpyHostToDevice, e->copy));
+        for (int i = 0; i < 3; i++)
+            if (h.in[i]) CK(cudaMemcpyAsync(io.in[i], h.in[i] + off * h.in_stride[i], m * h.in_stride[i], cudaMemcpyHostToDevice, e->copy));
         CK(cudaEventRecord(e->io_ready[k], e->copy));
         CK(cudaStreamWaitEvent(st, e->io_ready[k], 0));
-        if ((rc = launch(s, st, m, io))) return rc;
+        TRY(launch(s, st, m, io));
         if (e->g_keep) {   // screened call: status + nullifiers of the whole shard stay on the device for the gather
-            CK(cudaMemcpyAsync(e->g_st + off, io.st, m, cudaMemcpyDeviceToDevice, st));
-            CK(cudaMemcpyAsync(e->g_nul + off * 32, io.out1, m * 32, cudaMemcpyDeviceToDevice, st));
+            CK(cudaMemcpyAsync(e->g_st.p + off, io.st, m, cudaMemcpyDeviceToDevice, st));
+            CK(cudaMemcpyAsync(e->g_nul.p + off * 32, io.out[1], m * 32, cudaMemcpyDeviceToDevice, st));
         }
-        if (h.out[0]) CK(cudaMemcpyAsync(h.out[0] + off * h.out_stride[0], io.out0, m * h.out_stride[0], cudaMemcpyDeviceToHost, st));
-        if (h.out[1]) CK(cudaMemcpyAsync(h.out[1] + off * h.out_stride[1], io.out1, m * h.out_stride[1], cudaMemcpyDeviceToHost, st));
+        for (int i = 0; i < 2; i++)
+            if (h.out[i]) CK(cudaMemcpyAsync(h.out[i] + off * h.out_stride[i], io.out[i], m * h.out_stride[i], cudaMemcpyDeviceToHost, st));
         CK(cudaMemcpyAsync(h.out[2] + off, io.st, m, cudaMemcpyDeviceToHost, st));
         CK(cudaEventRecord(e->io_done[k], st));
         off += m;
@@ -1007,8 +1021,7 @@ static int run_chunked(act_engine* e, size_t n, size_t chunk, const host_io& h, 
     CK(cudaStreamSynchronize(e->stream[0]));
     CK(cudaStreamSynchronize(e->stream[1]));
     if (h.secret_in >= 0) {
-        int rc = scrub_after_signing(e, e->stream[0], h.secret_in);
-        if (rc) return rc;
+        TRY(scrub_after_signing(e, e->stream[0], h.secret_in));
         CK(cudaStreamSynchronize(e->stream[0]));
     }
     return 0;
@@ -1022,7 +1035,7 @@ extern "C" int act_batch_issue(act_engine* e, size_t n, const uint8_t* req, cons
         return act_batch_issue(r, m, req + lo * 128, c + lo * 32, rnd + lo * 128, resp + lo * 160, status + lo); });
     host_io h = {{req, c, rnd}, {128, 32, 128}, {resp, nullptr, status}, {160, 0, 1}, 2};
     return run_chunked(e, n, ACT_SMALL_CHUNK, h, [&](int, cudaStream_t st, size_t m, io_slot& io) {
-        return act_batch_issue_dev(e, m, io.in0, io.in1, io.in2, io.out0, io.st, st);
+        return act_batch_issue_dev(e, m, io.in[0], io.in[1], io.in[2], io.out[0], io.st, st);
     }, true);
 }
 extern "C" int act_batch_issuance_check(act_engine* e, size_t n, const uint8_t* K, const uint8_t* resp, uint8_t* status) {
@@ -1033,7 +1046,7 @@ extern "C" int act_batch_issuance_check(act_engine* e, size_t n, const uint8_t* 
         return act_batch_issuance_check(r, m, K + lo * 32, resp + lo * 160, status + lo); });
     host_io h = {{K, resp, nullptr}, {32, 160, 0}, {nullptr, nullptr, status}, {0, 0, 1}};
     return run_chunked(e, n, ACT_SMALL_CHUNK, h, [&](int, cudaStream_t st, size_t m, io_slot& io) {
-        return act_batch_issuance_check_dev(e, m, io.in0, io.in1, io.st, st);
+        return act_batch_issuance_check_dev(e, m, io.in[0], io.in[1], io.st, st);
     });
 }
 extern "C" int act_batch_refund_check(act_engine* e, size_t n, const uint8_t* com, const uint8_t* refund, uint8_t* status) {
@@ -1044,7 +1057,7 @@ extern "C" int act_batch_refund_check(act_engine* e, size_t n, const uint8_t* co
         return act_batch_refund_check(r, m, com + lo * 4096, refund + lo * 128, status + lo); });
     host_io h = {{com, refund, nullptr}, {4096, 128, 0}, {nullptr, nullptr, status}, {0, 0, 1}};
     return run_chunked(e, n, e->spend_chunk, h, [&](int, cudaStream_t st, size_t m, io_slot& io) {
-        return act_batch_refund_check_dev(e, m, io.in0, io.in1, io.st, st);
+        return act_batch_refund_check_dev(e, m, io.in[0], io.in[1], io.st, st);
     });
 }
 extern "C" int act_batch_verify_spend_and_refund(act_engine* e, size_t n, const uint8_t* proofs, const uint8_t* rnd, uint8_t* refunds,
@@ -1055,16 +1068,11 @@ extern "C" int act_batch_verify_spend_and_refund(act_engine* e, size_t n, const 
     if (is_multi(e)) return shard_over_replicas(e, n, [&](act_engine* r, size_t lo, size_t m) {
         return act_batch_verify_spend_and_refund(r, m, proofs + lo * ACT_PROOF_BYTES, rnd + lo * 128, refunds + lo * 128, nullifiers + lo * 32, status + lo); });
     host_io h = {{proofs, rnd, nullptr}, {ACT_PROOF_BYTES, 128, 0}, {refunds, nullifiers, status}, {128, 32, 1}, 1};
-    // both scratch sets at the size of the largest chunk before anything is in flight
-    {
-        CK(cudaSetDevice(e->device));
-        size_t cap = n < e->spend_chunk ? n : e->spend_chunk;
-        int rc = ensure_scratch(&e->scratch[0], cap);
-        if (!rc && n > e->spend_chunk) rc = ensure_scratch(&e->scratch[1], cap);
-        if (rc) return rc;
-    }
+    // the scratch sets before anything is in flight
+    CK(cudaSetDevice(e->device));
+    TRY(ensure_spend_scratch(e, n));
     return run_chunked(e, n, e->spend_chunk, h, [&](int s, cudaStream_t st, size_t m, io_slot& io) {
-        return spend_chunk_launch(e, &e->scratch[s], st, m, (const u32*)io.in0, (const u32*)io.in1, (u32*)io.out0, (u32*)io.out1, io.st);
+        return spend_chunk_launch(e, &e->scratch[s], st, m, (const u32*)io.in[0].p, (const u32*)io.in[1].p, (u32*)io.out[0].p, (u32*)io.out[1].p, io.st);
     }, true);
 }
 
@@ -1082,12 +1090,7 @@ extern "C" int act_flag_replays_dev(act_engine* e, size_t n, const void* status,
     cudaStream_t st = stream ? (cudaStream_t)stream : e->stream[0];
     size_t slots = 1024;
     while (slots < 2 * (n + n_seen)) slots <<= 1;
-    if (e->rp_cap < slots) {
-        CK(cudaStreamSynchronize(st));
-        cudaFree(e->d_rp_table); e->d_rp_table = nullptr; e->rp_cap = 0;
-        CK(cudaMalloc((void**)&e->d_rp_table, slots * 4));
-        e->rp_cap = slots;
-    }
+    TRY(ensure(e->d_rp_table, slots * 4, st));
     CK(cudaMemsetAsync(e->d_rp_table, 0xff, slots * 4, st));
     // secret per-engine key, tweaked per call: slots are unpredictable to whoever chose the nullifiers
     rp_key128 seed = {e->rp_key.k0 ^ (++e->rp_calls * 0x9e3779b97f4a7c15ull), e->rp_key.k1};
@@ -1107,21 +1110,15 @@ extern "C" int act_flag_replays(act_engine* e, size_t n, const uint8_t* status, 
     if (!status || !nullifiers || !status_out || (n_seen && !seen)) return fail_msg("act_flag_replays: null buffer");
     if (is_multi(e)) return act_flag_replays(e->replicas[0], n, status, nullifiers, n_seen, seen, status_out);   // the screen is global: one device
     CK(cudaSetDevice(e->device));
-    u8 *d_st = nullptr, *d_nul = nullptr, *d_seen = nullptr, *d_out = nullptr;
-    int rc = 0;
-    do {
-#define CKB(call) { cudaError_t e_ = (call); if (e_ != cudaSuccess) { rc = fail(#call, e_); break; } }
-        CKB(cudaMalloc((void**)&d_st, n)); CKB(cudaMalloc((void**)&d_nul, n * 32)); CKB(cudaMalloc((void**)&d_out, n));
-        if (n_seen) { CKB(cudaMalloc((void**)&d_seen, n_seen * 32)); CKB(cudaMemcpyAsync(d_seen, seen, n_seen * 32, cudaMemcpyHostToDevice, e->stream[0])); }
-        CKB(cudaMemcpyAsync(d_st, status, n, cudaMemcpyHostToDevice, e->stream[0]));
-        CKB(cudaMemcpyAsync(d_nul, nullifiers, n * 32, cudaMemcpyHostToDevice, e->stream[0]));
-        if ((rc = act_flag_replays_dev(e, n, d_st, d_nul, n_seen, d_seen, d_out, e->stream[0]))) break;
-        CKB(cudaMemcpyAsync(status_out, d_out, n, cudaMemcpyDeviceToHost, e->stream[0]));
-        CKB(cudaStreamSynchronize(e->stream[0]));
-#undef CKB
-    } while (0);
-    cudaFree(d_st); cudaFree(d_nul); cudaFree(d_seen); cudaFree(d_out);
-    return rc;
+    dev_buf<u8> d_st, d_nul, d_seen, d_out;
+    TRY(ensure(d_st, n)); TRY(ensure(d_nul, n * 32)); TRY(ensure(d_out, n));
+    if (n_seen) { TRY(ensure(d_seen, n_seen * 32)); CK(cudaMemcpyAsync(d_seen, seen, n_seen * 32, cudaMemcpyHostToDevice, e->stream[0])); }
+    CK(cudaMemcpyAsync(d_st, status, n, cudaMemcpyHostToDevice, e->stream[0]));
+    CK(cudaMemcpyAsync(d_nul, nullifiers, n * 32, cudaMemcpyHostToDevice, e->stream[0]));
+    TRY(act_flag_replays_dev(e, n, d_st, d_nul, n_seen, d_seen, d_out, e->stream[0]));
+    CK(cudaMemcpyAsync(status_out, d_out, n, cudaMemcpyDeviceToHost, e->stream[0]));
+    CK(cudaStreamSynchronize(e->stream[0]));
+    return 0;
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -1131,12 +1128,12 @@ struct act_nullifier_store {
     int device = 0;
     cudaStream_t stream = nullptr;        // the stream of calls that pass NULL
     cudaEvent_t done = nullptr;           // recorded after every call: the next one (any stream) waits on it
-    uint4* table = nullptr; size_t slots = 0;
+    dev_buf<uint4> table; size_t slots = 0;
     rp_key128 key = {0, 0}; uint64_t calls = 0;   // slot PRF key (OS CSPRNG, drawn at creation); per-call tweak of the dedupe table's
     // d_misc: [0] exact size, [1] bad-key flag, [2] export counter;  h_misc: pinned read-back of [0..1]
-    unsigned long long* d_misc = nullptr; unsigned long long* h_misc = nullptr;
-    u32* dd_table = nullptr; size_t dd_cap = 0;   // in-batch dedupe (replay_insert/resolve_kernel), slots
-    u8* st_tmp = nullptr; size_t st_cap = 0;      // statuses after the store lookup
+    dev_buf<unsigned long long> d_misc; unsigned long long* h_misc = nullptr;
+    dev_buf<u32> dd_table;   // in-batch dedupe (replay_insert/resolve_kernel)
+    dev_buf<u8> st_tmp;      // statuses after the store lookup
 };
 #define ACT_STORE_MIN_SLOTS 1024
 // slots for `keys` members at load <= 1/2; 0 when that is not representable
@@ -1150,12 +1147,26 @@ extern "C" void act_nullifier_store_destroy(act_nullifier_store* s) {
     cudaSetDevice(s->device);
     if (s->stream) cudaStreamSynchronize(s->stream);
     if (s->done) cudaEventSynchronize(s->done);
-    cudaFree(s->table); cudaFree(s->d_misc); cudaFree(s->dd_table); cudaFree(s->st_tmp);
     if (s->h_misc) cudaFreeHost(s->h_misc);
     if (s->done) cudaEventDestroy(s->done);
     if (s->stream) cudaStreamDestroy(s->stream);
     explicit_bzero(&s->key, sizeof s->key);
-    delete s;
+    delete s;   // frees every device buffer
+}
+// key, stream, event and an empty table of `slots` slots for a new store; the caller destroys s if this fails
+static int store_init(act_nullifier_store* s, size_t slots) {
+    if (!os_random(&s->key, sizeof s->key)) return fail_msg("act_nullifier_store_create: the OS random source (getrandom) failed");
+    CK(cudaStreamCreateWithFlags(&s->stream, cudaStreamNonBlocking));
+    CK(cudaEventCreateWithFlags(&s->done, cudaEventDisableTiming));
+    TRY(ensure(s->d_misc, 4 * sizeof(unsigned long long)));
+    CK(cudaHostAlloc((void**)&s->h_misc, 4 * sizeof(unsigned long long), cudaHostAllocDefault));
+    TRY(ensure(s->table, slots * 32));
+    s->slots = slots;
+    CK(cudaMemsetAsync(s->table, 0xff, slots * 32, s->stream));
+    CK(cudaMemsetAsync(s->d_misc, 0, 4 * sizeof(unsigned long long), s->stream));
+    CK(cudaEventRecord(s->done, s->stream));
+    CK(cudaStreamSynchronize(s->stream));
+    return 0;
 }
 extern "C" int act_nullifier_store_create(act_nullifier_store** out, int device, size_t capacity) {
     if (!out) return fail_msg("act_nullifier_store_create: null argument");
@@ -1169,29 +1180,7 @@ extern "C" int act_nullifier_store_create(act_nullifier_store** out, int device,
     CK(cudaSetDevice(device));
     act_nullifier_store* s = new act_nullifier_store();
     s->device = device;
-    int rc = 0;
-    do {
-#define CKB(call) { cudaError_t e_ = (call); if (e_ != cudaSuccess) { rc = fail(#call, e_); break; } }
-        size_t got = 0;
-        while (got < sizeof s->key) {
-            ssize_t r = getrandom(reinterpret_cast<char*>(&s->key) + got, sizeof s->key - got, 0);
-            if (r <= 0) break;
-            got += (size_t)r;
-        }
-        if (got < sizeof s->key) { rc = fail_msg("act_nullifier_store_create: the OS random source (getrandom) failed"); break; }
-        CKB(cudaStreamCreateWithFlags(&s->stream, cudaStreamNonBlocking));
-        CKB(cudaEventCreateWithFlags(&s->done, cudaEventDisableTiming));
-        CKB(cudaMalloc((void**)&s->d_misc, 4 * sizeof(unsigned long long)));
-        CKB(cudaHostAlloc((void**)&s->h_misc, 4 * sizeof(unsigned long long), cudaHostAllocDefault));
-        CKB(cudaMalloc((void**)&s->table, slots * 32));
-        s->slots = slots;
-        CKB(cudaMemsetAsync(s->table, 0xff, slots * 32, s->stream));
-        CKB(cudaMemsetAsync(s->d_misc, 0, 4 * sizeof(unsigned long long), s->stream));
-        CKB(cudaEventRecord(s->done, s->stream));
-        CKB(cudaStreamSynchronize(s->stream));
-#undef CKB
-    } while (0);
-    if (rc) { act_nullifier_store_destroy(s); return rc; }
+    if (int rc = store_init(s, slots)) { act_nullifier_store_destroy(s); return rc; }
     *out = s;
     return 0;
 }
@@ -1213,21 +1202,14 @@ extern "C" size_t act_nullifier_store_size(const act_nullifier_store* s) {
 // a table of at least `slots` slots holding every current member; the old one is freed only once the new one is complete, so a
 // failed allocation leaves the store as it was.  `st` is idle when this runs (act_nullifier_store_screen_dev has synchronised it).
 static int store_grow(act_nullifier_store* s, size_t slots, cudaStream_t st) {
-    uint4* t = nullptr;
-    cudaError_t ce = cudaMalloc((void**)&t, slots * 32);
-    if (ce != cudaSuccess) { cudaGetLastError(); return fail("act_nullifier_store: growing the table (cudaMalloc)", ce); }
-    int rc = 0;
-    do {
-#define CKB(call) { cudaError_t e_ = (call); if (e_ != cudaSuccess) { rc = fail(#call, e_); break; } }
-        CKB(cudaMemsetAsync(t, 0xff, slots * 32, st));
-        store_rehash_kernel<<<nblocks(s->slots, 256), 256, 0, st>>>((u64)s->slots, s->table, t, (u64)(slots - 1), s->key);
-        CKB(cudaGetLastError());
-        CKB(cudaStreamSynchronize(st));
-#undef CKB
-    } while (0);
-    if (rc) { cudaFree(t); return rc; }
-    cudaFree(s->table);
-    s->table = t; s->slots = slots;
+    dev_buf<uint4> t;
+    TRY(ensure(t, slots * 32));
+    CK(cudaMemsetAsync(t, 0xff, slots * 32, st));
+    store_rehash_kernel<<<nblocks(s->slots, 256), 256, 0, st>>>((u64)s->slots, s->table, t, (u64)(slots - 1), s->key);
+    CK(cudaGetLastError());
+    CK(cudaStreamSynchronize(st));
+    s->table = std::move(t);   // t takes the old table and frees it
+    s->slots = slots;
     return 0;
 }
 // Screen of n (status, nullifier) pairs against the store and the batch itself, then (record != 0) insertion of the survivors.
@@ -1249,23 +1231,14 @@ extern "C" int act_nullifier_store_screen_dev(act_nullifier_store* s, size_t n, 
     }
     cudaStream_t st = stream ? (cudaStream_t)stream : s->stream;
     CK(cudaStreamWaitEvent(st, s->done, 0));
-    if (s->st_cap < n) {   // the store's previous call has drained on st: its scratch can go
-        CK(cudaStreamSynchronize(st));
-        cudaFree(s->st_tmp); s->st_tmp = nullptr; s->st_cap = 0;
-        CK(cudaMalloc((void**)&s->st_tmp, n));
-        s->st_cap = n;
-    }
+    // growing drains st first: the store's previous call has then finished with its scratch
+    TRY(ensure(s->st_tmp, n, st));
     size_t dd = ACT_STORE_MIN_SLOTS;
     while (dd < 2 * n) dd <<= 1;
-    if (s->dd_cap < dd) {
-        CK(cudaStreamSynchronize(st));
-        cudaFree(s->dd_table); s->dd_table = nullptr; s->dd_cap = 0;
-        CK(cudaMalloc((void**)&s->dd_table, dd * 4));
-        s->dd_cap = dd;
-    }
-    CK(cudaMemsetAsync(s->d_misc + 1, 0, sizeof(unsigned long long), st));
+    TRY(ensure(s->dd_table, dd * 4, st));
+    CK(cudaMemsetAsync(s->d_misc.p + 1, 0, sizeof(unsigned long long), st));
     store_lookup_kernel<<<nblocks(n, 256), 256, 0, st>>>((u64)n, (const u8*)status, (const uint4*)nullifiers, s->table, (u64)(s->slots - 1), s->key,
-                                                        s->st_tmp, reinterpret_cast<u32*>(s->d_misc + 1));
+                                                        s->st_tmp, reinterpret_cast<u32*>(s->d_misc.p + 1));
     CK(cudaGetLastError());
     CK(cudaMemcpyAsync(s->h_misc, s->d_misc, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
@@ -1298,20 +1271,14 @@ extern "C" int act_nullifier_store_screen(act_nullifier_store* s, size_t n, cons
     if (n == 0) return 0;
     if (!status || !nullifiers || !status_out) return fail_msg("act_nullifier_store_screen: null buffer");
     CK(cudaSetDevice(s->device));
-    u8 *d_st = nullptr, *d_nul = nullptr, *d_out = nullptr;
-    int rc = 0;
-    do {
-#define CKB(call) { cudaError_t e_ = (call); if (e_ != cudaSuccess) { rc = fail(#call, e_); break; } }
-        CKB(cudaMalloc((void**)&d_st, n)); CKB(cudaMalloc((void**)&d_nul, n * 32)); CKB(cudaMalloc((void**)&d_out, n));
-        CKB(cudaMemcpyAsync(d_st, status, n, cudaMemcpyHostToDevice, s->stream));
-        CKB(cudaMemcpyAsync(d_nul, nullifiers, n * 32, cudaMemcpyHostToDevice, s->stream));
-        if ((rc = act_nullifier_store_screen_dev(s, n, d_st, d_nul, d_out, record, s->stream))) break;
-        CKB(cudaMemcpyAsync(status_out, d_out, n, cudaMemcpyDeviceToHost, s->stream));
-        CKB(cudaStreamSynchronize(s->stream));
-#undef CKB
-    } while (0);
-    cudaFree(d_st); cudaFree(d_nul); cudaFree(d_out);
-    return rc;
+    dev_buf<u8> d_st, d_nul, d_out;
+    TRY(ensure(d_st, n)); TRY(ensure(d_nul, n * 32)); TRY(ensure(d_out, n));
+    CK(cudaMemcpyAsync(d_st, status, n, cudaMemcpyHostToDevice, s->stream));
+    CK(cudaMemcpyAsync(d_nul, nullifiers, n * 32, cudaMemcpyHostToDevice, s->stream));
+    TRY(act_nullifier_store_screen_dev(s, n, d_st, d_nul, d_out, record, s->stream));
+    CK(cudaMemcpyAsync(status_out, d_out, n, cudaMemcpyDeviceToHost, s->stream));
+    CK(cudaStreamSynchronize(s->stream));
+    return 0;
 }
 #define ACT_STORE_EXPORT_SLOTS ((size_t)1 << 24)   // table slots compacted per round trip (512 MB of table, at most as much of keys)
 extern "C" int act_nullifier_store_export(act_nullifier_store* s, uint8_t* out, size_t cap, size_t* count) {
@@ -1325,39 +1292,40 @@ extern "C" int act_nullifier_store_export(act_nullifier_store* s, uint8_t* out, 
     if (size == 0) return 0;
     cudaStream_t st = s->stream;
     size_t chunk = s->slots < ACT_STORE_EXPORT_SLOTS ? s->slots : ACT_STORE_EXPORT_SLOTS;
-    uint4* d_out = nullptr;
     size_t written = 0;
-    do {
-#define CKB(call) { cudaError_t e_ = (call); if (e_ != cudaSuccess) { rc = fail(#call, e_); break; } }
-        CKB(cudaMalloc((void**)&d_out, chunk * 32));
-        for (size_t lo = 0; lo < s->slots && !rc; lo += chunk) {
-            CKB(cudaMemsetAsync(s->d_misc + 2, 0, sizeof(unsigned long long), st));
-            store_compact_kernel<<<nblocks(chunk, 256), 256, 0, st>>>((u64)chunk, s->table + 2 * lo, d_out, s->d_misc + 2);
-            CKB(cudaGetLastError());
-            CKB(cudaMemcpyAsync(s->h_misc + 2, s->d_misc + 2, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-            CKB(cudaStreamSynchronize(st));
+    auto rounds = [&]() -> int {
+        dev_buf<uint4> d_out;
+        TRY(ensure(d_out, chunk * 32));
+        for (size_t lo = 0; lo < s->slots; lo += chunk) {
+            CK(cudaMemsetAsync(s->d_misc.p + 2, 0, sizeof(unsigned long long), st));
+            store_compact_kernel<<<nblocks(chunk, 256), 256, 0, st>>>((u64)chunk, s->table.p + 2 * lo, d_out, s->d_misc.p + 2);
+            CK(cudaGetLastError());
+            CK(cudaMemcpyAsync(s->h_misc + 2, s->d_misc.p + 2, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+            CK(cudaStreamSynchronize(st));
             size_t k = (size_t)s->h_misc[2];
-            if (written + k > size) { rc = fail_msg("act_nullifier_store_export: more occupied slots than members"); break; }
-            CKB(cudaMemcpyAsync(out + written * 32, d_out, k * 32, cudaMemcpyDeviceToHost, st));
-            CKB(cudaStreamSynchronize(st));
+            if (written + k > size) return fail_msg("act_nullifier_store_export: more occupied slots than members");
+            CK(cudaMemcpyAsync(out + written * 32, d_out, k * 32, cudaMemcpyDeviceToHost, st));
+            CK(cudaStreamSynchronize(st));
             written += k;
         }
-#undef CKB
-    } while (0);
-    cudaFree(d_out);
-    cudaEventRecord(s->done, st);
+        return 0;
+    };
+    rc = rounds();
+    cudaEventRecord(s->done, st);   // on every way out: the next call waits for whatever the rounds queued
     if (!rc && written != size) rc = fail_msg("act_nullifier_store_export: fewer occupied slots than members");
     return rc;
 }
 
 static int ensure_skeleton(act_engine* e, int kind) {
     if (kind < 0 || kind > 3) return fail_msg("bad record kind (0 request, 1 response, 2 proof, 3 refund)");
-    if (e->d_skel[kind]) return 0;
+    if (e->d_skel[kind].p) return 0;
     size_t len = act_cbor_len(kind);
     std::vector<int32_t> h(len);
     act_build_skeleton(h.data(), kind);
-    CK(cudaMalloc((void**)&e->d_skel[kind], len * 4));
-    CK(cudaMemcpy(e->d_skel[kind], h.data(), len * 4, cudaMemcpyHostToDevice));
+    dev_buf<int32_t> d;
+    TRY(ensure(d, len * 4));
+    CK(cudaMemcpy(d, h.data(), len * 4, cudaMemcpyHostToDevice));
+    e->d_skel[kind] = std::move(d);   // only once it holds the skeleton
     return 0;
 }
 extern "C" int act_unpack_cbor_dev(act_engine* e, int kind, size_t n, const void* cbor, void* records, void* status, void* stream) {
@@ -1366,8 +1334,7 @@ extern "C" int act_unpack_cbor_dev(act_engine* e, int kind, size_t n, const void
     if (n == 0) return 0;
     if (!cbor || !records || !status) return fail_msg("act_unpack_cbor_dev: null buffer");
     CK(cudaSetDevice(e->device));
-    int rc = ensure_skeleton(e, kind);
-    if (rc) return rc;
+    TRY(ensure_skeleton(e, kind));
     cudaStream_t st = stream ? (cudaStream_t)stream : e->stream[0];
     unsigned grid = (unsigned)(n < 148 * 8 ? n : 148 * 8);
     cbor_unpack_kernel<<<grid, 256, 0, st>>>(n, e->d_skel[kind], (u32)act_cbor_len(kind), (u32)act_rec_len(kind), (const u8*)cbor, (u8*)records, (u8*)status);
@@ -1381,8 +1348,7 @@ extern "C" int act_encode_cbor_dev(act_engine* e, int kind, size_t n, const void
     if (n == 0) return 0;
     if (!cbor || !records) return fail_msg("act_encode_cbor_dev: null buffer");
     CK(cudaSetDevice(e->device));
-    int rc = ensure_skeleton(e, kind);
-    if (rc) return rc;
+    TRY(ensure_skeleton(e, kind));
     cudaStream_t st = stream ? (cudaStream_t)stream : e->stream[0];
     size_t total = n * act_cbor_len(kind);
     unsigned grid = (unsigned)((total + 255) / 256 < 148 * 16 ? (total + 255) / 256 : 148 * 16);
@@ -1394,22 +1360,15 @@ extern "C" int act_encode_cbor_dev(act_engine* e, int kind, size_t n, const void
 // host-buffer forms (one staging round trip; meant for ingest/egress next to the batch calls)
 static int cbor_host_roundtrip(act_engine* e, int kind, size_t n, const uint8_t* in, size_t in_rec, uint8_t* out, size_t out_rec, uint8_t* status, bool unpack) {
     CK(cudaSetDevice(e->device));
-    u8 *d_in = nullptr, *d_out = nullptr, *d_st = nullptr;
-    int rc = 0;
-    do {
-#define CKB(call) { cudaError_t e_ = (call); if (e_ != cudaSuccess) { rc = fail(#call, e_); break; } }
-        CKB(cudaMalloc((void**)&d_in, n * in_rec)); CKB(cudaMalloc((void**)&d_out, n * out_rec));
-        if (unpack) CKB(cudaMalloc((void**)&d_st, n));
-        CKB(cudaMemcpyAsync(d_in, in, n * in_rec, cudaMemcpyHostToDevice, e->stream[0]));
-        rc = unpack ? act_unpack_cbor_dev(e, kind, n, d_in, d_out, d_st, e->stream[0]) : act_encode_cbor_dev(e, kind, n, d_in, d_out, e->stream[0]);
-        if (rc) break;
-        CKB(cudaMemcpyAsync(out, d_out, n * out_rec, cudaMemcpyDeviceToHost, e->stream[0]));
-        if (unpack) CKB(cudaMemcpyAsync(status, d_st, n, cudaMemcpyDeviceToHost, e->stream[0]));
-        CKB(cudaStreamSynchronize(e->stream[0]));
-#undef CKB
-    } while (0);
-    cudaFree(d_in); cudaFree(d_out); cudaFree(d_st);
-    return rc;
+    dev_buf<u8> d_in, d_out, d_st;
+    TRY(ensure(d_in, n * in_rec)); TRY(ensure(d_out, n * out_rec));
+    if (unpack) TRY(ensure(d_st, n));
+    CK(cudaMemcpyAsync(d_in, in, n * in_rec, cudaMemcpyHostToDevice, e->stream[0]));
+    TRY(unpack ? act_unpack_cbor_dev(e, kind, n, d_in, d_out, d_st, e->stream[0]) : act_encode_cbor_dev(e, kind, n, d_in, d_out, e->stream[0]));
+    CK(cudaMemcpyAsync(out, d_out, n * out_rec, cudaMemcpyDeviceToHost, e->stream[0]));
+    if (unpack) CK(cudaMemcpyAsync(status, d_st, n, cudaMemcpyDeviceToHost, e->stream[0]));
+    CK(cudaStreamSynchronize(e->stream[0]));
+    return 0;
 }
 extern "C" int act_unpack_cbor(act_engine* e, int kind, size_t n, const uint8_t* cbor, uint8_t* records, uint8_t* status) {
     if (!e) return fail_msg("null engine");
@@ -1455,17 +1414,11 @@ extern "C" int act_batch_prove_spend_dev(act_engine* e, size_t n, const void* to
     CK(cudaSetDevice(e->device));
     cudaStream_t st = stream ? (cudaStream_t)stream : e->stream[0];
     size_t cap = n < ACT_PROVE_CHUNK ? n : ACT_PROVE_CHUNK;
-    if (e->pv_cap < cap) {
-        CK(cudaStreamSynchronize(st));
-        cudaFree(e->pv_items); cudaFree(e->pv_cpts); cudaFree(e->pv_cvs); cudaFree(e->pv_gammas); cudaFree(e->pv_aux);
-        e->pv_items = e->pv_cpts = e->pv_cvs = e->pv_gammas = e->pv_aux = nullptr; e->pv_cap = 0;
-        CK(cudaMalloc((void**)&e->pv_items, cap * ACT_ITEM_WORDS * 4));
-        CK(cudaMalloc((void**)&e->pv_cpts, cap * ACT_PROVE_PTS * 128));
-        CK(cudaMalloc((void**)&e->pv_cvs, cap * ACT_SPEND_CHUNKS * 32));
-        CK(cudaMalloc((void**)&e->pv_gammas, cap * 32));
-        CK(cudaMalloc((void**)&e->pv_aux, cap * 32));
-        e->pv_cap = cap;
-    }
+    TRY(ensure(e->pv_items, cap * ACT_ITEM_WORDS * 4, st));
+    TRY(ensure(e->pv_cpts, cap * ACT_PROVE_PTS * 128, st));
+    TRY(ensure(e->pv_cvs, cap * ACT_SPEND_CHUNKS * 32, st));
+    TRY(ensure(e->pv_gammas, cap * 32, st));
+    TRY(ensure(e->pv_aux, cap * 32, st));
     int sms = 0;
     CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, e->device));
     for (size_t off = 0; off < n; off += ACT_PROVE_CHUNK) {
@@ -1499,20 +1452,14 @@ extern "C" int act_batch_request(act_engine* e, size_t n, const uint8_t* pre, co
     if (is_multi(e)) return shard_over_replicas(e, n, [&](act_engine* r, size_t lo, size_t m) {
         return act_batch_request(r, m, pre + lo * 64, rnd + lo * 128, req + lo * 128); });
     CK(cudaSetDevice(e->device));
-    u8 *d_pre = nullptr, *d_rnd = nullptr, *d_req = nullptr;
-    int rc = 0;
-    do {
-#define CKB(call) { cudaError_t e_ = (call); if (e_ != cudaSuccess) { rc = fail(#call, e_); break; } }
-        CKB(cudaMalloc((void**)&d_pre, n * 64)); CKB(cudaMalloc((void**)&d_rnd, n * 128)); CKB(cudaMalloc((void**)&d_req, n * 128));
-        CKB(cudaMemcpyAsync(d_pre, pre, n * 64, cudaMemcpyHostToDevice, e->stream[0]));
-        CKB(cudaMemcpyAsync(d_rnd, rnd, n * 128, cudaMemcpyHostToDevice, e->stream[0]));
-        if ((rc = act_batch_request_dev(e, n, d_pre, d_rnd, d_req, e->stream[0]))) break;
-        CKB(cudaMemcpyAsync(req, d_req, n * 128, cudaMemcpyDeviceToHost, e->stream[0]));
-        CKB(cudaStreamSynchronize(e->stream[0]));
-#undef CKB
-    } while (0);
-    cudaFree(d_pre); cudaFree(d_rnd); cudaFree(d_req);
-    return rc;
+    dev_buf<u8> d_pre, d_rnd, d_req;
+    TRY(ensure(d_pre, n * 64)); TRY(ensure(d_rnd, n * 128)); TRY(ensure(d_req, n * 128));
+    CK(cudaMemcpyAsync(d_pre, pre, n * 64, cudaMemcpyHostToDevice, e->stream[0]));
+    CK(cudaMemcpyAsync(d_rnd, rnd, n * 128, cudaMemcpyHostToDevice, e->stream[0]));
+    TRY(act_batch_request_dev(e, n, d_pre, d_rnd, d_req, e->stream[0]));
+    CK(cudaMemcpyAsync(req, d_req, n * 128, cudaMemcpyDeviceToHost, e->stream[0]));
+    CK(cudaStreamSynchronize(e->stream[0]));
+    return 0;
 }
 extern "C" int act_batch_prove_spend(act_engine* e, size_t n, const uint8_t* tokens, const uint8_t* charges, const uint8_t* rnd, const uint8_t seed[32],
                                      uint64_t first_index, uint8_t* proofs, uint8_t* prerefunds, uint8_t* status) {
@@ -1523,24 +1470,18 @@ extern "C" int act_batch_prove_spend(act_engine* e, size_t n, const uint8_t* tok
         return act_batch_prove_spend(r, m, tokens + lo * 160, charges + lo * 32, rnd ? rnd + lo * (size_t)ACT_PROVE_SCALARS * 64 : nullptr, seed, first_index + lo,
                                      proofs + lo * ACT_PROOF_BYTES, prerefunds + lo * 96, status + lo); });
     CK(cudaSetDevice(e->device));
-    u8 *d_tk = nullptr, *d_ch = nullptr, *d_rnd = nullptr, *d_pf = nullptr, *d_pr = nullptr, *d_st = nullptr;
-    int rc = 0;
-    do {
-#define CKB(call) { cudaError_t e_ = (call); if (e_ != cudaSuccess) { rc = fail(#call, e_); break; } }
-        CKB(cudaMalloc((void**)&d_tk, n * 160)); CKB(cudaMalloc((void**)&d_ch, n * 32)); CKB(cudaMalloc((void**)&d_pf, n * ACT_PROOF_BYTES));
-        CKB(cudaMalloc((void**)&d_pr, n * 96)); CKB(cudaMalloc((void**)&d_st, n));
-        if (rnd) { CKB(cudaMalloc((void**)&d_rnd, n * ACT_PROVE_SCALARS * 64)); CKB(cudaMemcpyAsync(d_rnd, rnd, n * ACT_PROVE_SCALARS * 64, cudaMemcpyHostToDevice, e->stream[0])); }
-        CKB(cudaMemcpyAsync(d_tk, tokens, n * 160, cudaMemcpyHostToDevice, e->stream[0]));
-        CKB(cudaMemcpyAsync(d_ch, charges, n * 32, cudaMemcpyHostToDevice, e->stream[0]));
-        if ((rc = act_batch_prove_spend_dev(e, n, d_tk, d_ch, d_rnd, seed, first_index, d_pf, d_pr, d_st, e->stream[0]))) break;
-        CKB(cudaMemcpyAsync(proofs, d_pf, n * ACT_PROOF_BYTES, cudaMemcpyDeviceToHost, e->stream[0]));
-        CKB(cudaMemcpyAsync(prerefunds, d_pr, n * 96, cudaMemcpyDeviceToHost, e->stream[0]));
-        CKB(cudaMemcpyAsync(status, d_st, n, cudaMemcpyDeviceToHost, e->stream[0]));
-        CKB(cudaStreamSynchronize(e->stream[0]));
-#undef CKB
-    } while (0);
-    cudaFree(d_tk); cudaFree(d_ch); cudaFree(d_rnd); cudaFree(d_pf); cudaFree(d_pr); cudaFree(d_st);
-    return rc;
+    dev_buf<u8> d_tk, d_ch, d_rnd, d_pf, d_pr, d_st;
+    TRY(ensure(d_tk, n * 160)); TRY(ensure(d_ch, n * 32)); TRY(ensure(d_pf, n * ACT_PROOF_BYTES));
+    TRY(ensure(d_pr, n * 96)); TRY(ensure(d_st, n));
+    if (rnd) { TRY(ensure(d_rnd, n * ACT_PROVE_SCALARS * 64)); CK(cudaMemcpyAsync(d_rnd, rnd, n * ACT_PROVE_SCALARS * 64, cudaMemcpyHostToDevice, e->stream[0])); }
+    CK(cudaMemcpyAsync(d_tk, tokens, n * 160, cudaMemcpyHostToDevice, e->stream[0]));
+    CK(cudaMemcpyAsync(d_ch, charges, n * 32, cudaMemcpyHostToDevice, e->stream[0]));
+    TRY(act_batch_prove_spend_dev(e, n, d_tk, d_ch, d_rnd, seed, first_index, d_pf, d_pr, d_st, e->stream[0]));
+    CK(cudaMemcpyAsync(proofs, d_pf, n * ACT_PROOF_BYTES, cudaMemcpyDeviceToHost, e->stream[0]));
+    CK(cudaMemcpyAsync(prerefunds, d_pr, n * 96, cudaMemcpyDeviceToHost, e->stream[0]));
+    CK(cudaMemcpyAsync(status, d_st, n, cudaMemcpyDeviceToHost, e->stream[0]));
+    CK(cudaStreamSynchronize(e->stream[0]));
+    return 0;
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -1601,7 +1542,7 @@ extern "C" int act_batch_issue_verify(act_engine* e, size_t n, const uint8_t* re
     if (is_multi(e)) return shard_over_replicas(e, n, [&](act_engine* r, size_t lo, size_t m) { return act_batch_issue_verify(r, m, req + lo * 128, status + lo); });
     host_io h = {{req, nullptr, nullptr}, {128, 0, 0}, {nullptr, nullptr, status}, {0, 0, 1}};
     return run_chunked(e, n, ACT_SMALL_CHUNK, h, [&](int, cudaStream_t st, size_t m, io_slot& io) {
-        issue_mode_kernel<<<nblocks(m, ACT_ISSUE_BLOCK), ACT_ISSUE_BLOCK, 0, st>>>(e->d_ctx, m, (const u32*)io.in0, nullptr, nullptr, nullptr, io.st, ACT_MODE_VERIFY, nullptr);
+        issue_mode_kernel<<<nblocks(m, ACT_ISSUE_BLOCK), ACT_ISSUE_BLOCK, 0, st>>>(e->d_ctx, m, (const u32*)io.in[0].p, nullptr, nullptr, nullptr, io.st, ACT_MODE_VERIFY, nullptr);
         e->launches += 1;
         CK(cudaGetLastError());
         return 0;
@@ -1623,30 +1564,28 @@ extern "C" int act_batch_issue_sign(act_engine* e, size_t n, const uint8_t* req,
     CK(cudaSetDevice(e->device));
     std::vector<u32> idx;
     size_t used = 0;
-    int rc = seq_positions(status, n, idx, rnd_len, &used);
-    if (rc) return rc;
+    TRY(seq_positions(status, n, idx, rnd_len, &used));
     cudaStream_t st = e->stream[0];
-    u8 *d_req = nullptr, *d_c = nullptr, *d_rnd = nullptr, *d_resp = nullptr, *d_st = nullptr; u32* d_idx = nullptr;
-    do {
-#define CKB(call) { cudaError_t e_ = (call); if (e_ != cudaSuccess) { rc = fail(#call, e_); break; } }
-        CKB(cudaMalloc((void**)&d_req, n * 128)); CKB(cudaMalloc((void**)&d_c, n * 32)); CKB(cudaMalloc((void**)&d_resp, n * 160));
-        CKB(cudaMalloc((void**)&d_st, n)); CKB(cudaMalloc((void**)&d_idx, n * 4)); CKB(cudaMalloc((void**)&d_rnd, used ? used : 128));
-        CKB(cudaMemcpyAsync(d_req, req, n * 128, cudaMemcpyHostToDevice, st));
-        CKB(cudaMemcpyAsync(d_c, c, n * 32, cudaMemcpyHostToDevice, st));
-        CKB(cudaMemcpyAsync(d_st, status, n, cudaMemcpyHostToDevice, st));
-        CKB(cudaMemcpyAsync(d_idx, idx.data(), n * 4, cudaMemcpyHostToDevice, st));
-        if (used) CKB(cudaMemcpyAsync(d_rnd, rnd, used, cudaMemcpyHostToDevice, st));
-        issue_mode_kernel<<<nblocks(n, ACT_ISSUE_BLOCK), ACT_ISSUE_BLOCK, 0, st>>>(e->d_ctx, n, (const u32*)d_req, (const u32*)d_c, (const u32*)d_rnd, (u32*)d_resp, d_st, ACT_MODE_SIGN, d_idx);
-        e->launches += 1;
-        CKB(cudaGetLastError());
-        CKB(cudaMemcpyAsync(resp, d_resp, n * 160, cudaMemcpyDeviceToHost, st));
-        CKB(cudaMemsetAsync(d_rnd, 0, used ? used : 128, st));     // the device copy of the signer randomness
-        if (scrub_after_signing(e, st, -1)) { rc = -2; break; }
-        CKB(cudaStreamSynchronize(st));
-#undef CKB
-    } while (0);
-    cudaFree(d_req); cudaFree(d_c); cudaFree(d_rnd); cudaFree(d_resp); cudaFree(d_st); cudaFree(d_idx);
-    return rc;
+    size_t rnd_bytes = used ? used : 128;
+    dev_buf<u8> d_req, d_c, d_rnd, d_resp, d_st; dev_buf<u32> d_idx;
+    wipe_dev_on_exit rnd_wipe{nullptr, rnd_bytes, st};   // the device copy of the signer randomness, if a step below fails
+    TRY(ensure(d_req, n * 128)); TRY(ensure(d_c, n * 32)); TRY(ensure(d_resp, n * 160));
+    TRY(ensure(d_st, n)); TRY(ensure(d_idx, n * 4)); TRY(ensure(d_rnd, rnd_bytes));
+    rnd_wipe.p = d_rnd;
+    CK(cudaMemcpyAsync(d_req, req, n * 128, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(d_c, c, n * 32, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(d_st, status, n, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(d_idx, idx.data(), n * 4, cudaMemcpyHostToDevice, st));
+    if (used) CK(cudaMemcpyAsync(d_rnd, rnd, used, cudaMemcpyHostToDevice, st));
+    issue_mode_kernel<<<nblocks(n, ACT_ISSUE_BLOCK), ACT_ISSUE_BLOCK, 0, st>>>(e->d_ctx, n, (const u32*)d_req.p, (const u32*)d_c.p, (const u32*)d_rnd.p, (u32*)d_resp.p, d_st, ACT_MODE_SIGN, d_idx);
+    e->launches += 1;
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(resp, d_resp, n * 160, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemsetAsync(d_rnd, 0, rnd_bytes, st));     // the device copy of the signer randomness
+    rnd_wipe.p = nullptr;
+    TRY(scrub_after_signing(e, st, -1));
+    CK(cudaStreamSynchronize(st));
+    return 0;
 }
 extern "C" int act_batch_spend_verify(act_engine* e, size_t n, const uint8_t* proofs, uint8_t* nullifiers, uint8_t* status, uint8_t* kprime) {
     if (!e) return fail_msg("null engine");
@@ -1654,16 +1593,11 @@ extern "C" int act_batch_spend_verify(act_engine* e, size_t n, const uint8_t* pr
     if (!proofs || !nullifiers || !status || !kprime) return fail_msg("act_batch_spend_verify: null buffer");
     if (is_multi(e)) return shard_over_replicas(e, n, [&](act_engine* r, size_t lo, size_t m) {
         return act_batch_spend_verify(r, m, proofs + lo * ACT_PROOF_BYTES, nullifiers + lo * 32, status + lo, kprime + lo * 128); });
-    {
-        CK(cudaSetDevice(e->device));
-        size_t cap = n < e->spend_chunk ? n : e->spend_chunk;
-        int rc = ensure_scratch(&e->scratch[0], cap);
-        if (!rc && n > e->spend_chunk) rc = ensure_scratch(&e->scratch[1], cap);
-        if (rc) return rc;
-    }
+    CK(cudaSetDevice(e->device));
+    TRY(ensure_spend_scratch(e, n));
     host_io h = {{proofs, nullptr, nullptr}, {ACT_PROOF_BYTES, 0, 0}, {kprime, nullifiers, status}, {128, 32, 1}};
     return run_chunked(e, n, e->spend_chunk, h, [&](int s, cudaStream_t st, size_t m, io_slot& io) {
-        return spend_chunk_launch(e, &e->scratch[s], st, m, (const u32*)io.in0, nullptr, nullptr, (u32*)io.out1, io.st, (u32*)io.out0);
+        return spend_chunk_launch(e, &e->scratch[s], st, m, (const u32*)io.in[0].p, nullptr, nullptr, (u32*)io.out[1].p, io.st, (u32*)io.out[0].p);
     }, true);
 }
 extern "C" int act_batch_refund_sign(act_engine* e, size_t n, const uint8_t* kprime, const uint8_t* status, const uint8_t* rnd, size_t rnd_len, uint8_t* refunds) {
@@ -1681,29 +1615,27 @@ extern "C" int act_batch_refund_sign(act_engine* e, size_t n, const uint8_t* kpr
     CK(cudaSetDevice(e->device));
     std::vector<u32> idx;
     size_t used = 0;
-    int rc = seq_positions(status, n, idx, rnd_len, &used);
-    if (rc) return rc;
+    TRY(seq_positions(status, n, idx, rnd_len, &used));
     cudaStream_t st = e->stream[0];
-    u8 *d_kp = nullptr, *d_rnd = nullptr, *d_ref = nullptr, *d_st = nullptr; u32* d_idx = nullptr;
-    do {
-#define CKB(call) { cudaError_t e_ = (call); if (e_ != cudaSuccess) { rc = fail(#call, e_); break; } }
-        CKB(cudaMalloc((void**)&d_kp, n * 128)); CKB(cudaMalloc((void**)&d_ref, n * 128)); CKB(cudaMalloc((void**)&d_st, n));
-        CKB(cudaMalloc((void**)&d_idx, n * 4)); CKB(cudaMalloc((void**)&d_rnd, used ? used : 128));
-        CKB(cudaMemcpyAsync(d_kp, kprime, n * 128, cudaMemcpyHostToDevice, st));
-        CKB(cudaMemcpyAsync(d_st, status, n, cudaMemcpyHostToDevice, st));
-        CKB(cudaMemcpyAsync(d_idx, idx.data(), n * 4, cudaMemcpyHostToDevice, st));
-        if (used) CKB(cudaMemcpyAsync(d_rnd, rnd, used, cudaMemcpyHostToDevice, st));
-        refund_sign_seq_kernel<<<nblocks(n, ACT_SIGN_BLOCK), ACT_SIGN_BLOCK, 0, st>>>(e->d_ctx, n, nullptr, (const u32*)d_rnd, (const u32*)d_kp, d_st, (u32*)d_ref, nullptr, d_idx, nullptr);
-        e->launches += 1;
-        CKB(cudaGetLastError());
-        CKB(cudaMemcpyAsync(refunds, d_ref, n * 128, cudaMemcpyDeviceToHost, st));
-        CKB(cudaMemsetAsync(d_rnd, 0, used ? used : 128, st));
-        if (scrub_after_signing(e, st, -1)) { rc = -2; break; }
-        CKB(cudaStreamSynchronize(st));
-#undef CKB
-    } while (0);
-    cudaFree(d_kp); cudaFree(d_rnd); cudaFree(d_ref); cudaFree(d_st); cudaFree(d_idx);
-    return rc;
+    size_t rnd_bytes = used ? used : 128;
+    dev_buf<u8> d_kp, d_rnd, d_ref, d_st; dev_buf<u32> d_idx;
+    wipe_dev_on_exit rnd_wipe{nullptr, rnd_bytes, st};   // the device copy of the signer randomness, if a step below fails
+    TRY(ensure(d_kp, n * 128)); TRY(ensure(d_ref, n * 128)); TRY(ensure(d_st, n));
+    TRY(ensure(d_idx, n * 4)); TRY(ensure(d_rnd, rnd_bytes));
+    rnd_wipe.p = d_rnd;
+    CK(cudaMemcpyAsync(d_kp, kprime, n * 128, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(d_st, status, n, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(d_idx, idx.data(), n * 4, cudaMemcpyHostToDevice, st));
+    if (used) CK(cudaMemcpyAsync(d_rnd, rnd, used, cudaMemcpyHostToDevice, st));
+    refund_sign_seq_kernel<<<nblocks(n, ACT_SIGN_BLOCK), ACT_SIGN_BLOCK, 0, st>>>(e->d_ctx, n, nullptr, (const u32*)d_rnd.p, (const u32*)d_kp.p, d_st, (u32*)d_ref.p, nullptr, d_idx, nullptr);
+    e->launches += 1;
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(refunds, d_ref, n * 128, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemsetAsync(d_rnd, 0, rnd_bytes, st));
+    rnd_wipe.p = nullptr;
+    TRY(scrub_after_signing(e, st, -1));
+    CK(cudaStreamSynchronize(st));
+    return 0;
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -1749,13 +1681,9 @@ extern "C" int act_batch_verify_spend_and_refund_seq(act_engine* e, size_t n, co
 // never calls refund() for it); its nullifier is kept so that the caller can tell which token was replayed.
 // ---------------------------------------------------------------------------------------------------
 static int ensure_gather(act_engine* r, size_t m) {
-    if (r->g_cap >= m) return 0;
     CK(cudaSetDevice(r->device));
-    cudaFree(r->g_st); cudaFree(r->g_nul);
-    r->g_st = r->g_nul = nullptr; r->g_cap = 0;
-    CK(cudaMalloc((void**)&r->g_st, m + 16));
-    CK(cudaMalloc((void**)&r->g_nul, m * 32 + 16));
-    r->g_cap = m;
+    TRY(ensure(r->g_st, m + 16));
+    TRY(ensure(r->g_nul, m * 32 + 16));
     return 0;
 }
 // the screen runs against `seen` (n_seen keys, host memory) when store is null, else against the store, recording the survivors
@@ -1765,9 +1693,8 @@ static int verify_refund_and_screen(act_engine* e, size_t n, const uint8_t* proo
     if (store && store->device != reps[0]->device)
         return fail_msg("act_batch_verify_spend_and_refund_recorded: the store must be on the device of replica 0 (where the gather lands)");
     size_t G = reps.size();
-    int rc = 0;
-    for (size_t g = 0; g < G && !rc; g++) rc = ensure_gather(reps[g], shard_lo(n, g + 1, G) - shard_lo(n, g, G));
-    if (rc) return rc;
+    for (size_t g = 0; g < G; g++) TRY(ensure_gather(reps[g], shard_lo(n, g + 1, G) - shard_lo(n, g, G)));
+    int rc;
     for (auto* r : reps) r->g_keep = true;
     if (G == 1) rc = act_batch_verify_spend_and_refund(reps[0], n, proofs, rnd, refunds, nullifiers, status);
     else {
@@ -1779,32 +1706,24 @@ static int verify_refund_and_screen(act_engine* e, size_t n, const uint8_t* proo
     act_engine* r0 = reps[0];
     CK(cudaSetDevice(r0->device));
     cudaStream_t st = r0->stream[0];
-    u8 *d_st = nullptr, *d_nul = nullptr, *d_seen = nullptr, *d_out = nullptr;
-    do {
-#define CKB(call) { cudaError_t e_ = (call); if (e_ != cudaSuccess) { rc = fail(#call, e_); break; } }
-        if (G > 1) {
-            CKB(cudaMalloc((void**)&d_st, n)); CKB(cudaMalloc((void**)&d_nul, n * 32));
-            for (size_t g = 0; g < G && !rc; g++) {
-                size_t lo = shard_lo(n, g, G), m = shard_lo(n, g + 1, G) - lo;
-                if (!m) continue;
-                CKB(cudaMemcpyPeerAsync(d_st + lo, r0->device, reps[g]->g_st, reps[g]->device, m, st));
-                CKB(cudaMemcpyPeerAsync(d_nul + lo * 32, r0->device, reps[g]->g_nul, reps[g]->device, m * 32, st));
-            }
-            if (rc) break;
+    dev_buf<u8> d_st, d_nul, d_seen, d_out;
+    if (G > 1) {
+        TRY(ensure(d_st, n)); TRY(ensure(d_nul, n * 32));
+        for (size_t g = 0; g < G; g++) {
+            size_t lo = shard_lo(n, g, G), m = shard_lo(n, g + 1, G) - lo;
+            if (!m) continue;
+            CK(cudaMemcpyPeerAsync(d_st.p + lo, r0->device, reps[g]->g_st, reps[g]->device, m, st));
+            CK(cudaMemcpyPeerAsync(d_nul.p + lo * 32, r0->device, reps[g]->g_nul, reps[g]->device, m * 32, st));
         }
-        CKB(cudaMalloc((void**)&d_out, n));
-        if (n_seen) { CKB(cudaMalloc((void**)&d_seen, n_seen * 32)); CKB(cudaMemcpyAsync(d_seen, seen, n_seen * 32, cudaMemcpyHostToDevice, st)); }
-        const u8* g_st = G > 1 ? d_st : r0->g_st;
-        const u8* g_nul = G > 1 ? d_nul : r0->g_nul;
-        if (store) rc = act_nullifier_store_screen_dev(store, n, g_st, g_nul, d_out, 1, st);
-        else rc = act_flag_replays_dev(r0, n, g_st, g_nul, n_seen, d_seen, d_out, st);
-        if (rc) break;
-        CKB(cudaMemcpyAsync(status, d_out, n, cudaMemcpyDeviceToHost, st));
-        CKB(cudaStreamSynchronize(st));
-#undef CKB
-    } while (0);
-    cudaFree(d_st); cudaFree(d_nul); cudaFree(d_seen); cudaFree(d_out);
-    if (rc) return rc;
+    }
+    TRY(ensure(d_out, n));
+    if (n_seen) { TRY(ensure(d_seen, n_seen * 32)); CK(cudaMemcpyAsync(d_seen, seen, n_seen * 32, cudaMemcpyHostToDevice, st)); }
+    const u8* g_st = G > 1 ? d_st.p : r0->g_st.p;
+    const u8* g_nul = G > 1 ? d_nul.p : r0->g_nul.p;
+    if (store) TRY(act_nullifier_store_screen_dev(store, n, g_st, g_nul, d_out, 1, st));
+    else TRY(act_flag_replays_dev(r0, n, g_st, g_nul, n_seen, d_seen, d_out, st));
+    CK(cudaMemcpyAsync(status, d_out, n, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
     for (size_t i = 0; i < n; i++) if (status[i] == 3) memset(refunds + i * 128, 0, 128);
     return 0;
 }
