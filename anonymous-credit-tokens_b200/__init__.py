@@ -34,6 +34,7 @@ NOT_CANONICAL = 0xFF
 TOKEN_BYTES = 160
 PREREFUND_BYTES = 96
 PROVE_RND_BYTES = 524 * 64
+KEY_SLOTS = 16
 
 # status codes (include/act_engine.h; 1 + discriminant of the reference's `Error`, src/lib.rs:102-112)
 OK = 0
@@ -77,6 +78,8 @@ EXPORTED_SYMBOLS = [
     "act_nullifier_store_create", "act_nullifier_store_destroy", "act_nullifier_store_device", "act_nullifier_store_size",
     "act_nullifier_store_screen_dev", "act_nullifier_store_screen", "act_nullifier_store_export",
     "act_batch_verify_spend_and_refund_recorded",
+    "act_engine_set_key", "act_engine_clear_key", "act_engine_select_key", "act_engine_selected_key", "act_engine_key_slots",
+    "act_batch_verify_spend_and_refund_keyed_dev", "act_batch_verify_spend_and_refund_keyed", "act_batch_spend_verify_keyed",
 ]
 
 
@@ -152,6 +155,15 @@ def load_library():
     lib.act_nullifier_store_screen.argtypes = [vp, sz, vp, vp, vp, i32]; lib.act_nullifier_store_screen.restype = i32
     lib.act_nullifier_store_export.argtypes = [vp, vp, sz, C.POINTER(sz)]; lib.act_nullifier_store_export.restype = i32
     lib.act_batch_verify_spend_and_refund_recorded.argtypes = [vp, vp, sz, vp, vp, vp, vp, vp]; lib.act_batch_verify_spend_and_refund_recorded.restype = i32
+    lib.act_engine_set_key.argtypes = [vp, i32, vp, vp]; lib.act_engine_set_key.restype = i32
+    lib.act_engine_clear_key.argtypes = [vp, i32]; lib.act_engine_clear_key.restype = i32
+    lib.act_engine_select_key.argtypes = [vp, i32]; lib.act_engine_select_key.restype = i32
+    lib.act_engine_selected_key.argtypes = [vp]; lib.act_engine_selected_key.restype = i32
+    lib.act_engine_key_slots.argtypes = [vp]; lib.act_engine_key_slots.restype = C.c_uint32
+    lib.act_batch_verify_spend_and_refund_keyed_dev.argtypes = [vp, sz, vp, vp, vp, vp, vp, vp, vp]
+    lib.act_batch_verify_spend_and_refund_keyed_dev.restype = i32
+    lib.act_batch_verify_spend_and_refund_keyed.argtypes = [vp, sz, vp, vp, vp, vp, vp, vp, vp]; lib.act_batch_verify_spend_and_refund_keyed.restype = i32
+    lib.act_batch_spend_verify_keyed.argtypes = [vp, sz, vp, vp, vp, vp, vp]; lib.act_batch_spend_verify_keyed.restype = i32
     _lib = lib
     return lib
 
@@ -403,6 +415,67 @@ class Engine:
         _check(self.lib.act_batch_verify_spend_and_refund_recorded(self._h, store._h, n, pf.ctypes.data, r.ctypes.data, ref.ctypes.data, nul.ctypes.data,
                                                                    st.ctypes.data), "act_batch_verify_spend_and_refund_recorded")
         return ref, nul, st
+
+    # ---- issuer key slots (key rotation) ----
+    def set_key(self, slot, key):
+        """Installs or replaces the PrivateKey of a slot (0 .. KEY_SLOTS-1); fails, leaving the slot as it was, if key.w != G*key.x."""
+        xb, wb = _u8(key.x, 32, "x"), _u8(key.w, 32, "w")
+        _check(self.lib.act_engine_set_key(self._h, slot, xb.ctypes.data, wb.ctypes.data), "act_engine_set_key")
+
+    def clear_key(self, slot):
+        """Wipes the slot's secret and frees its tables; the selected slot cannot be cleared."""
+        _check(self.lib.act_engine_clear_key(self._h, slot), "act_engine_clear_key")
+
+    def select_key(self, slot):
+        """The key every single-key call (issue, refund signing, verification, client-side checks) uses from now on."""
+        _check(self.lib.act_engine_select_key(self._h, slot), "act_engine_select_key")
+
+    @property
+    def selected_key(self):
+        return int(self.lib.act_engine_selected_key(self._h))
+
+    @property
+    def key_slots(self):
+        """The slots that hold a key, ascending."""
+        m = int(self.lib.act_engine_key_slots(self._h))
+        return [s for s in range(KEY_SLOTS) if m >> s & 1]
+
+    def batch_verify_spend_and_refund_keyed(self, proofs, key_ids, rnd, stores=None, out=None):
+        """Proof i is verified under the key of slot key_ids[i] and refunded under the selected key; an empty or out-of-range slot
+        gives status 7.  stores: None (no screen), or a NullifierStore per slot that holds a key (a sequence indexed by slot, or a
+        dict {slot: store}; slots may share one): each store screens and records the proofs of its slots, as the _recorded call
+        does for one.  Returns (refunds, nullifiers, status)."""
+        pf = _u8(proofs); n = pf.size // PROOF_BYTES
+        ids, r = _u8(key_ids, n, "key_ids"), _u8(rnd, n * RND_BYTES, "rnd")
+        if out is None:
+            ref = np.zeros(n * REFUND_BYTES, np.uint8); nul = np.zeros(n * 32, np.uint8); st = np.zeros(n, np.uint8)
+        else:
+            ref, nul, st = out
+        table = None
+        if stores is not None:
+            items = stores.items() if isinstance(stores, dict) else enumerate(stores)
+            table = (C.c_void_p * KEY_SLOTS)()
+            for slot, store in items:
+                if store is not None:
+                    table[slot] = store._h.value
+        _check(self.lib.act_batch_verify_spend_and_refund_keyed(self._h, n, pf.ctypes.data, ids.ctypes.data, r.ctypes.data,
+                                                                C.cast(table, C.c_void_p) if table is not None else None,
+                                                                ref.ctypes.data, nul.ctypes.data, st.ctypes.data),
+               "act_batch_verify_spend_and_refund_keyed")
+        return ref, nul, st
+
+    def batch_spend_verify_keyed(self, proofs, key_ids):
+        """-> (nullifiers, status, kprime): the verification pass of the keyed call; sign with batch_refund_sign (selected key)."""
+        pf = _u8(proofs); n = pf.size // PROOF_BYTES
+        ids = _u8(key_ids, n, "key_ids")
+        nul = np.zeros(n * 32, np.uint8); st = np.zeros(n, np.uint8); kp = np.zeros(n * 128, np.uint8)
+        _check(self.lib.act_batch_spend_verify_keyed(self._h, n, pf.ctypes.data, ids.ctypes.data, nul.ctypes.data, st.ctypes.data, kp.ctypes.data),
+               "act_batch_spend_verify_keyed")
+        return nul, st, kp
+
+    def batch_verify_spend_and_refund_keyed_dev(self, n, proofs, key_ids, rnd, refunds, nullifiers, status, stream=0):
+        _check(self.lib.act_batch_verify_spend_and_refund_keyed_dev(self._h, n, proofs, key_ids, rnd, refunds, nullifiers, status, stream),
+               "act_batch_verify_spend_and_refund_keyed_dev")
 
     def batch_verify_spend_and_refund_screened_ptr(self, n, proofs, rnd, n_seen, seen, refunds, nullifiers, status):
         _check(self.lib.act_batch_verify_spend_and_refund_screened(self._h, n, proofs, rnd, n_seen, seen, refunds, nullifiers, status),

@@ -156,4 +156,23 @@ __global__ void __launch_bounds__(256) replay_resolve_kernel(u32 n, u32 n_seen, 
     }
     out[i] = st;
 }
+
+// ---- per-store screen of a keyed batch: key id -> store index through a map of ACT_KEY_SLOTS bytes (0xFF = no store) ----
+#ifndef ACT_KEY_SLOTS
+#define ACT_KEY_SLOTS 16
+#endif
+struct act_store_map { u8 of_slot[ACT_KEY_SLOTS]; };
+__device__ __forceinline__ u32 store_of(const act_store_map& m, u8 key_id) { return key_id < ACT_KEY_SLOTS ? m.of_slot[key_id] : 0xFFu; }
+// the statuses store j screens: the proofs of other stores (and of no store) get a nonzero status, so they take no part
+__global__ void __launch_bounds__(256) store_mask_kernel(size_t n, const u8* __restrict__ status, const u8* __restrict__ key_ids, act_store_map m, u32 j,
+                                                         u8* __restrict__ out) {
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) out[i] = store_of(m, key_ids[i]) == j ? status[i] : (u8)0xFF;
+}
+// store j's outcomes back into the batch's statuses
+__global__ void __launch_bounds__(256) store_merge_kernel(size_t n, const u8* __restrict__ screened, const u8* __restrict__ key_ids, act_store_map m, u32 j,
+                                                          u8* __restrict__ status) {
+    size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n && store_of(m, key_ids[i]) == j) status[i] = screened[i];
+}
 #endif

@@ -28,6 +28,12 @@
 #define ACT_FLAG_BAD_POINT 1u
 #define ACT_FLAG_IDENTITY 2u
 #define ACT_FLAG_BAD_PROOF 4u
+#define ACT_FLAG_NO_KEY 8u          // keyed verification: the proof's key id names no key (finish: status 7)
+
+// issuer key slots of an engine (include/act_engine.h); a keyed spend names one per proof
+#ifndef ACT_KEY_SLOTS
+#define ACT_KEY_SLOTS 16
+#endif
 
 // ---- layout constants -----------------------------------------------------------------------------
 #define ACT_L 128
@@ -769,9 +775,14 @@ ACT_FN void spend_encode_thread(const act_ctx* C, size_t p, int part, const u32*
 // =============================================================================================================
 // spend verification, stage 2: one thread per proof.  A-bar (secret x), A1, A2, K' (Horner), C
 // (src/lib.rs:787-799, 819-829).  Writes items 0..4 and 389, K' for the signing tail; completes C'_00, C'_01 in cpts.
+// KEYED: the secret of the A1 term is the x of slots[key_ids[p]] (ACT_KEY_SLOTS entries, null = empty slot) instead of C's.
+// An empty or out-of-range id raises ACT_FLAG_NO_KEY and the proof runs on with C's x, so that every proof takes the same
+// path; its result is discarded.  The key id is public: the load it selects depends on public data only.
 // =============================================================================================================
+template <bool KEYED = false>
 ACT_FN void spend_head_thread(const act_ctx* C, size_t p, const u32* proofs, u32* items, const u32* com_niels, u32* kprime, u32* flags,
-                              u32* cpts /* halves of stage 1: the two of j = 0 get their h2 terms here, BEFORE the encode stage */) {
+                              u32* cpts /* halves of stage 1: the two of j = 0 get their h2 terms here, BEFORE the encode stage */,
+                              const u8* key_ids = nullptr, const act_ctx* const* slots = nullptr) {
     const u32* pf = proofs + (size_t)ACT_PROOF_WORDS * p;
     u32* it = items + (size_t)ACT_ITEM_WORDS * p;
     ACT_NOUNROLL for (int b = 0; b < 2; b++) {   // C'_00 += h2*w00, C'_01 += h2*w01 (as halves)            (:806,808)
@@ -788,6 +799,13 @@ ACT_FN void spend_head_thread(const act_ctx* C, size_t p, const u32* proofs, u32
     u32 fl = 0;
     if (!valid) fl |= ACT_FLAG_BAD_POINT;
     if (ristretto_is_identity(Ap)) fl |= ACT_FLAG_IDENTITY;                                // (:787-789)
+    const act_ctx* K = C;   // whose secret the A1 term uses
+    if (KEYED) {
+        u32 id = key_ids[p];
+        const act_ctx* named = id < ACT_KEY_SLOTS ? slots[id] : nullptr;
+        if (named) K = named;
+        else fl |= ACT_FLAG_NO_KEY;
+    }
     if (fl) ACT_ATOMIC_OR(&flags[p], fl);
     sc k = load_scalar(pf), s = load_scalar(pf + 8), gamma = load_scalar(pf + 8 * 132);
     sc e_bar = load_scalar(pf + 8 * 133), r2_bar = load_scalar(pf + 8 * 134), r3_bar = load_scalar(pf + 8 * 135);
@@ -801,7 +819,7 @@ ACT_FN void spend_head_thread(const act_ctx* C, size_t p, const u32* proofs, u32
         //    = A'*(e_bar - x*gamma) + B*r2_bar: Abar is never formed (it is not hashed); the scalar on A' depends on the
         //    secret x, so that term scans its table in full, the B term (public scalar) indexes directly.  One doubling chain.
         vb_table_build(&t[0], Ap); vb_table_build(&t[1], Bb);
-        sc sa = sc_bias<4>(sc_sub(e_bar, sc_mul(C->x, gamma))), sb = sc_bias<4>(r2_bar);
+        sc sa = sc_bias<4>(sc_sub(e_bar, sc_mul(K->x, gamma))), sb = sc_bias<4>(r2_bar);
         ge A1 = ge_identity();
         ACT_NOUNROLL for (int i = 63; i >= 0; i--) {
             if (i != 63) {
@@ -896,7 +914,7 @@ ACT_FN void spend_finish_thread(const act_ctx* C, size_t p, const u32* proofs, c
     u32 st = ACT_ST_OK;
     if (fl & ACT_FLAG_BAD_POINT) st = ACT_ST_DECODE_INVALID_POINT;
     else if (fl & ACT_FLAG_IDENTITY) st = ACT_ST_IDENTITY_POINT;
-    else if (!sc_eq(g2, gamma)) st = ACT_ST_INVALID_CLIENT_SPEND_PROOF;                    // (:842-844)
+    else if ((fl & ACT_FLAG_NO_KEY) || !sc_eq(g2, gamma)) st = ACT_ST_INVALID_CLIENT_SPEND_PROOF;   // (:842-844); no key: as a failed check
     status[p] = (u8)st;
 }
 

@@ -1,7 +1,7 @@
 // act_engine.cu -- CUDA kernels (sm_100a) and the C-ABI engine of include/act_engine.h.
 //
-// One engine = one (Params, PrivateKey) pair on one GPU: generator tables, the secret scalar, two
-// CUDA streams and the scratch buffers of the spend pipeline.  Batches are processed in chunks; the
+// One engine = one Params on one GPU with up to ACT_KEY_SLOTS issuer keys (one of them selected): generator tables, the secret
+// scalars, two CUDA streams and the scratch buffers of the spend pipeline.  Batches are processed in chunks; the
 // host-buffer entry points double-buffer H2D / compute / D2H across the two streams.
 //
 // There is no CPU path: every entry point needs a CUDA device and fails otherwise.
@@ -164,6 +164,12 @@ __global__ void __launch_bounds__(ACT_ISSUE_BLOCK, ACT_ISSUE_BPS) request_kernel
 __global__ void __launch_bounds__(ACT_HEAD_BLOCK, ACT_HEAD_BPS) spend_head_kernel(const act_ctx* C, size_t n, const u32* proofs, u32* items, const u32* com_niels, u32* kprime, u32* flags, u32* cpts) {
     size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (p < n) spend_head_thread(C, p, proofs, items, com_niels, kprime, flags, cpts);
+}
+// the keyed form: proof p is verified under the key of slot key_ids[p] (slots: ACT_KEY_SLOTS contexts, null = empty)
+__global__ void __launch_bounds__(ACT_HEAD_BLOCK, ACT_HEAD_BPS) spend_head_keyed_kernel(const act_ctx* C, size_t n, const u32* proofs, u32* items, const u32* com_niels, u32* kprime,
+                                                                                     u32* flags, u32* cpts, const u8* key_ids, const act_ctx* const* slots) {
+    size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (p < n) spend_head_thread<true>(C, p, proofs, items, com_niels, kprime, flags, cpts, key_ids, slots);
 }
 __global__ void __launch_bounds__(ACT_HASH_BLOCK) spend_chunk_kernel(const act_ctx* C, size_t n, const u32* items, u32* cvs) {
     size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -434,12 +440,22 @@ struct io_slot {  // device staging for the host-buffer entry points, indexed li
     dev_buf<u8> in[3], out[2], st;
 };
 
+// One issuer key: its device context -- the shared tables of the engine, its own x, W, W/2 and W table -- and that W table.
+// The creation key's W table lies in the engine's d_tables; a key installed later has one of its own (2^13 wide, 7.9 MB).
+struct key_slot {
+    dev_buf<act_ctx> ctx;
+    dev_buf<ge_niels> w_table;
+};
+
 #define ACT_IO_SLOTS 3
 struct act_engine {
     int device = 0;
     cudaStream_t stream[2] = {nullptr, nullptr};
     cudaEvent_t fork = nullptr, join[2] = {nullptr, nullptr};
-    dev_buf<act_ctx> d_ctx;
+    key_slot key[ACT_KEY_SLOTS];      // slot 0 holds the creation key
+    int selected = 0;                 // the slot every single-key entry point uses
+    dev_buf<const act_ctx*> d_slots;  // ctx of every slot, null when empty: what the keyed head reads
+    act_ctx pub;                      // host template of a slot's context: table pointers, H encodings, prefixes; no key
     dev_buf<ge_niels> d_tables;
     dev_buf<ge> d_bases;
     spend_scratch scratch[2];
@@ -466,6 +482,7 @@ struct act_engine {
     std::vector<timed> events;
 };
 static inline bool is_multi(const act_engine* e) { return !e->replicas.empty(); }
+static inline act_ctx* sel_ctx(const act_engine* e) { return e->key[e->selected].ctx; }
 #define NOT_MULTI(e, what) do { if (is_multi(e)) return fail_msg(what ": device-buffer calls need a single-device engine (act_engine_replica)"); } while (0)
 // call(replica, first index of its shard, shard length) on every replica, each from its own host thread: contiguous shards
 // (bounds of sharding.shard_bounds), no cross-GPU arithmetic (SURVEY 8e)
@@ -607,7 +624,7 @@ extern "C" void act_engine_destroy(act_engine* e) {
             scrub_local_kernel<<<sms * 2, 1024, 0, e->stream[0]>>>(nullptr);
         cudaStreamSynchronize(e->stream[0]);
     }
-    if (e->d_ctx.p) cudaMemset(e->d_ctx, 0, sizeof(act_ctx));  // zeroise x on the device
+    for (key_slot& k : e->key) if (k.ctx.p) cudaMemset(k.ctx, 0, sizeof(act_ctx));  // zeroise every x on the device
     if (e->fork) cudaEventDestroy(e->fork);
     for (int s = 0; s < 2; s++) if (e->join[s]) cudaEventDestroy(e->join[s]);
     for (int s = 0; s < 2; s++) {
@@ -622,6 +639,13 @@ extern "C" void act_engine_destroy(act_engine* e) {
     delete e;   // frees every device buffer
 }
 
+// the slot table the keyed head reads; the device has no work in flight that reads it (callers synchronise first)
+static int upload_slots(act_engine* e) {
+    const act_ctx* h[ACT_KEY_SLOTS];
+    for (int k = 0; k < ACT_KEY_SLOTS; k++) h[k] = e->key[k].ctx;
+    CK(cudaMemcpy(e->d_slots, h, sizeof h, cudaMemcpyHostToDevice));
+    return 0;
+}
 // streams, events, tables and the device context of a new engine; the caller destroys e if this fails
 static int engine_init(act_engine* e, const uint8_t h[96], const uint8_t sk_x[32], const uint8_t pk_w[32]) {
     CK(cudaStreamCreateWithFlags(&e->stream[0], cudaStreamNonBlocking));
@@ -634,7 +658,7 @@ static int engine_init(act_engine* e, const uint8_t h[96], const uint8_t sk_x[32
     CK(cudaEventCreateWithFlags(&e->fork, cudaEventDisableTiming));
     CK(cudaEventCreateWithFlags(&e->join[0], cudaEventDisableTiming));
     CK(cudaEventCreateWithFlags(&e->join[1], cudaEventDisableTiming));
-    TRY(ensure(e->d_ctx, sizeof(act_ctx)));
+    TRY(ensure(e->key[0].ctx, sizeof(act_ctx)));
     // replay-screen PRF key
     if (!os_random(&e->rp_key, sizeof e->rp_key)) return fail_msg("act_engine_create: the OS random source (getrandom) failed");
     size_t fb_entries = 0;
@@ -666,17 +690,20 @@ static int engine_init(act_engine* e, const uint8_t h[96], const uint8_t sk_x[32
     build_prefix(&hc, ACT_TR_RESPOND, "respond", h);
     build_prefix(&hc, ACT_TR_REFUND, "refund", h);
     build_prefix(&hc, ACT_TR_SPEND, "spend", h);
+    e->pub = hc;   // before any key material enters hc
+    e->pub.fb[ACT_BASE_W] = fb_tab{};
     CK(cudaMemcpy(&hc.W, d_W, sizeof(ge), cudaMemcpyDeviceToHost));
     // raw key words; finalize_ctx_kernel reduces them mod l on the device
     memcpy(hc.x.v, sk_x, 32);
-    CK(cudaMemcpy(e->d_ctx, &hc, sizeof hc, cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(e->key[0].ctx, &hc, sizeof hc, cudaMemcpyHostToDevice));
     explicit_bzero(&hc, sizeof hc);
-    finalize_ctx_kernel<<<1, 1>>>(e->d_ctx, d_enc.p + 24, d_ok);
+    finalize_ctx_kernel<<<1, 1>>>(e->key[0].ctx, d_enc.p + 24, d_ok);
     CK(cudaGetLastError());
     CK(cudaDeviceSynchronize());
     CK(cudaMemcpy(&ok, d_ok, 4, cudaMemcpyDeviceToHost));
     if (!ok) return fail_msg("act_engine_create: pk_w is not the public key of sk_x (W != G*x)");
-    return 0;
+    TRY(ensure(e->d_slots, sizeof(const act_ctx*) * ACT_KEY_SLOTS));
+    return upload_slots(e);
 }
 extern "C" int act_engine_create(act_engine** out, int device, const uint8_t h[96], const uint8_t sk_x[32], const uint8_t pk_w[32]) {
     if (!out || !h || !sk_x || !pk_w) return fail_msg("act_engine_create: null argument");
@@ -733,6 +760,99 @@ extern "C" int act_public_key(int device, const uint8_t sk_x[32], uint8_t pk_w[3
     CK(cudaMemcpy(pk_w, d_o, 32, cudaMemcpyDeviceToHost));
     return 0;
 }
+
+// ---------------------------------------------------------------------------------------------------
+// issuer key slots: every slot shares the engine's Params, tables and scratch and holds its own x, W and W table
+// ---------------------------------------------------------------------------------------------------
+// a one-base layout of build_fb_tables_kernel: the W table alone, 2^ACT_FB_BITS wide
+static fb_layout w_layout() {
+    fb_layout L;
+    memset(&L, 0, sizeof L);
+    L.bits[0] = ACT_FB_BITS;
+    u32 threads = fb_win_of(ACT_FB_BITS) * fb_parts_of(ACT_FB_BITS);
+    for (int b = 1; b <= ACT_FB_BASES; b++) L.first_thread[b] = threads;
+    return L;
+}
+static int slot_install(act_engine* e, int slot, const uint8_t sk_x[32], const uint8_t pk_w[32]) {
+    CK(cudaSetDevice(e->device));
+    key_slot k;
+    TRY(ensure(k.ctx, sizeof(act_ctx)));
+    TRY(ensure(k.w_table, sizeof(ge_niels) * fb_size_of(ACT_FB_BITS)));
+    dev_buf<u32> d_enc, d_ok;
+    dev_buf<ge> d_bases, d_W;
+    TRY(ensure(d_enc, 128)); TRY(ensure(d_ok, 4));
+    TRY(ensure(d_bases, sizeof(ge) * ACT_FB_BASES)); TRY(ensure(d_W, sizeof(ge)));
+    CK(cudaMemcpy(d_enc, e->pub.h_enc, 96, cudaMemcpyHostToDevice));
+    CK(cudaMemcpy(d_enc.p + 24, pk_w, 32, cudaMemcpyHostToDevice));
+    fb_layout L = w_layout();
+    setup_decode_kernel<<<1, 1>>>(d_enc, d_bases, d_W, d_ok);
+    build_fb_tables_kernel<<<(L.first_thread[ACT_FB_BASES] + 31) / 32, 32>>>(d_bases.p + ACT_BASE_W, k.w_table, L);
+    CK(cudaGetLastError());
+    u32 ok = 0;
+    CK(cudaMemcpy(&ok, d_ok, 4, cudaMemcpyDeviceToHost));
+    if (!ok) return fail_msg("act_engine_set_key: pk_w is not a valid ristretto255 encoding");
+    act_ctx hc = e->pub;
+    struct wipe_on_exit { void* p; size_t n; ~wipe_on_exit() { explicit_bzero(p, n); } } hc_guard{&hc, sizeof hc};
+    hc.fb[ACT_BASE_W] = fb_tab{k.w_table.p, ACT_FB_BITS, fb_win_of(ACT_FB_BITS), fb_ent_of(ACT_FB_BITS)};
+    CK(cudaMemcpy(&hc.W, d_W, sizeof(ge), cudaMemcpyDeviceToHost));
+    memcpy(hc.x.v, sk_x, 32);
+    wipe_dev_on_exit ctx_wipe{k.ctx.p, sizeof(act_ctx), nullptr};   // the new context holds x from here on; wiped unless installed
+    CK(cudaMemcpy(k.ctx, &hc, sizeof hc, cudaMemcpyHostToDevice));
+    explicit_bzero(&hc, sizeof hc);
+    finalize_ctx_kernel<<<1, 1>>>(k.ctx, d_enc.p + 24, d_ok);
+    CK(cudaGetLastError());
+    CK(cudaMemcpy(&ok, d_ok, 4, cudaMemcpyDeviceToHost));
+    if (!ok) return fail_msg("act_engine_set_key: pk_w is not the public key of sk_x (W != G*x)");
+    // in-flight work (also _dev calls on callers' streams) may still read the slot's old key and table
+    CK(cudaDeviceSynchronize());
+    key_slot& old = e->key[slot];
+    if (old.ctx.p) CK(cudaMemset(old.ctx, 0, sizeof(act_ctx)));
+    ctx_wipe.p = nullptr;
+    std::swap(old, k);   // k takes the old key and frees it
+    return upload_slots(e);
+}
+static int slot_clear(act_engine* e, int slot) {
+    CK(cudaSetDevice(e->device));
+    CK(cudaDeviceSynchronize());
+    key_slot& k = e->key[slot];
+    CK(cudaMemset(k.ctx, 0, sizeof(act_ctx)));
+    k = key_slot();   // frees the context and the W table
+    return upload_slots(e);
+}
+static uint32_t slots_held(const act_engine* e) {
+    uint32_t m = 0;
+    for (int k = 0; k < ACT_KEY_SLOTS; k++) if (e->key[k].ctx.p) m |= 1u << k;
+    return m;
+}
+static inline const act_engine* replica0(const act_engine* e) { return is_multi(e) ? e->replicas[0] : e; }
+extern "C" int act_engine_set_key(act_engine* e, int slot, const uint8_t sk_x[32], const uint8_t pk_w[32]) {
+    if (!e) return fail_msg("null engine");
+    if (!sk_x || !pk_w) return fail_msg("act_engine_set_key: null argument");
+    if (slot < 0 || slot >= ACT_KEY_SLOTS) return fail_msg("act_engine_set_key: slot out of range (0 .. ACT_KEY_SLOTS - 1)");
+    if (!is_multi(e)) return slot_install(e, slot, sk_x, pk_w);
+    for (act_engine* r : e->replicas) TRY(slot_install(r, slot, sk_x, pk_w));   // replica 0 checks the key before any other changes
+    return 0;
+}
+extern "C" int act_engine_clear_key(act_engine* e, int slot) {
+    if (!e) return fail_msg("null engine");
+    if (slot < 0 || slot >= ACT_KEY_SLOTS) return fail_msg("act_engine_clear_key: slot out of range (0 .. ACT_KEY_SLOTS - 1)");
+    const act_engine* r0 = replica0(e);
+    if (slot == r0->selected) return fail_msg("act_engine_clear_key: the selected slot cannot be cleared (select another first)");
+    if (!(slots_held(r0) >> slot & 1u)) return fail_msg("act_engine_clear_key: the slot holds no key");
+    if (!is_multi(e)) return slot_clear(e, slot);
+    for (act_engine* r : e->replicas) TRY(slot_clear(r, slot));
+    return 0;
+}
+extern "C" int act_engine_select_key(act_engine* e, int slot) {
+    if (!e) return fail_msg("null engine");
+    if (slot < 0 || slot >= ACT_KEY_SLOTS) return fail_msg("act_engine_select_key: slot out of range (0 .. ACT_KEY_SLOTS - 1)");
+    if (!(slots_held(replica0(e)) >> slot & 1u)) return fail_msg("act_engine_select_key: the slot holds no key");
+    for (act_engine* r : e->replicas) r->selected = slot;
+    e->selected = slot;
+    return 0;
+}
+extern "C" int act_engine_selected_key(const act_engine* e) { return e ? replica0(e)->selected : -1; }
+extern "C" uint32_t act_engine_key_slots(const act_engine* e) { return e ? slots_held(replica0(e)) : 0u; }
 
 extern "C" int act_engine_set_timing(act_engine* e, int enable) {
     if (!e) return fail_msg("null engine");
@@ -858,7 +978,7 @@ extern "C" int act_batch_issue_dev(act_engine* e, size_t n, const void* req, con
     NEED_ALIGNED("act_batch_issue_dev", req, c, rnd, resp);
     CK(cudaSetDevice(e->device));
     cudaStream_t st = stream ? (cudaStream_t)stream : e->stream[0];
-    LAUNCH(e, K_ISSUE, st, (issue_kernel<<<nblocks(n, ACT_ISSUE_BLOCK), ACT_ISSUE_BLOCK, 0, st>>>(e->d_ctx, n, (const u32*)req, (const u32*)c, (const u32*)rnd, (u32*)resp, (u8*)status)));
+    LAUNCH(e, K_ISSUE, st, (issue_kernel<<<nblocks(n, ACT_ISSUE_BLOCK), ACT_ISSUE_BLOCK, 0, st>>>(sel_ctx(e), n, (const u32*)req, (const u32*)c, (const u32*)rnd, (u32*)resp, (u8*)status)));
     CK(cudaGetLastError());
     return 0;
 }
@@ -870,7 +990,7 @@ extern "C" int act_batch_issuance_check_dev(act_engine* e, size_t n, const void*
     NEED_ALIGNED("act_batch_issuance_check_dev", K, resp);
     CK(cudaSetDevice(e->device));
     cudaStream_t st = stream ? (cudaStream_t)stream : e->stream[0];
-    LAUNCH(e, K_ISSUANCE_CHECK, st, (issuance_check_kernel<<<nblocks(n, ACT_ISSUE_BLOCK), ACT_ISSUE_BLOCK, 0, st>>>(e->d_ctx, n, (const u32*)K, (const u32*)resp, (u8*)status)));
+    LAUNCH(e, K_ISSUANCE_CHECK, st, (issuance_check_kernel<<<nblocks(n, ACT_ISSUE_BLOCK), ACT_ISSUE_BLOCK, 0, st>>>(sel_ctx(e), n, (const u32*)K, (const u32*)resp, (u8*)status)));
     CK(cudaGetLastError());
     return 0;
 }
@@ -882,29 +1002,34 @@ extern "C" int act_batch_refund_check_dev(act_engine* e, size_t n, const void* c
     NEED_ALIGNED("act_batch_refund_check_dev", com, refund);
     CK(cudaSetDevice(e->device));
     cudaStream_t st = stream ? (cudaStream_t)stream : e->stream[0];
-    LAUNCH(e, K_REFUND_CHECK, st, (refund_check_kernel<<<nblocks(n, ACT_HEAD_BLOCK), ACT_HEAD_BLOCK, 0, st>>>(e->d_ctx, n, (const u32*)com, (const u32*)refund, (u8*)status)));
+    LAUNCH(e, K_REFUND_CHECK, st, (refund_check_kernel<<<nblocks(n, ACT_HEAD_BLOCK), ACT_HEAD_BLOCK, 0, st>>>(sel_ctx(e), n, (const u32*)com, (const u32*)refund, (u8*)status)));
     CK(cudaGetLastError());
     return 0;
 }
 // one chunk of the spend pipeline on one stream with one scratch set
 // kprime_out != nullptr: verification only -- K' of every proof goes to kprime_out (m x 128 B) and the signing stage is left
 // to the caller (sequential-RNG contract)
+// key_ids != nullptr: keyed verification (one key id per proof; the refund is signed under the selected key)
 static int spend_chunk_launch(act_engine* e, spend_scratch* s, cudaStream_t st, size_t m, const u32* proofs, const u32* rnd,
-                              u32* refunds, u32* nullifiers, u8* status, u32* kprime_out = nullptr) {
+                              u32* refunds, u32* nullifiers, u8* status, u32* kprime_out = nullptr, const u8* key_ids = nullptr) {
     if (s->used) CK(cudaStreamWaitEvent(st, s->done, 0));   // the previous pipeline on this scratch set (any stream) has drained
     CK(cudaMemsetAsync(s->flags, 0, m * 4, st));
     CK(cudaMemsetAsync(s->counter, 0, 4, st));
     size_t rblocks = (m * ACT_L + ACT_RANGE_BLOCK - 1) / ACT_RANGE_BLOCK;   // blocks that would hold one thread per com_j
     unsigned rgrid = rblocks < s->range_grid ? (unsigned)rblocks : s->range_grid;
-    LAUNCH(e, K_RANGE, st, (spend_range_kernel<<<rgrid, ACT_RANGE_BLOCK, 0, st>>>(e->d_ctx, m, proofs, s->items, s->com_niels, s->flags, s->tabs, s->cpts, s->counter)));
+    LAUNCH(e, K_RANGE, st, (spend_range_kernel<<<rgrid, ACT_RANGE_BLOCK, 0, st>>>(sel_ctx(e), m, proofs, s->items, s->com_niels, s->flags, s->tabs, s->cpts, s->counter)));
     // head before encode: it completes the two half-commitments of j = 0 (their h2 terms) that the encode stage then reads
     u32* kp = kprime_out ? kprime_out : s->kprime;
-    LAUNCH(e, K_HEAD, st, (spend_head_kernel<<<nblocks(m, ACT_HEAD_BLOCK), ACT_HEAD_BLOCK, 0, st>>>(e->d_ctx, m, proofs, s->items, s->com_niels, kp, s->flags, s->cpts)));
-    LAUNCH(e, K_ENCODE, st, (spend_encode_kernel<<<nblocks(m * ACT_ENC_PARTS, ACT_ENC_BLOCK), ACT_ENC_BLOCK, 0, st>>>(e->d_ctx, m, s->cpts, s->items, 2 * ACT_L, 133)));
-    LAUNCH(e, K_CHUNK, st, (spend_chunk_kernel<<<nblocks(m * ACT_SPEND_CHUNKS, ACT_HASH_BLOCK), ACT_HASH_BLOCK, 0, st>>>(e->d_ctx, m, s->items, s->cvs)));
-    LAUNCH(e, K_FINISH, st, (spend_finish_kernel<<<nblocks(m, ACT_HASH_BLOCK), ACT_HASH_BLOCK, 0, st>>>(e->d_ctx, m, proofs, s->cvs, s->flags, status)));
+    if (key_ids)
+        LAUNCH(e, K_HEAD, st, (spend_head_keyed_kernel<<<nblocks(m, ACT_HEAD_BLOCK), ACT_HEAD_BLOCK, 0, st>>>(sel_ctx(e), m, proofs, s->items, s->com_niels, kp, s->flags, s->cpts,
+                                                                                                           key_ids, e->d_slots)));
+    else
+        LAUNCH(e, K_HEAD, st, (spend_head_kernel<<<nblocks(m, ACT_HEAD_BLOCK), ACT_HEAD_BLOCK, 0, st>>>(sel_ctx(e), m, proofs, s->items, s->com_niels, kp, s->flags, s->cpts)));
+    LAUNCH(e, K_ENCODE, st, (spend_encode_kernel<<<nblocks(m * ACT_ENC_PARTS, ACT_ENC_BLOCK), ACT_ENC_BLOCK, 0, st>>>(sel_ctx(e), m, s->cpts, s->items, 2 * ACT_L, 133)));
+    LAUNCH(e, K_CHUNK, st, (spend_chunk_kernel<<<nblocks(m * ACT_SPEND_CHUNKS, ACT_HASH_BLOCK), ACT_HASH_BLOCK, 0, st>>>(sel_ctx(e), m, s->items, s->cvs)));
+    LAUNCH(e, K_FINISH, st, (spend_finish_kernel<<<nblocks(m, ACT_HASH_BLOCK), ACT_HASH_BLOCK, 0, st>>>(sel_ctx(e), m, proofs, s->cvs, s->flags, status)));
     if (!kprime_out)
-        LAUNCH(e, K_SIGN, st, (refund_sign_kernel<<<nblocks(m, ACT_SIGN_BLOCK), ACT_SIGN_BLOCK, 0, st>>>(e->d_ctx, m, proofs, rnd, s->kprime, status, refunds, nullifiers)));
+        LAUNCH(e, K_SIGN, st, (refund_sign_kernel<<<nblocks(m, ACT_SIGN_BLOCK), ACT_SIGN_BLOCK, 0, st>>>(sel_ctx(e), m, proofs, rnd, s->kprime, status, refunds, nullifiers)));
     else if (nullifiers) {   // verification-only pass that also delivers nullifier() of every accepted proof
         nullifier_kernel<<<nblocks(m * 8, 256), 256, 0, st>>>(m, s->items, status, nullifiers);
         e->launches += 1;
@@ -914,13 +1039,9 @@ static int spend_chunk_launch(act_engine* e, spend_scratch* s, cudaStream_t st, 
     s->used = true;
     return 0;
 }
-extern "C" int act_batch_verify_spend_and_refund_dev(act_engine* e, size_t n, const void* proofs, const void* rnd, void* refunds,
-                                                      void* nullifiers, void* status, void* stream) {
-    if (!e) return fail_msg("null engine");
-    NOT_MULTI(e, "act_batch_verify_spend_and_refund_dev");
-    if (n == 0) return 0;
-    if (!proofs || !rnd || !refunds || !nullifiers || !status) return fail_msg("act_batch_verify_spend_and_refund_dev: null buffer");
-    NEED_ALIGNED("act_batch_verify_spend_and_refund_dev", proofs, rnd, refunds, nullifiers);
+// the body of act_batch_verify_spend_and_refund_dev and of its keyed form (key_ids != nullptr)
+static int verify_spend_dev(act_engine* e, size_t n, const void* proofs, const u8* key_ids, const void* rnd, void* refunds, void* nullifiers,
+                            void* status, void* stream) {
     CK(cudaSetDevice(e->device));
     cudaStream_t user = stream ? (cudaStream_t)stream : e->stream[0];
     const size_t ACT_SPEND_CHUNK_RT = e->spend_chunk;
@@ -939,7 +1060,7 @@ extern "C" int act_batch_verify_spend_and_refund_dev(act_engine* e, size_t n, co
         int slot = two ? (int)(ci & 1) : 0;
         cudaStream_t st = two ? e->stream[slot] : user;
         TRY(spend_chunk_launch(e, &e->scratch[slot], st, m, (const u32*)proofs + off * ACT_PROOF_WORDS, (const u32*)rnd + off * 32,
-                               (u32*)refunds + off * 32, (u32*)nullifiers + off * 8, (u8*)status + off));
+                               (u32*)refunds + off * 32, (u32*)nullifiers + off * 8, (u8*)status + off, nullptr, key_ids ? key_ids + off : nullptr));
     }
     if (two) {
         CK(cudaEventRecord(e->join[0], e->stream[0]));
@@ -948,6 +1069,24 @@ extern "C" int act_batch_verify_spend_and_refund_dev(act_engine* e, size_t n, co
         CK(cudaStreamWaitEvent(user, e->join[1], 0));
     }
     return 0;
+}
+extern "C" int act_batch_verify_spend_and_refund_dev(act_engine* e, size_t n, const void* proofs, const void* rnd, void* refunds,
+                                                      void* nullifiers, void* status, void* stream) {
+    if (!e) return fail_msg("null engine");
+    NOT_MULTI(e, "act_batch_verify_spend_and_refund_dev");
+    if (n == 0) return 0;
+    if (!proofs || !rnd || !refunds || !nullifiers || !status) return fail_msg("act_batch_verify_spend_and_refund_dev: null buffer");
+    NEED_ALIGNED("act_batch_verify_spend_and_refund_dev", proofs, rnd, refunds, nullifiers);
+    return verify_spend_dev(e, n, proofs, nullptr, rnd, refunds, nullifiers, status, stream);
+}
+extern "C" int act_batch_verify_spend_and_refund_keyed_dev(act_engine* e, size_t n, const void* proofs, const void* key_ids, const void* rnd, void* refunds,
+                                                            void* nullifiers, void* status, void* stream) {
+    if (!e) return fail_msg("null engine");
+    NOT_MULTI(e, "act_batch_verify_spend_and_refund_keyed_dev");
+    if (n == 0) return 0;
+    if (!proofs || !key_ids || !rnd || !refunds || !nullifiers || !status) return fail_msg("act_batch_verify_spend_and_refund_keyed_dev: null buffer");
+    NEED_ALIGNED("act_batch_verify_spend_and_refund_keyed_dev", proofs, rnd, refunds, nullifiers);   // key ids are read byte by byte
+    return verify_spend_dev(e, n, proofs, (const u8*)key_ids, rnd, refunds, nullifiers, status, stream);
 }
 
 // ---- host-buffer entry points: chunked, double-buffered over the engine's two streams ----
@@ -1060,6 +1199,18 @@ extern "C" int act_batch_refund_check(act_engine* e, size_t n, const uint8_t* co
         return act_batch_refund_check_dev(e, m, io.in[0], io.in[1], io.st, st);
     });
 }
+// one replica's host-buffer verify + refund; key_ids (one byte per proof, optional) travel with the proofs
+static int verify_spend_host(act_engine* e, size_t n, const uint8_t* proofs, const uint8_t* key_ids, const uint8_t* rnd, uint8_t* refunds,
+                             uint8_t* nullifiers, uint8_t* status) {
+    host_io h = {{proofs, rnd, key_ids}, {ACT_PROOF_BYTES, 128, 1}, {refunds, nullifiers, status}, {128, 32, 1}, 1};
+    // the scratch sets before anything is in flight
+    CK(cudaSetDevice(e->device));
+    TRY(ensure_spend_scratch(e, n));
+    return run_chunked(e, n, e->spend_chunk, h, [&](int s, cudaStream_t st, size_t m, io_slot& io) {
+        return spend_chunk_launch(e, &e->scratch[s], st, m, (const u32*)io.in[0].p, (const u32*)io.in[1].p, (u32*)io.out[0].p, (u32*)io.out[1].p, io.st,
+                                  nullptr, key_ids ? io.in[2].p : nullptr);
+    }, true);
+}
 extern "C" int act_batch_verify_spend_and_refund(act_engine* e, size_t n, const uint8_t* proofs, const uint8_t* rnd, uint8_t* refunds,
                                                   uint8_t* nullifiers, uint8_t* status) {
     if (!e) return fail_msg("null engine");
@@ -1067,13 +1218,7 @@ extern "C" int act_batch_verify_spend_and_refund(act_engine* e, size_t n, const 
     if (!proofs || !rnd || !refunds || !nullifiers || !status) return fail_msg("act_batch_verify_spend_and_refund: null buffer");
     if (is_multi(e)) return shard_over_replicas(e, n, [&](act_engine* r, size_t lo, size_t m) {
         return act_batch_verify_spend_and_refund(r, m, proofs + lo * ACT_PROOF_BYTES, rnd + lo * 128, refunds + lo * 128, nullifiers + lo * 32, status + lo); });
-    host_io h = {{proofs, rnd, nullptr}, {ACT_PROOF_BYTES, 128, 0}, {refunds, nullifiers, status}, {128, 32, 1}, 1};
-    // the scratch sets before anything is in flight
-    CK(cudaSetDevice(e->device));
-    TRY(ensure_spend_scratch(e, n));
-    return run_chunked(e, n, e->spend_chunk, h, [&](int s, cudaStream_t st, size_t m, io_slot& io) {
-        return spend_chunk_launch(e, &e->scratch[s], st, m, (const u32*)io.in[0].p, (const u32*)io.in[1].p, (u32*)io.out[0].p, (u32*)io.out[1].p, io.st);
-    }, true);
+    return verify_spend_host(e, n, proofs, nullptr, rnd, refunds, nullifiers, status);
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -1212,6 +1357,55 @@ static int store_grow(act_nullifier_store* s, size_t slots, cudaStream_t st) {
     s->slots = slots;
     return 0;
 }
+// slots of the in-batch dedupe table for n keys
+static size_t dedupe_slots(size_t n) {
+    size_t dd = ACT_STORE_MIN_SLOTS;
+    while (dd < 2 * n) dd <<= 1;
+    return dd;
+}
+// A screen of n (status, nullifier) pairs against the store and the batch itself, then (record != 0) insertion of the survivors,
+// in two halves.  The first does everything that can fail: scratch, the lookup (+ key check), one 16-byte read-back (bad-key flag
+// and exact size), growth if `adds` more members could cross the load limit.  It leaves the membership as it was.  The second
+// launches the in-batch dedupe and the insert and cannot fail but for a launch error.  A call over several stores prepares every
+// store before it commits the first.
+static int store_prepare(act_nullifier_store* s, size_t n, const void* status, const void* nullifiers, int record, size_t adds, cudaStream_t st) {
+    CK(cudaStreamWaitEvent(st, s->done, 0));
+    // growing drains st first: the store's previous call has then finished with its scratch
+    TRY(ensure(s->st_tmp, n, st));
+    TRY(ensure(s->dd_table, dedupe_slots(n) * 4, st));
+    CK(cudaMemsetAsync(s->d_misc.p + 1, 0, sizeof(unsigned long long), st));
+    store_lookup_kernel<<<nblocks(n, 256), 256, 0, st>>>((u64)n, (const u8*)status, (const uint4*)nullifiers, s->table, (u64)(s->slots - 1), s->key,
+                                                        s->st_tmp, reinterpret_cast<u32*>(s->d_misc.p + 1));
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(s->h_misc, s->d_misc, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    if (s->h_misc[1]) {
+        CK(cudaEventRecord(s->done, st));
+        return fail_msg("act_nullifier_store_screen_dev: a nullifier with status 0 is not reduced mod l");
+    }
+    size_t size = (size_t)s->h_misc[0];
+    if (record && size + adds > s->slots / 2) {
+        size_t want = store_slots_for(size + adds);
+        if (!want) return fail_msg("act_nullifier_store_screen_dev: store too large");
+        int rc = store_grow(s, want, st);
+        if (rc) { cudaEventRecord(s->done, st); return rc; }
+    }
+    return 0;
+}
+static int store_commit(act_nullifier_store* s, size_t n, const void* nullifiers, void* status_out, int record, cudaStream_t st) {
+    size_t dd = dedupe_slots(n);
+    CK(cudaMemsetAsync(s->dd_table, 0xff, dd * 4, st));
+    rp_key128 seed = {s->key.k0 ^ (++s->calls * 0x9e3779b97f4a7c15ull), s->key.k1};
+    replay_insert_kernel<<<nblocks(n, 256), 256, 0, st>>>((u32)n, 0, s->st_tmp, nullptr, (const uint4*)nullifiers, s->dd_table, (u32)(dd - 1), seed);
+    replay_resolve_kernel<<<nblocks(n, 256), 256, 0, st>>>((u32)n, 0, s->st_tmp, nullptr, (const uint4*)nullifiers, s->dd_table, (u32)(dd - 1), seed,
+                                                           (u8*)status_out);
+    if (record)
+        store_insert_kernel<<<nblocks(n, 256), 256, 0, st>>>((u64)n, (const u8*)status_out, (const uint4*)nullifiers, s->table, (u64)(s->slots - 1),
+                                                            s->key, s->d_misc);
+    CK(cudaGetLastError());
+    CK(cudaEventRecord(s->done, st));
+    return 0;
+}
 // Screen of n (status, nullifier) pairs against the store and the batch itself, then (record != 0) insertion of the survivors.
 // In stream order: lookup (+ key check) -> one 16-byte read-back (bad-key flag and exact size) -> growth if the survivors could
 // cross the load limit -> in-batch dedupe -> insert.  Everything that can fail is decided before the insert is launched.
@@ -1230,40 +1424,8 @@ extern "C" int act_nullifier_store_screen_dev(act_nullifier_store* s, size_t n, 
             return fail_msg("act_nullifier_store_screen_dev: buffers must be device memory on the store's device");
     }
     cudaStream_t st = stream ? (cudaStream_t)stream : s->stream;
-    CK(cudaStreamWaitEvent(st, s->done, 0));
-    // growing drains st first: the store's previous call has then finished with its scratch
-    TRY(ensure(s->st_tmp, n, st));
-    size_t dd = ACT_STORE_MIN_SLOTS;
-    while (dd < 2 * n) dd <<= 1;
-    TRY(ensure(s->dd_table, dd * 4, st));
-    CK(cudaMemsetAsync(s->d_misc.p + 1, 0, sizeof(unsigned long long), st));
-    store_lookup_kernel<<<nblocks(n, 256), 256, 0, st>>>((u64)n, (const u8*)status, (const uint4*)nullifiers, s->table, (u64)(s->slots - 1), s->key,
-                                                        s->st_tmp, reinterpret_cast<u32*>(s->d_misc.p + 1));
-    CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(s->h_misc, s->d_misc, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    if (s->h_misc[1]) {
-        CK(cudaEventRecord(s->done, st));
-        return fail_msg("act_nullifier_store_screen_dev: a nullifier with status 0 is not reduced mod l");
-    }
-    size_t size = (size_t)s->h_misc[0];
-    if (record && size + n > s->slots / 2) {
-        size_t want = store_slots_for(size + n);
-        if (!want) return fail_msg("act_nullifier_store_screen_dev: store too large");
-        int rc = store_grow(s, want, st);
-        if (rc) { cudaEventRecord(s->done, st); return rc; }
-    }
-    CK(cudaMemsetAsync(s->dd_table, 0xff, dd * 4, st));
-    rp_key128 seed = {s->key.k0 ^ (++s->calls * 0x9e3779b97f4a7c15ull), s->key.k1};
-    replay_insert_kernel<<<nblocks(n, 256), 256, 0, st>>>((u32)n, 0, s->st_tmp, nullptr, (const uint4*)nullifiers, s->dd_table, (u32)(dd - 1), seed);
-    replay_resolve_kernel<<<nblocks(n, 256), 256, 0, st>>>((u32)n, 0, s->st_tmp, nullptr, (const uint4*)nullifiers, s->dd_table, (u32)(dd - 1), seed,
-                                                           (u8*)status_out);
-    if (record)
-        store_insert_kernel<<<nblocks(n, 256), 256, 0, st>>>((u64)n, (const u8*)status_out, (const uint4*)nullifiers, s->table, (u64)(s->slots - 1),
-                                                            s->key, s->d_misc);
-    CK(cudaGetLastError());
-    CK(cudaEventRecord(s->done, st));
-    return 0;
+    TRY(store_prepare(s, n, status, nullifiers, record, n, st));
+    return store_commit(s, n, nullifiers, status_out, record, st);
 }
 extern "C" int act_nullifier_store_screen(act_nullifier_store* s, size_t n, const uint8_t* status, const uint8_t* nullifiers, uint8_t* status_out,
                                           int record) {
@@ -1400,7 +1562,7 @@ extern "C" int act_batch_request_dev(act_engine* e, size_t n, const void* pre, c
     if (!pre || !rnd || !req) return fail_msg("act_batch_request_dev: null buffer");
     CK(cudaSetDevice(e->device));
     cudaStream_t st = stream ? (cudaStream_t)stream : e->stream[0];
-    request_kernel<<<nblocks(n, ACT_ISSUE_BLOCK), ACT_ISSUE_BLOCK, 0, st>>>(e->d_ctx, n, (const u32*)pre, (const u32*)rnd, (u32*)req);
+    request_kernel<<<nblocks(n, ACT_ISSUE_BLOCK), ACT_ISSUE_BLOCK, 0, st>>>(sel_ctx(e), n, (const u32*)pre, (const u32*)rnd, (u32*)req);
     e->launches += 1;
     CK(cudaGetLastError());
     return 0;
@@ -1432,12 +1594,12 @@ extern "C" int act_batch_prove_spend_dev(act_engine* e, size_t n, const void* to
         const u32* ch = (const u32*)charges + off * 8;
         u8* stt = (u8*)status + off;
         unsigned grid = (unsigned)(m < (size_t)sms * 4 ? m : (size_t)sms * 4);
-        prove_range_kernel<<<grid, ACT_L, 0, st>>>(e->d_ctx, R, m, tk, ch, e->pv_cpts);
-        spend_encode_kernel<<<nblocks(m * ACT_PROVE_PARTS, ACT_ENC_BLOCK), ACT_ENC_BLOCK, 0, st>>>(e->d_ctx, m, e->pv_cpts, e->pv_items, ACT_PROVE_PTS, 5);
-        prove_head_kernel<<<nblocks(m, ACT_HEAD_BLOCK), ACT_HEAD_BLOCK, 0, st>>>(e->d_ctx, R, m, tk, e->pv_items, e->pv_aux, stt);
-        spend_chunk_kernel<<<nblocks(m * ACT_SPEND_CHUNKS, ACT_HASH_BLOCK), ACT_HASH_BLOCK, 0, st>>>(e->d_ctx, m, e->pv_items, e->pv_cvs);
+        prove_range_kernel<<<grid, ACT_L, 0, st>>>(sel_ctx(e), R, m, tk, ch, e->pv_cpts);
+        spend_encode_kernel<<<nblocks(m * ACT_PROVE_PARTS, ACT_ENC_BLOCK), ACT_ENC_BLOCK, 0, st>>>(sel_ctx(e), m, e->pv_cpts, e->pv_items, ACT_PROVE_PTS, 5);
+        prove_head_kernel<<<nblocks(m, ACT_HEAD_BLOCK), ACT_HEAD_BLOCK, 0, st>>>(sel_ctx(e), R, m, tk, e->pv_items, e->pv_aux, stt);
+        spend_chunk_kernel<<<nblocks(m * ACT_SPEND_CHUNKS, ACT_HASH_BLOCK), ACT_HASH_BLOCK, 0, st>>>(sel_ctx(e), m, e->pv_items, e->pv_cvs);
         prove_challenge_kernel<<<nblocks(m, ACT_HASH_BLOCK), ACT_HASH_BLOCK, 0, st>>>(m, e->pv_cvs, e->pv_gammas);
-        prove_finish_kernel<<<grid, ACT_L, 0, st>>>(e->d_ctx, R, m, tk, ch, e->pv_items, e->pv_aux, e->pv_gammas, stt,
+        prove_finish_kernel<<<grid, ACT_L, 0, st>>>(sel_ctx(e), R, m, tk, ch, e->pv_items, e->pv_aux, e->pv_gammas, stt,
                                                    (u32*)proofs + off * ACT_PROOF_WORDS, (u32*)prerefunds + off * 24);
         e->launches += 6;
         CK(cudaGetLastError());
@@ -1542,7 +1704,7 @@ extern "C" int act_batch_issue_verify(act_engine* e, size_t n, const uint8_t* re
     if (is_multi(e)) return shard_over_replicas(e, n, [&](act_engine* r, size_t lo, size_t m) { return act_batch_issue_verify(r, m, req + lo * 128, status + lo); });
     host_io h = {{req, nullptr, nullptr}, {128, 0, 0}, {nullptr, nullptr, status}, {0, 0, 1}};
     return run_chunked(e, n, ACT_SMALL_CHUNK, h, [&](int, cudaStream_t st, size_t m, io_slot& io) {
-        issue_mode_kernel<<<nblocks(m, ACT_ISSUE_BLOCK), ACT_ISSUE_BLOCK, 0, st>>>(e->d_ctx, m, (const u32*)io.in[0].p, nullptr, nullptr, nullptr, io.st, ACT_MODE_VERIFY, nullptr);
+        issue_mode_kernel<<<nblocks(m, ACT_ISSUE_BLOCK), ACT_ISSUE_BLOCK, 0, st>>>(sel_ctx(e), m, (const u32*)io.in[0].p, nullptr, nullptr, nullptr, io.st, ACT_MODE_VERIFY, nullptr);
         e->launches += 1;
         CK(cudaGetLastError());
         return 0;
@@ -1577,7 +1739,7 @@ extern "C" int act_batch_issue_sign(act_engine* e, size_t n, const uint8_t* req,
     CK(cudaMemcpyAsync(d_st, status, n, cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(d_idx, idx.data(), n * 4, cudaMemcpyHostToDevice, st));
     if (used) CK(cudaMemcpyAsync(d_rnd, rnd, used, cudaMemcpyHostToDevice, st));
-    issue_mode_kernel<<<nblocks(n, ACT_ISSUE_BLOCK), ACT_ISSUE_BLOCK, 0, st>>>(e->d_ctx, n, (const u32*)d_req.p, (const u32*)d_c.p, (const u32*)d_rnd.p, (u32*)d_resp.p, d_st, ACT_MODE_SIGN, d_idx);
+    issue_mode_kernel<<<nblocks(n, ACT_ISSUE_BLOCK), ACT_ISSUE_BLOCK, 0, st>>>(sel_ctx(e), n, (const u32*)d_req.p, (const u32*)d_c.p, (const u32*)d_rnd.p, (u32*)d_resp.p, d_st, ACT_MODE_SIGN, d_idx);
     e->launches += 1;
     CK(cudaGetLastError());
     CK(cudaMemcpyAsync(resp, d_resp, n * 160, cudaMemcpyDeviceToHost, st));
@@ -1587,18 +1749,32 @@ extern "C" int act_batch_issue_sign(act_engine* e, size_t n, const uint8_t* req,
     CK(cudaStreamSynchronize(st));
     return 0;
 }
+// one replica's verification pass (key_ids optional)
+static int spend_verify_host(act_engine* e, size_t n, const uint8_t* proofs, const uint8_t* key_ids, uint8_t* nullifiers, uint8_t* status, uint8_t* kprime) {
+    CK(cudaSetDevice(e->device));
+    TRY(ensure_spend_scratch(e, n));
+    host_io h = {{proofs, key_ids, nullptr}, {ACT_PROOF_BYTES, 1, 0}, {kprime, nullifiers, status}, {128, 32, 1}};
+    return run_chunked(e, n, e->spend_chunk, h, [&](int s, cudaStream_t st, size_t m, io_slot& io) {
+        return spend_chunk_launch(e, &e->scratch[s], st, m, (const u32*)io.in[0].p, nullptr, nullptr, (u32*)io.out[1].p, io.st, (u32*)io.out[0].p,
+                                  key_ids ? io.in[1].p : nullptr);
+    }, true);
+}
 extern "C" int act_batch_spend_verify(act_engine* e, size_t n, const uint8_t* proofs, uint8_t* nullifiers, uint8_t* status, uint8_t* kprime) {
     if (!e) return fail_msg("null engine");
     if (n == 0) return 0;
     if (!proofs || !nullifiers || !status || !kprime) return fail_msg("act_batch_spend_verify: null buffer");
     if (is_multi(e)) return shard_over_replicas(e, n, [&](act_engine* r, size_t lo, size_t m) {
         return act_batch_spend_verify(r, m, proofs + lo * ACT_PROOF_BYTES, nullifiers + lo * 32, status + lo, kprime + lo * 128); });
-    CK(cudaSetDevice(e->device));
-    TRY(ensure_spend_scratch(e, n));
-    host_io h = {{proofs, nullptr, nullptr}, {ACT_PROOF_BYTES, 0, 0}, {kprime, nullifiers, status}, {128, 32, 1}};
-    return run_chunked(e, n, e->spend_chunk, h, [&](int s, cudaStream_t st, size_t m, io_slot& io) {
-        return spend_chunk_launch(e, &e->scratch[s], st, m, (const u32*)io.in[0].p, nullptr, nullptr, (u32*)io.out[1].p, io.st, (u32*)io.out[0].p);
-    }, true);
+    return spend_verify_host(e, n, proofs, nullptr, nullifiers, status, kprime);
+}
+extern "C" int act_batch_spend_verify_keyed(act_engine* e, size_t n, const uint8_t* proofs, const uint8_t* key_ids, uint8_t* nullifiers, uint8_t* status,
+                                            uint8_t* kprime) {
+    if (!e) return fail_msg("null engine");
+    if (n == 0) return 0;
+    if (!proofs || !key_ids || !nullifiers || !status || !kprime) return fail_msg("act_batch_spend_verify_keyed: null buffer");
+    if (is_multi(e)) return shard_over_replicas(e, n, [&](act_engine* r, size_t lo, size_t m) {
+        return act_batch_spend_verify_keyed(r, m, proofs + lo * ACT_PROOF_BYTES, key_ids + lo, nullifiers + lo * 32, status + lo, kprime + lo * 128); });
+    return spend_verify_host(e, n, proofs, key_ids, nullifiers, status, kprime);
 }
 extern "C" int act_batch_refund_sign(act_engine* e, size_t n, const uint8_t* kprime, const uint8_t* status, const uint8_t* rnd, size_t rnd_len, uint8_t* refunds) {
     if (!e) return fail_msg("null engine");
@@ -1627,7 +1803,7 @@ extern "C" int act_batch_refund_sign(act_engine* e, size_t n, const uint8_t* kpr
     CK(cudaMemcpyAsync(d_st, status, n, cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(d_idx, idx.data(), n * 4, cudaMemcpyHostToDevice, st));
     if (used) CK(cudaMemcpyAsync(d_rnd, rnd, used, cudaMemcpyHostToDevice, st));
-    refund_sign_seq_kernel<<<nblocks(n, ACT_SIGN_BLOCK), ACT_SIGN_BLOCK, 0, st>>>(e->d_ctx, n, nullptr, (const u32*)d_rnd.p, (const u32*)d_kp.p, d_st, (u32*)d_ref.p, nullptr, d_idx, nullptr);
+    refund_sign_seq_kernel<<<nblocks(n, ACT_SIGN_BLOCK), ACT_SIGN_BLOCK, 0, st>>>(sel_ctx(e), n, nullptr, (const u32*)d_rnd.p, (const u32*)d_kp.p, d_st, (u32*)d_ref.p, nullptr, d_idx, nullptr);
     e->launches += 1;
     CK(cudaGetLastError());
     CK(cudaMemcpyAsync(refunds, d_ref, n * 128, cudaMemcpyDeviceToHost, st));
@@ -1680,26 +1856,78 @@ extern "C" int act_batch_verify_spend_and_refund_seq(act_engine* e, size_t n, co
 // occurred earlier in the slice or in `seen` gets status 3 (DoubleSpendError) and NO refund (zero-filled, as the reference
 // never calls refund() for it); its nullifier is kept so that the caller can tell which token was replayed.
 // ---------------------------------------------------------------------------------------------------
+// The screen of a keyed batch: proof i against the store of its key's slot (map), each store in slice order over its own proofs.
+// Every store is prepared (lookup, key check, growth) before the first is committed, so a call that fails changes no store.
+static int screen_stores_keyed(act_engine* r0, size_t n, const uint8_t* key_ids, const u8* g_st, const u8* g_nul,
+                               const std::vector<act_nullifier_store*>& stores, const act_store_map& map, u8* d_out, cudaStream_t st) {
+    size_t D = stores.size();
+    std::vector<size_t> adds(D, 0);   // proofs per store: a bound on what it may record
+    for (size_t i = 0; i < n; i++) {
+        u8 j = key_ids[i] < ACT_KEY_SLOTS ? map.of_slot[key_ids[i]] : 0xFF;
+        if (j != 0xFF) adds[j]++;
+    }
+    dev_buf<u8> d_kid;
+    std::vector<dev_buf<u8>> masked(D);
+    TRY(ensure(d_kid, n));
+    for (size_t j = 0; j < D; j++) if (adds[j]) TRY(ensure(masked[j], n));
+    CK(cudaMemcpyAsync(d_kid, key_ids, n, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(d_out, g_st, n, cudaMemcpyDeviceToDevice, st));
+    for (size_t j = 0; j < D; j++) {
+        if (!adds[j]) continue;
+        store_mask_kernel<<<nblocks(n, 256), 256, 0, st>>>(n, g_st, d_kid, map, (u32)j, masked[j]);
+        r0->launches += 1;
+        CK(cudaGetLastError());
+        TRY(store_prepare(stores[j], n, masked[j], g_nul, 1, adds[j], st));
+    }
+    for (size_t j = 0; j < D; j++) {
+        if (!adds[j]) continue;
+        TRY(store_commit(stores[j], n, g_nul, masked[j], 1, st));
+        store_merge_kernel<<<nblocks(n, 256), 256, 0, st>>>(n, masked[j], d_kid, map, (u32)j, d_out);
+        r0->launches += 1;
+        CK(cudaGetLastError());
+    }
+    return 0;
+}
 static int ensure_gather(act_engine* r, size_t m) {
     CK(cudaSetDevice(r->device));
     TRY(ensure(r->g_st, m + 16));
     TRY(ensure(r->g_nul, m * 32 + 16));
     return 0;
 }
-// the screen runs against `seen` (n_seen keys, host memory) when store is null, else against the store, recording the survivors
-static int verify_refund_and_screen(act_engine* e, size_t n, const uint8_t* proofs, const uint8_t* rnd, size_t n_seen, const uint8_t* seen,
-                                    act_nullifier_store* store, uint8_t* refunds, uint8_t* nullifiers, uint8_t* status) {
+// The screen runs against `seen` (n_seen keys, host memory) when stores is null.  Otherwise it runs against stores[0] for every
+// proof (key_ids null), or proof i against stores[key_ids[i]] (ACT_KEY_SLOTS entries: the keyed call), recording the survivors.
+static int verify_refund_and_screen(act_engine* e, size_t n, const uint8_t* proofs, const uint8_t* key_ids, const uint8_t* rnd, size_t n_seen,
+                                    const uint8_t* seen, act_nullifier_store* const* stores, uint8_t* refunds, uint8_t* nullifiers, uint8_t* status) {
     std::vector<act_engine*> reps = e->replicas.empty() ? std::vector<act_engine*>{e} : e->replicas;
-    if (store && store->device != reps[0]->device)
-        return fail_msg("act_batch_verify_spend_and_refund_recorded: the store must be on the device of replica 0 (where the gather lands)");
+    // the stores this call screens against, and (keyed) the index of each slot's store among them (0xFF: slot without a key)
+    std::vector<act_nullifier_store*> distinct;
+    act_store_map map;
+    memset(map.of_slot, 0xff, sizeof map.of_slot);
+    if (stores && !key_ids) distinct.push_back(stores[0]);
+    if (stores && key_ids) {
+        uint32_t held = slots_held(reps[0]);
+        for (int k = 0; k < ACT_KEY_SLOTS; k++) {
+            if (!(held >> k & 1u)) continue;
+            if (!stores[k]) return fail_msg(("act_batch_verify_spend_and_refund_keyed: slot " + std::to_string(k) + " holds a key but has no store").c_str());
+            size_t j = 0;
+            while (j < distinct.size() && distinct[j] != stores[k]) j++;
+            if (j == distinct.size()) distinct.push_back(stores[k]);
+            map.of_slot[k] = (u8)j;
+        }
+    }
+    for (act_nullifier_store* s : distinct)
+        if (s->device != reps[0]->device)
+            return fail_msg(key_ids ? "act_batch_verify_spend_and_refund_keyed: every store must be on the device of replica 0 (where the gather lands)"
+                                    : "act_batch_verify_spend_and_refund_recorded: the store must be on the device of replica 0 (where the gather lands)");
     size_t G = reps.size();
     for (size_t g = 0; g < G; g++) TRY(ensure_gather(reps[g], shard_lo(n, g + 1, G) - shard_lo(n, g, G)));
     int rc;
     for (auto* r : reps) r->g_keep = true;
-    if (G == 1) rc = act_batch_verify_spend_and_refund(reps[0], n, proofs, rnd, refunds, nullifiers, status);
+    if (G == 1) rc = verify_spend_host(reps[0], n, proofs, key_ids, rnd, refunds, nullifiers, status);
     else {
         rc = shard_over(reps, n, [&](act_engine* r, size_t lo, size_t m) {
-            return act_batch_verify_spend_and_refund(r, m, proofs + lo * ACT_PROOF_BYTES, rnd + lo * 128, refunds + lo * 128, nullifiers + lo * 32, status + lo); });
+            return verify_spend_host(r, m, proofs + lo * ACT_PROOF_BYTES, key_ids ? key_ids + lo : nullptr, rnd + lo * 128, refunds + lo * 128,
+                                     nullifiers + lo * 32, status + lo); });
     }
     for (auto* r : reps) r->g_keep = false;
     if (rc) return rc;
@@ -1720,8 +1948,9 @@ static int verify_refund_and_screen(act_engine* e, size_t n, const uint8_t* proo
     if (n_seen) { TRY(ensure(d_seen, n_seen * 32)); CK(cudaMemcpyAsync(d_seen, seen, n_seen * 32, cudaMemcpyHostToDevice, st)); }
     const u8* g_st = G > 1 ? d_st.p : r0->g_st.p;
     const u8* g_nul = G > 1 ? d_nul.p : r0->g_nul.p;
-    if (store) TRY(act_nullifier_store_screen_dev(store, n, g_st, g_nul, d_out, 1, st));
-    else TRY(act_flag_replays_dev(r0, n, g_st, g_nul, n_seen, d_seen, d_out, st));
+    if (!stores) TRY(act_flag_replays_dev(r0, n, g_st, g_nul, n_seen, d_seen, d_out, st));
+    else if (!key_ids) TRY(act_nullifier_store_screen_dev(distinct[0], n, g_st, g_nul, d_out, 1, st));
+    else TRY(screen_stores_keyed(r0, n, key_ids, g_st, g_nul, distinct, map, d_out, st));
     CK(cudaMemcpyAsync(status, d_out, n, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     for (size_t i = 0; i < n; i++) if (status[i] == 3) memset(refunds + i * 128, 0, 128);
@@ -1732,7 +1961,7 @@ extern "C" int act_batch_verify_spend_and_refund_screened(act_engine* e, size_t 
     if (!e) return fail_msg("null engine");
     if (n == 0) return 0;
     if (!proofs || !rnd || !refunds || !nullifiers || !status || (n_seen && !seen)) return fail_msg("act_batch_verify_spend_and_refund_screened: null buffer");
-    return verify_refund_and_screen(e, n, proofs, rnd, n_seen, seen, nullptr, refunds, nullifiers, status);
+    return verify_refund_and_screen(e, n, proofs, nullptr, rnd, n_seen, seen, nullptr, refunds, nullifiers, status);
 }
 extern "C" int act_batch_verify_spend_and_refund_recorded(act_engine* e, act_nullifier_store* s, size_t n, const uint8_t* proofs, const uint8_t* rnd,
                                                            uint8_t* refunds, uint8_t* nullifiers, uint8_t* status) {
@@ -1740,5 +1969,16 @@ extern "C" int act_batch_verify_spend_and_refund_recorded(act_engine* e, act_nul
     if (!s) return fail_msg("null store");
     if (n == 0) return 0;
     if (!proofs || !rnd || !refunds || !nullifiers || !status) return fail_msg("act_batch_verify_spend_and_refund_recorded: null buffer");
-    return verify_refund_and_screen(e, n, proofs, rnd, 0, nullptr, s, refunds, nullifiers, status);
+    return verify_refund_and_screen(e, n, proofs, nullptr, rnd, 0, nullptr, &s, refunds, nullifiers, status);
+}
+extern "C" int act_batch_verify_spend_and_refund_keyed(act_engine* e, size_t n, const uint8_t* proofs, const uint8_t* key_ids, const uint8_t* rnd,
+                                                        act_nullifier_store* const* stores, uint8_t* refunds, uint8_t* nullifiers, uint8_t* status) {
+    if (!e) return fail_msg("null engine");
+    if (n == 0) return 0;
+    if (!proofs || !key_ids || !rnd || !refunds || !nullifiers || !status) return fail_msg("act_batch_verify_spend_and_refund_keyed: null buffer");
+    if (stores) return verify_refund_and_screen(e, n, proofs, key_ids, rnd, 0, nullptr, stores, refunds, nullifiers, status);
+    if (is_multi(e)) return shard_over_replicas(e, n, [&](act_engine* r, size_t lo, size_t m) {
+        return act_batch_verify_spend_and_refund_keyed(r, m, proofs + lo * ACT_PROOF_BYTES, key_ids + lo, rnd + lo * 128, nullptr, refunds + lo * 128,
+                                                       nullifiers + lo * 32, status + lo); });
+    return verify_spend_host(e, n, proofs, key_ids, rnd, refunds, nullifiers, status);
 }

@@ -248,6 +248,57 @@ class Engine {
         }
         return out;
     }
+    // key rotation (include/act_engine.h, issuer key slots): install, select and retire keys; the selected key issues and refunds
+    void set_key(int slot, const PrivateKey& key) {
+        if (act_engine_set_key(e_, slot, key.secret().data(), key.public_key().w.data())) throw EngineError("act_engine_set_key");
+    }
+    void clear_key(int slot) { if (act_engine_clear_key(e_, slot)) throw EngineError("act_engine_clear_key"); }
+    void select_key(int slot) { if (act_engine_select_key(e_, slot)) throw EngineError("act_engine_select_key"); }
+    int selected_key() const { return act_engine_selected_key(e_); }
+    uint32_t key_slots() const { return act_engine_key_slots(e_); }
+    // the loop above for an issuer with several keys, over ONE rng: proof i is verified under the key of slot key_ids[i], its nullifier
+    // is checked against stores[key_ids[i]] (a replay of that store or of an earlier proof of the same store is Err(DoubleSpendError)),
+    // and the survivors -- 128 bytes drawn for each, in slice order -- are refunded under the selected key and recorded.  Every slot
+    // that holds a key needs a store; slots may share one.  Every store is screened once without recording before any records,
+    // so a failure leaves the stores as they were.
+    template <typename Rng>
+    std::vector<Result<RefundWithNullifier>> batch_verify_spend_and_refund(const std::vector<SpendProof>& proofs, const std::vector<uint8_t>& key_ids,
+                                                                           Rng& rng, const std::array<NullifierStore*, ACT_KEY_SLOTS>& stores) {
+        size_t n = proofs.size();
+        if (key_ids.size() != n) throw std::invalid_argument("keyed call: one key id per proof");
+        uint32_t held = key_slots();
+        std::vector<NullifierStore*> distinct;
+        std::array<int, ACT_KEY_SLOTS> of_slot;
+        of_slot.fill(-1);
+        for (int k = 0; k < ACT_KEY_SLOTS; k++) {
+            if (!(held >> k & 1u)) continue;
+            if (!stores[k]) throw std::invalid_argument("keyed call: every slot that holds a key needs a store");
+            size_t j = 0;
+            while (j < distinct.size() && distinct[j] != stores[k]) j++;
+            if (j == distinct.size()) distinct.push_back(stores[k]);
+            of_slot[k] = (int)j;
+        }
+        std::vector<uint8_t> status(n), nul(n * 32), kprime(n * 128), refunds(n * ACT_REFUND_BYTES);
+        const uint8_t* pf = n ? proofs[0].bytes.data() : nullptr;
+        if (act_batch_spend_verify_keyed(e_, n, pf, key_ids.data(), nul.data(), status.data(), kprime.data())) throw EngineError("act_batch_spend_verify_keyed");
+        // each store sees the statuses of its own proofs; the others are nonzero and take no part
+        auto store_of = [&](size_t i) { return key_ids[i] < ACT_KEY_SLOTS ? of_slot[key_ids[i]] : -1; };
+        std::vector<std::vector<uint8_t>> mine(distinct.size(), std::vector<uint8_t>(n, 0xFF));
+        for (size_t i = 0; i < n; i++) if (store_of(i) >= 0) mine[(size_t)store_of(i)][i] = status[i];
+        for (size_t j = 0; j < distinct.size(); j++) { std::vector<uint8_t> dry = mine[j]; distinct[j]->screen(dry, nul, false); }
+        for (size_t j = 0; j < distinct.size(); j++) distinct[j]->screen(mine[j], nul, true);
+        for (size_t i = 0; i < n; i++) if (store_of(i) >= 0) status[i] = mine[(size_t)store_of(i)][i];
+        std::vector<uint8_t> rnd = draw(status, rng);
+        if (act_batch_refund_sign(e_, n, kprime.data(), status.data(), rnd.data(), rnd.size(), refunds.data())) throw EngineError("act_batch_refund_sign");
+        wipe(rnd);
+        std::vector<Result<RefundWithNullifier>> out(n);
+        for (size_t i = 0; i < n; i++) {
+            out[i].status = status[i];
+            std::memcpy(out[i].value.nullifier.data(), nul.data() + 32 * i, 32);
+            std::memcpy(out[i].value.refund.bytes.data(), refunds.data() + i * ACT_REFUND_BYTES, ACT_REFUND_BYTES);
+        }
+        return out;
+    }
     // the same behind the caller's nullifier check (examples/act.rs:60-77): a proof whose nullifier occurred earlier in the slice or
     // in `seen` is Err(DoubleSpendError) and gets no refund.  Randomness is per request here (rnd: n x 128 bytes).
     std::vector<Result<RefundWithNullifier>> batch_verify_spend_and_refund_screened(const std::vector<SpendProof>& proofs, const std::vector<uint8_t>& rnd,

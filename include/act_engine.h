@@ -21,6 +21,9 @@
  *                                      = refund() behind the caller's nullifier check (examples/act.rs:60-77) for a slice
  *   act_nullifier_store_*, act_batch_verify_spend_and_refund_recorded
  *                                      = that check against a nullifier database resident on the GPU, recorded as it goes
+ *   act_engine_set_key / _select_key, act_batch_verify_spend_and_refund_keyed
+ *                                      = key rotation: refund() of a proof under the key it names, signed under the current key
+ *                                        (the client checks it with PreRefund::to_credit_token(.., public key), src/lib.rs:1217)
  *
  * Records hold WIRE bytes: points are 32-byte compressed ristretto255 encodings (validated on the
  * device exactly like CompressedRistretto::decompress, src/cbor.rs:62-77) and scalars are 32-byte
@@ -255,6 +258,46 @@ ACT_API int act_nullifier_store_export(act_nullifier_store* s, uint8_t* out, siz
    Replays get status 3 and a zero-filled refund, as in _screened.  The store must be on the device of replica 0. */
 ACT_API int act_batch_verify_spend_and_refund_recorded(act_engine* e, act_nullifier_store* s, size_t n, const uint8_t* proofs,
                                                        const uint8_t* rnd, uint8_t* refunds, uint8_t* nullifiers, uint8_t* status);
+
+/* ---- issuer key slots: key rotation on one engine ----
+ * An engine has ACT_KEY_SLOTS slots.  All of them share the engine's Params, tables and scratch; each holds its own secret x, W
+ * and W table (7.9 MB of device memory).  Slot 0 holds the key given at creation and is selected at first.  The SELECTED slot's key
+ * is what every single-key entry point uses: issue, refund signing (also act_batch_refund_sign and the _seq, _screened and _recorded
+ * calls), spend verification and the client-side checks (act_batch_issuance_check / act_batch_refund_check use its W).
+ *
+ * Keyed spend verification: proof i is verified under the key of slot key_ids[i] (one byte per proof, no alignment needed), and an
+ * accepted proof is refunded under the selected key: that is how tokens move to the current key.  The nullifier is the reduced k,
+ * as in the unkeyed call.  A key id that names an empty slot or a slot >= ACT_KEY_SLOTS gives status 7 (InvalidClientSpendProof),
+ * like a failed challenge; the decode (0x81) and identity (6) checks come first as for every proof.  Key ids come from clients, so a
+ * bad one rejects that request and never the whole call.
+ *
+ * Spent sets per key: `stores` is NULL (no screen) or ACT_KEY_SLOTS entries indexed by slot.  Every slot that holds a key must
+ * map to a non-null store on the device of replica 0, or the call fails before it verifies anything; several slots may share a
+ * store.  Each distinct store screens the status-0 proofs of the slots that map to it, in slice order, with the semantics of
+ * _recorded: a nullifier already in the store or seen at an earlier index of the same store gets status 3 and a zero-filled
+ * refund; the others are recorded.  Proofs of different stores are never compared (two tokens under two keys may carry the same
+ * k).  A call that fails leaves the membership of every store unchanged.  When a key retires, its store is destroyed with it.
+ *
+ * set_key / clear_key wait for the engine's work in flight (also _dev calls on other streams) before they overwrite or free
+ * anything such a call may read.  On a multi-device engine the key calls apply to every replica and the host-buffer keyed calls
+ * shard key_ids with the proofs. */
+#define ACT_KEY_SLOTS 16
+/* installs or replaces the key of a slot; checks pk_w == G*sk_x like act_engine_create.  On failure the slot is unchanged. */
+ACT_API int act_engine_set_key(act_engine* e, int slot, const uint8_t sk_x[32], const uint8_t pk_w[32]);
+/* wipes the slot's secret on the device and the host, then frees its W table; refuses the selected slot and an empty one */
+ACT_API int act_engine_clear_key(act_engine* e, int slot);
+/* the key every single-key entry point uses from now on; the slot must hold a key */
+ACT_API int act_engine_select_key(act_engine* e, int slot);
+ACT_API int act_engine_selected_key(const act_engine* e);            /* -1 for NULL */
+ACT_API uint32_t act_engine_key_slots(const act_engine* e);          /* bit s = slot s holds a key; 0 for NULL */
+ACT_API int act_batch_verify_spend_and_refund_keyed_dev(act_engine* e, size_t n, const void* proofs, const void* key_ids, const void* rnd,
+                                                        void* refunds, void* nullifiers, void* status, void* stream);
+ACT_API int act_batch_verify_spend_and_refund_keyed(act_engine* e, size_t n, const uint8_t* proofs, const uint8_t* key_ids, const uint8_t* rnd,
+                                                    act_nullifier_store* const* stores /* NULL or ACT_KEY_SLOTS entries */,
+                                                    uint8_t* refunds, uint8_t* nullifiers, uint8_t* status);
+/* verification pass of the two-pass form; signing is act_batch_refund_sign (selected key) */
+ACT_API int act_batch_spend_verify_keyed(act_engine* e, size_t n, const uint8_t* proofs, const uint8_t* key_ids, uint8_t* nullifiers, uint8_t* status,
+                                         uint8_t* kprime);
 
 /* Client-side batch generators (SURVEY.md 8f-1), bit-exact with the reference's prover for the same RNG bytes but NOT
  * constant time: they exist to synthesise full-size batches of valid, unique fixtures on the device.

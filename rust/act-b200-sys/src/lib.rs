@@ -30,6 +30,7 @@ pub const ACT_KIND_RESPONSE: c_int = 1;
 pub const ACT_KIND_PROOF: c_int = 2;
 pub const ACT_KIND_REFUND: c_int = 3;
 pub const ACT_STATUS_NOT_CANONICAL: u8 = 0xFF;
+pub const ACT_KEY_SLOTS: usize = 16;
 
 extern "C" {
     pub fn act_last_error() -> *const c_char;
@@ -91,6 +92,21 @@ extern "C" {
     // the issuer's step with the store in place of `seen`; survivors are recorded (store on the device of replica 0)
     pub fn act_batch_verify_spend_and_refund_recorded(e: *mut act_engine, s: *mut act_nullifier_store, n: usize, proofs: *const u8,
                                                       rnd: *const u8, refunds: *mut u8, nullifiers: *mut u8, status: *mut u8) -> c_int;
+    // issuer key slots: verify each spend under the key it names, refund under the selected key, a spent set per key
+    pub fn act_engine_set_key(e: *mut act_engine, slot: c_int, sk_x: *const u8, pk_w: *const u8) -> c_int;
+    pub fn act_engine_clear_key(e: *mut act_engine, slot: c_int) -> c_int;
+    pub fn act_engine_select_key(e: *mut act_engine, slot: c_int) -> c_int;
+    pub fn act_engine_selected_key(e: *const act_engine) -> c_int;
+    pub fn act_engine_key_slots(e: *const act_engine) -> u32;
+    pub fn act_batch_verify_spend_and_refund_keyed_dev(e: *mut act_engine, n: usize, proofs: *const c_void, key_ids: *const c_void,
+                                                       rnd: *const c_void, refunds: *mut c_void, nullifiers: *mut c_void, status: *mut c_void,
+                                                       stream: *mut c_void) -> c_int;
+    // stores: null, or ACT_KEY_SLOTS entries indexed by slot
+    pub fn act_batch_verify_spend_and_refund_keyed(e: *mut act_engine, n: usize, proofs: *const u8, key_ids: *const u8, rnd: *const u8,
+                                                   stores: *const *mut act_nullifier_store, refunds: *mut u8, nullifiers: *mut u8,
+                                                   status: *mut u8) -> c_int;
+    pub fn act_batch_spend_verify_keyed(e: *mut act_engine, n: usize, proofs: *const u8, key_ids: *const u8, nullifiers: *mut u8, status: *mut u8,
+                                        kprime: *mut u8) -> c_int;
     pub fn act_flag_replays(e: *mut act_engine, n: usize, status: *const u8, nullifiers: *const u8, n_seen: usize, seen: *const u8,
                             status_out: *mut u8) -> c_int;
     pub fn act_flag_replays_dev(e: *mut act_engine, n: usize, status: *const c_void, nullifiers: *const c_void, n_seen: usize,
